@@ -2,6 +2,7 @@
 """bench.py - particle-steps/sec of the SandCrate step on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--particles P] [--scene dam_break|box_fill|dam_break_wide]
+    python bench.py --dump-outputs DIR ...      # also write the state after the last timed step as DIR/*.npy
     python bench.py --impl reference ...        # the reference's CPU step on the host cores (same scene mapping)
 
 One "step" = one `physics_tick` over the whole synthetic scene.
@@ -11,6 +12,12 @@ One "step" = one `physics_tick` over the whole synthetic scene.
 The scene is first RELAXED for `--relax` ticks (default 100, SURVEY.md section 8(d): part of the scene, never timed and
 independent of --warmup), then W warm-up ticks, then K timed ticks.  Timed with CUDA events on the stream the kernels
 are launched on; L2 is flushed between timed steps.  Prints ONE JSON line.
+
+--dump-outputs DIR: what the caller of the timed path holds after the last timed step, in float64, rows in ascending
+uid (the particle's insertion index): uid.npy, positions.npy, velocities.npy and, on one GPU, pressure.npy.  Where
+those would exceed DUMP_BYTES (64 MB, headers included), only the rows of a fixed, seeded sample of uids are written.
+The scene is seeded, so the same arguments give the same inputs on every run and two builds can be compared file by
+file.
 """
 from __future__ import annotations
 
@@ -33,6 +40,9 @@ UNIT = "particle-steps/s"
 # cell id), each record moved once per kernel.  These are the figures `roofline.achieved` is computed from.
 SURVEY_BYTES = {"prepass_wall_key": 20, "place": 14, "rank_gather": 56, "density": 28, "force_integrate": 60}
 DEFAULT_PARTICLES = 1_000_000
+DUMP_BYTES = 64_000_000   # all files of --dump-outputs together: 64 MB, so also under 64 MiB
+NPY_HEADER_BYTES = 4096   # allowance per file; np.save writes a 128-byte header for these arrays
+DUMP_SEED = 0
 
 
 def peaks():
@@ -66,6 +76,37 @@ def coeff_vec(world):
     return np.array([p[k] for k in ("dt", "particle_radius", "wall_collision_decay", "pressure_amplifier",
                                     "ignored_pressure", "collider_noise_level", "viscosity", "surface_smoothing",
                                     "target_pressure", "gravity_x", "gravity_y")])
+
+
+def dump_sample(n_total, cols, budget=DUMP_BYTES):
+    """The uids (of 0 .. n_total - 1) whose rows --dump-outputs writes, so that uid.npy plus one float64 file per
+    array of `cols` (name -> per-particle array) stays within `budget` bytes, headers included: None (all of them)
+    when every row fits, else a sorted sample drawn with DUMP_SEED, the same on every run and every rank."""
+    row_bytes = 8 * (1 + sum(int(np.prod(v.shape[1:])) for v in cols.values()))
+    k = (budget - NPY_HEADER_BYTES * (1 + len(cols))) // row_bytes
+    if n_total <= k:
+        return None
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n_total, size=k, replace=False))
+
+
+def select_rows(uid, cols, sample):
+    """The rows of the per-particle arrays `cols` (aligned with `uid`) whose uid is in `sample`, in ascending uid."""
+    order = np.argsort(uid, kind="stable")
+    if sample is not None:
+        order = order[np.isin(uid[order], sample)]
+    return uid[order], {name: v[order] for name, v in cols.items()}
+
+
+def merge_rows(parts):
+    """One (uid, cols) in ascending uid from the (uid, cols) of every rank."""
+    return select_rows(np.concatenate([p[0] for p in parts]),
+                       {k: np.concatenate([p[1][k] for p in parts]) for k in parts[0][1]}, None)
+
+
+def write_dump(out_dir, uid, cols):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in {"uid": uid, **cols}.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(v, dtype=np.float64))
 
 
 class ClockSampler:
@@ -259,8 +300,8 @@ def main():
     os.dup2(2, 1)  # anything a library prints to stdout from here on goes to stderr
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
-    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None, help="timed ticks (default 200; 20 with --impl reference)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up ticks (default 10; 3 with --impl reference)")
     ap.add_argument("--relax", type=int, default=100, help="untimed relaxation ticks that are part of the scene")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--scene", default="dam_break", choices=["dam_break", "box_fill", "dam_break_wide"])
@@ -280,13 +321,20 @@ def main():
     ap.add_argument("--no-numpy-reference", action="store_true")
     ap.add_argument("--no-weak-baseline", action="store_true", help="N > 1: skip the same-scene 1-GPU baseline on rank 0")
     ap.add_argument("--e2e-steps", type=int, default=20)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the state after the last timed step as DIR/<name>.npy "
+                    "(float64, at most 64 MB in all; see the module docstring)")
     a = ap.parse_args()
+    if a.steps is not None and a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.impl == "reference":
-        if a.steps == 200:  # default sized for the GPU arm; keep the CPU arm to about a minute
+        if a.dump_outputs:
+            ap.error("--dump-outputs applies to the GPU arm")
+        if a.steps is None:  # the GPU arm's default would keep the CPU arm busy for minutes; about one is enough
             a.steps = 20
-        a.warmup = max(a.warmup, 1) if a.warmup != 10 else 3
+        a.warmup = 3 if a.warmup is None else max(a.warmup, 1)
         return run_reference_arm(a)
-    a.warmup = max(a.warmup, 3)
+    a.steps = 200 if a.steps is None else a.steps
+    a.warmup = 10 if a.warmup is None else max(a.warmup, 3)
 
     import torch
     import torch.distributed as dist
@@ -375,6 +423,19 @@ def main():
     # pass 1 = THE timed region (value, ms_per_step): plain launches, nothing but the step kernels on the stream
     total_ms, wall, _ = timed_pass(ctx, step_fn, False)
     launches = ctx.launch_count() - launches0
+    dumped = None
+    if a.dump_outputs:   # read back now: the passes below step the scene further
+        if dom is None:
+            pos_d, vel_d, prs_d = ctx.get_state()
+            uid_d, cols = ctx.get_uids(), {"positions": pos_d, "velocities": vel_d, "pressure": prs_d}
+        else:
+            pos_d, vel_d, uid_d = ctx.dist_get_owned()
+            cols = {"positions": pos_d, "velocities": vel_d}
+        dumped = select_rows(uid_d, cols, dump_sample(n_total, cols))
+        if world_size > 1:   # only rank 0 writes
+            parts = [None] * world_size if rank == 0 else None
+            dist.gather_object(dumped, parts, dst=0)
+            dumped = merge_rows(parts) if rank == 0 else None
     # pass 2 = the same K steps again with a CUDA-event pair around every kernel launch (per-kernel durations for
     # the roofline); the extra event records stretch the gaps between kernels, so its step time is not the headline
     total_ms_prof, _, kernels = timed_pass(ctx, step_fn, True)
@@ -457,6 +518,8 @@ def main():
         dist.all_reduce(h2d)
     h2d_bytes, d2h_bytes = int(h2d[0].item()), int(h2d[1].item())
 
+    if dumped is not None and rank == 0:
+        write_dump(a.dump_outputs, *dumped)
     if rank == 0:
         peak, peak_src = peaks()
         top = max((k for k in kernels if k in SURVEY_BYTES), key=lambda k: kernels[k]["ms"], default="density")

@@ -4,7 +4,6 @@ import os
 import sys
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
@@ -42,15 +41,6 @@ def params_from_coeffs(c):
     names = ("dt", "particle_radius", "wall_collision_decay", "pressure_amplifier", "ignored_pressure",
              "collider_noise_level", "viscosity", "surface_smoothing", "target_pressure", "gravity_x", "gravity_y")
     return {n: float(v) for n, v in zip(names, c)}
-
-
-@pytest.fixture(scope="session")
-def have_gpu():
-    try:
-        import torch
-        return torch.cuda.is_available()
-    except Exception:
-        return False
 
 
 def aggregates(pos, vel, prs):
