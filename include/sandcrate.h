@@ -175,19 +175,24 @@ double sc_debug_rerun(sc_ctx *ctx, int which, int reps);
 /* blocks of the tiled density kernel that ran in pass-through mode in the last tick (windows too large to stage) */
 int64_t sc_debug_untiled_blocks(sc_ctx *ctx);
 
-/* ---- multi-GPU strip decomposition (one context per rank; the transport is the caller's: NCCL send/recv) ------ */
+/* ---- multi-GPU strip decomposition (one context per rank) ------------------------------------------------------ */
 /* The reference's search is already a 1-D strip decomposition in y with strip height one diameter
  * (collision_detector.py:10-31, 124-128); rank k owns the cell rows row_lo <= floor(y / d) < row_hi.  Every tick,
- * before sc_step:
- *   sc_dist_pack    drops last tick's ghosts, turns particles whose row left the strip into MIGRANT records for the
- *                   neighbor (they stay here as ghosts for this tick) and copies owned particles within `halo_rows`
- *                   of a cut into HALO records;  send_*_dev: device buffers of sc_dist_wire_bytes(capacity) bytes
- *                   (16-byte header with the record count, then 40-byte records), NULL where there is no neighbor
- *   (caller)        exchanges the buffers, whole, with rank - 1 / rank + 1
- *   sc_dist_unpack  appends received migrants as owned particles and received halos as ghosts
- * A ghost is simulated like any particle and discarded by the next pack.  With halo_rows >= 4 every owned particle
- * sees the neighbors, pressures and normals of the global computation in the same order: SC_PRECISION_F64 results
- * are bit-identical to a single-GPU run.
+ * before sc_step, one of two transports:
+ *   caller's send/recv   sc_dist_pack -> the caller exchanges the buffers, whole, with rank - 1 / rank + 1 (e.g. NCCL)
+ *                        -> sc_dist_unpack
+ *   direct (NVLink)      sc_dist_pack_push -> sc_dist_unpack_flagged
+ * The pack drops last tick's ghosts, turns particles whose row left the strip into MIGRANT records for the neighbor
+ * (they stay here as ghosts for this tick) and copies owned particles within `halo_rows` of a cut into HALO records;
+ * send_*_dev: device buffers of sc_dist_wire_bytes(capacity) bytes (16-byte header with the record count, then 40-byte
+ * records), NULL where there is no neighbor.  The unpack appends received migrants as owned particles and received
+ * halos as ghosts.  A ghost is simulated like any particle and discarded by the next pack.  With halo_rows >= 4 every
+ * owned particle sees the neighbors, pressures and normals of the global computation in the same order:
+ * SC_PRECISION_F64 results are bit-identical to a single-GPU run.
+ * The unpack only records the receive buffers: the next step's first kernel appends their records.  Until then the
+ * particle state is incomplete, so the next call on the context must be sc_step, sc_step_n or sc_step_begin; only
+ * sc_set_tick, sc_synchronize, sc_destroy, sc_last_error, sc_profile_*, sc_launch_count and sc_sync_count may come
+ * before it.  Every other call that takes the context returns an error.
  * Restrictions of the strip mode: noise must be SC_NOISE_COUNTER or SC_NOISE_NONE (the reference's global RNG
  * stream cannot be split across ranks); uids must be < 2^31 (bit 31 marks a ghost copy); the host mirror
  * (sand_crate_b200/strips.py) additionally requires closed scenes (no particle sources) and fixed walls; on a context
@@ -197,20 +202,16 @@ int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_lo, int64_t
                       int64_t wire_capacity);
 int sc_dist_pack(sc_ctx *ctx, void *send_lo_dev, void *send_hi_dev);
 int sc_dist_unpack(sc_ctx *ctx, const void *recv_lo_dev, const void *recv_hi_dev);
-/* Direct NVLink transport instead of send/recv.  sc_dist_push copies header + used records of both packed buffers
- * into the neighbors' receive buffers through peer-mapped device pointers (e.g. torch symmetric memory) and then
- * stores `value` (release, system scope) to each neighbor's flag word; sc_dist_unpack_flagged is sc_dist_unpack whose
- * kernel first waits (on the device) until this rank's flag words have reached `value`.  Use the tick number as
- * `value`: monotonic, never reset.  NULL where there is no neighbor. */
-int sc_dist_push(sc_ctx *ctx, const void *send_lo_dev, void *peer_recv_lo_dev, void *peer_flag_lo_dev,
-                 const void *send_hi_dev, void *peer_recv_hi_dev, void *peer_flag_hi_dev, uint32_t value);
-int sc_dist_unpack_flagged(sc_ctx *ctx, const void *recv_lo_dev, const void *flag_lo_dev, const void *recv_hi_dev,
-                           const void *flag_hi_dev, uint32_t value);
-/* sc_dist_pack and sc_dist_push as ONE kernel: the records are written straight into the neighbors' receive buffers
- * as they are produced (peer stores over NVLink), the last block to finish publishes the counts and raises the flags.
- * send_*_dev are still needed (their headers hold the record counters and the sticky overflow / too_far marks). */
+/* The direct transport.  sc_dist_pack_push is sc_dist_pack whose records are written straight into the neighbors'
+ * receive buffers through peer-mapped device pointers (e.g. torch symmetric memory) as they are produced; the last
+ * block to finish publishes the counts and stores `value` (release, system scope) to each neighbor's flag word.
+ * send_*_dev are still needed (their headers hold the record counters and the sticky overflow / too_far marks).
+ * sc_dist_unpack_flagged is sc_dist_unpack whose records are read (on the device) only once this rank's flag words
+ * have reached `value`.  Use the tick number as `value`: monotonic, never reset.  NULL where there is no neighbor. */
 int sc_dist_pack_push(sc_ctx *ctx, void *send_lo_dev, void *peer_recv_lo_dev, void *peer_flag_lo_dev, void *send_hi_dev,
                       void *peer_recv_hi_dev, void *peer_flag_hi_dev, uint32_t value);
+int sc_dist_unpack_flagged(sc_ctx *ctx, const void *recv_lo_dev, const void *flag_lo_dev, const void *recv_hi_dev,
+                           const void *flag_hi_dev, uint32_t value);
 /* owned particles of this rank, in arbitrary order; uid[i] identifies row i.  Synchronises. */
 int sc_dist_get_owned(sc_ctx *ctx, double *pos, double *vel, uint32_t *uid, int64_t cap, int64_t *n);
 /* device-side flags since creation: capacity overflow, a particle that crossed a whole halo in one tick; the

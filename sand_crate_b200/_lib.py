@@ -82,7 +82,6 @@ SIGNATURES = {
     "sc_dist_configure": (C.c_int, [_ctx, C.c_int, C.c_int, C.c_int64, C.c_int64, C.c_int, C.c_int64]),
     "sc_dist_pack": (C.c_int, [_ctx, C.c_void_p, C.c_void_p]),
     "sc_dist_unpack": (C.c_int, [_ctx, C.c_void_p, C.c_void_p]),
-    "sc_dist_push": (C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]),
     "sc_dist_unpack_flagged": (C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]),
     "sc_dist_pack_push": (C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint32]),
     "sc_dist_get_owned": (C.c_int, [_ctx, _dp, _dp, _up, C.c_int64, _lp]),
@@ -367,14 +366,9 @@ class Context:
     def dist_unpack(self, recv_lo, recv_hi):
         self._ck(self._L.sc_dist_unpack(self._h, self._devptr(recv_lo), self._devptr(recv_hi)))
 
-    def dist_push(self, lo, hi, value):
-        """lo / hi: None or (send buffer, peer receive address, peer flag address)."""
-        lo, hi = lo or (None, None, None), hi or (None, None, None)
-        self._ck(self._L.sc_dist_push(self._h, *[self._devptr(x) for x in lo], *[self._devptr(x) for x in hi],
-                                      C.c_uint32(value)))
-
     def dist_pack_push(self, lo, hi, value):
-        """pack + push fused.  lo / hi: None or (send buffer, peer receive address, peer flag address)."""
+        """pack with the records written straight into the neighbors' receive buffers.  lo / hi: None or (send buffer,
+        peer receive address, peer flag address)."""
         lo, hi = lo or (None, None, None), hi or (None, None, None)
         self._ck(self._L.sc_dist_pack_push(self._h, *[self._devptr(x) for x in lo], *[self._devptr(x) for x in hi],
                                            C.c_uint32(value)))

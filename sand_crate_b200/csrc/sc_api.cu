@@ -18,11 +18,11 @@ static std::string g_create_error;
 
 enum Slot {
     SLOT_CLEAR = 0, SLOT_PREPASS, SLOT_SCAN, SLOT_PLACE, SLOT_RANK_GATHER, SLOT_DENSITY, SLOT_FORCE, SLOT_COUNT,
-    SLOT_RANKMAP, SLOT_IO, SLOT_END, SLOT_DIST_PACK, SLOT_DIST_PUSH, SLOT_DIST_UNPACK
+    SLOT_RANKMAP, SLOT_IO, SLOT_END, SLOT_DIST_PACK
 };
 static const char *k_slot_names[SC_PROFILE_SLOTS] = {
     "clear", "prepass_wall_key", "scan", "place", "rank_gather", "density", "force_integrate", "count_neighbors",
-    "rank_map", "io_scatter", "end_tick", "dist_pack", "dist_push", "dist_unpack", "", ""};
+    "rank_map", "io_scatter", "end_tick", "dist_pack", "", "", "", ""};
 // NVTX range per launch, named after the section of the reference's tick the kernel replaces (the `debug_timer`
 // sections of crate.py:97-124, utils/timer.py:10-48) so a timeline reads like the reference's own Timer overlay
 static const char *k_slot_nvtx[SC_PROFILE_SLOTS] = {
@@ -31,7 +31,7 @@ static const char *k_slot_nvtx[SC_PROFILE_SLOTS] = {
     "Collisions + Colliders + Pressure + tension pass 1 (density kernel)",
     "tension, gravity, pressure, viscosity, wall_bounce, continuous_collision, integrate (force kernel)",
     "tap: neighbor counts", "readback: uid -> row map", "readback / upload", "end tick",
-    "strips: pack", "strips: NVLink push", "strips: unpack", "", ""};
+    "strips: pack", "", "", "", ""};
 
 struct ProfEvent { int slot; cudaEvent_t e0, e1; };
 
@@ -89,14 +89,16 @@ struct sc_ctx {
     double *monitor = nullptr; // 6 sums + particle count of the last tick
     bool dist_on = false;     // strip decomposition: particle arrays hold owned + ghost particles
     DistCfg dist{};
-    WireHeader *wire_dummy = nullptr;  // stands in for a missing neighbor's buffers (+ push completion counters)
-    WireHeader *send_lo = nullptr, *send_hi = nullptr;  // the send buffers of the last sc_dist_pack (re-armed by unpack)
-    unsigned push_toggle = 0;
+    // [0], [1]: send headers standing in for a missing lower / upper neighbor's; [2].count: the "blocks done"
+    // counter of the direct pack kernel (k_dist_pack<..., true>)
+    WireHeader *wire_dummy = nullptr;
+    WireHeader *send_lo = nullptr, *send_hi = nullptr;  // the send buffers of the last pack (re-armed by the pre-pass)
     // The unpack waits for the neighbors' records, and nothing of the tick's first pass over the particles this rank
     // already holds (walls, cell keys) depends on them: the unpack is therefore DEFERRED - recorded here by
     // sc_dist_unpack[_flagged] and carried out by the step's pre-pass itself (PrepassUnpack), whose blocks behind the
     // particles already held wait for the flags and read the receive buffers directly.  One launch less on the critical
-    // path; the neighbors' latency hides behind the pass over the resident particles.
+    // path; the neighbors' latency hides behind the pass over the resident particles.  Until that step, the particle
+    // arrays and the device count lack the records: enter() refuses every call that would read or change them.
     struct { bool on = false; const void *recv_lo = nullptr, *flag_lo = nullptr, *recv_hi = nullptr, *flag_hi = nullptr;
              uint32_t value = 0; } pend;
     int64_t launches = 0;
@@ -128,6 +130,18 @@ static cudaError_t stream_sync(sc_ctx *c) { c->syncs++; return cudaStreamSynchro
         if (r_) return r_;   \
     } while (0)
 
+// Prologue of the entry points that take a context.  Between sc_dist_unpack[_flagged] and the step that carries the
+// unpack out, only the calls that consume it (`consumes_unpack`: sc_step, sc_step_n, sc_step_begin) pass.  The calls
+// that never touch the particle state (sc_set_tick, sc_synchronize, sc_destroy, sc_last_error, measurement) skip it.
+static int enter(sc_ctx *ctx, const char *who, bool consumes_unpack = false) {
+    if (!ctx) return fail(ctx, std::string(who) + ": NULL ctx");
+    if (ctx->pend.on && !consumes_unpack)
+        return fail(ctx, std::string(who) + ": a strip unpack is pending (the next call must be a step)");
+    cudaError_t e = cudaSetDevice(ctx->device);
+    if (e != cudaSuccess) return fail(ctx, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+    return 0;
+}
+
 // launch with programmatic stream serialization (see pdl_enter in sc_common.cuh)
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream, Args &&...args) {
@@ -138,27 +152,6 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, c
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr; cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-
-// launch with or without programmatic stream serialization
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_maybe_pdl(bool pdl, void (*kernel)(KArgs...), dim3 grid, dim3 block, cudaStream_t stream,
-                                    Args &&...args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = 0; cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl ? 1 : 0;
-    cfg.attrs = attr; cfg.numAttrs = 1;
-    return cudaLaunchKernelEx(&cfg, kernel, static_cast<KArgs>(args)...);
-}
-// Which of the strip-exchange kernels (1 pack, 2 push, 4 unpack) are launched with programmatic stream serialization:
-// all of them.  SC_DIST_PDL overrides (developer switch, kept from the hunt for the stale-read hazard described in
-// sc_common.cuh: before that fix, push + unpack launched this way faulted on interior ranks).
-static int dist_pdl_mask() {
-    static int m = -1;
-    if (m < 0) { const char *e = getenv("SC_DIST_PDL"); m = e ? atoi(e) : 7; }
-    return m;
 }
 
 static inline unsigned blocks_for(int64_t n) { return (unsigned)((n + SC_BLOCK - 1) / SC_BLOCK); }
@@ -254,7 +247,6 @@ static int setup_grid(sc_ctx *ctx, double d, int row_min, int row_max, int col_m
 }
 
 static void refresh_wall_boxes(sc_ctx *ctx);
-static int flush_pending_unpack(sc_ctx *ctx);
 static int sync_count(sc_ctx *ctx);
 
 #define SC_DIST_ROW_SLACK 96
@@ -376,8 +368,8 @@ extern "C" void sc_destroy(sc_ctx *c) {
 }
 
 extern "C" int sc_set_params(sc_ctx *ctx, const sc_params *p) {
-    if (!ctx || !p) return fail(ctx, "sc_set_params: NULL argument");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_set_params"));
+    if (!p) return fail(ctx, "sc_set_params: NULL argument");
     if (!(p->particle_radius > 0) || !(p->dt == p->dt)) return fail(ctx, "sc_set_params: particle_radius must be > 0");
     const bool regrid = !ctx->params_set || p->particle_radius != ctx->hp.particle_radius;
     if (regrid && ctx->in_step) return fail(ctx, "sc_set_params: radius change inside a split step");
@@ -460,7 +452,7 @@ static void refresh_wall_boxes(sc_ctx *ctx) {
 
 extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const int32_t *body_len,
                             const double *body_kin, int nbodies) {
-    if (!ctx) return fail(ctx, "sc_set_walls: NULL ctx");
+    CKR(enter(ctx, "sc_set_walls"));
     if (S < 0 || S > SC_MAX_SEGMENTS) return fail(ctx, "sc_set_walls: more than SC_MAX_SEGMENTS segments");
     if (nbodies < 0 || nbodies > SC_MAX_BODIES) return fail(ctx, "sc_set_walls: more than SC_MAX_BODIES bodies");
     if (!ctx->params_set) return fail(ctx, "sc_set_walls: call sc_set_params first (padding needs the radius)");
@@ -483,7 +475,7 @@ extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const in
 }
 
 extern "C" int sc_set_noise(sc_ctx *ctx, int mode, uint64_t seed) {
-    if (!ctx) return fail(ctx, "sc_set_noise: NULL ctx");
+    CKR(enter(ctx, "sc_set_noise"));
     if (mode < SC_NOISE_NONE || mode > SC_NOISE_HOST) return fail(ctx, "sc_set_noise: bad mode");
     ctx->noise_mode = mode; ctx->seed = seed;
     return 0;
@@ -494,12 +486,16 @@ extern "C" int sc_set_tick(sc_ctx *ctx, uint64_t tick) {
     return 0;
 }
 
+// a step ran since cnt->n was last written (no force kernel carried the count): its scan total is the live count
+static void refresh_count(sc_ctx *ctx) {
+    if (!ctx->carry_count) return;
+    ProfScope ps(ctx, SLOT_END);
+    k_end_tick<<<1, 1, 0, ctx->stream>>>(ctx->cnt, ctx->cell_start + ctx->grid.ncells);
+    ctx->carry_count = false;
+}
+
 static int sync_count(sc_ctx *ctx) {
-    if (ctx->carry_count) {  // a step ran since cnt->n was last written: its scan total is the live count
-        ProfScope ps(ctx, SLOT_END);
-        k_end_tick<<<1, 1, 0, ctx->stream>>>(ctx->cnt, ctx->cell_start + ctx->grid.ncells);
-        ctx->carry_count = false;
-    }
+    refresh_count(ctx);
     if (ctx->n_exact) return 0;
     Counters h;
     CK(cudaMemcpyAsync(&h, ctx->cnt, sizeof(Counters), cudaMemcpyDeviceToHost, ctx->stream));
@@ -539,8 +535,7 @@ static int upload_particles(sc_ctx *ctx, const double *pos, const double *vel, i
 }
 
 extern "C" int sc_set_state(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
-    if (!ctx) return fail(ctx, "sc_set_state: NULL ctx");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_set_state"));
     if (n < 0 || n > ctx->cap) return fail(ctx, "sc_set_state: n exceeds capacity");
     if (ctx->in_step) return fail(ctx, "sc_set_state: inside a split step");
     ctx->next_uid = 0;
@@ -553,6 +548,7 @@ extern "C" int sc_set_state(sc_ctx *ctx, const double *pos, const double *vel, i
 }
 
 extern "C" int sc_set_state_uids(sc_ctx *ctx, const double *pos, const double *vel, const uint32_t *uid, int64_t n) {
+    CKR(enter(ctx, "sc_set_state_uids"));
     if (!uid) return fail(ctx, "sc_set_state_uids: uid is NULL");
     uint32_t top = 0;
     for (int64_t i = 0; i < n; ++i) {
@@ -567,8 +563,7 @@ extern "C" int sc_set_state_uids(sc_ctx *ctx, const double *pos, const double *v
 }
 
 extern "C" int sc_append_particles(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
-    if (!ctx) return fail(ctx, "sc_append_particles: NULL ctx");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_append_particles"));
     if (ctx->in_step) return fail(ctx, "sc_append_particles: inside a split step");
     if (n < 0) return fail(ctx, "sc_append_particles: n < 0");
     CKR(sync_count(ctx));
@@ -584,8 +579,8 @@ extern "C" uint64_t sc_source_stream(uint64_t seed, uint64_t tick, uint32_t sour
 }
 
 extern "C" int sc_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsources, int64_t max_particles) {
-    if (!ctx || (nsources > 0 && !sources)) return fail(ctx, "sc_emit_particles: NULL argument");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_emit_particles"));
+    if (nsources > 0 && !sources) return fail(ctx, "sc_emit_particles: NULL argument");
     if (ctx->in_step) return fail(ctx, "sc_emit_particles: inside a split step");
     if (nsources < 0 || nsources > SC_MAX_SOURCES) return fail(ctx, "sc_emit_particles: more than SC_MAX_SOURCES sources");
     if (ctx->dist_on) return fail(ctx, "sc_emit_particles: strips support closed scenes only");
@@ -607,11 +602,7 @@ extern "C" int sc_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsou
     if (!E.nsrc) return 0;
     if ((uint64_t)ctx->next_uid + total >= (uint64_t)SC_GHOST_BIT)
         return fail(ctx, "particle identities exhausted (2^31 particles created in this context)");
-    if (ctx->carry_count) {  // no force kernel ran since the last search: the count still sits in the scan total
-        ProfScope ps(ctx, SLOT_END);
-        k_end_tick<<<1, 1, 0, ctx->stream>>>(ctx->cnt, ctx->cell_start + ctx->grid.ncells);
-        ctx->carry_count = false;
-    }
+    refresh_count(ctx);
     {
         ProfScope ps(ctx, SLOT_IO);
         if (ctx->precision == SC_PRECISION_F64)
@@ -643,8 +634,8 @@ extern "C" int sc_host_free(void *p) {
 }
 
 extern "C" int sc_particle_count(sc_ctx *ctx, int64_t *n) {
-    if (!ctx || !n) return fail(ctx, "sc_particle_count: NULL argument");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_particle_count"));
+    if (!n) return fail(ctx, "sc_particle_count: NULL argument");
     CKR(sync_count(ctx));
     *n = ctx->n_host;
     return 0;
@@ -692,11 +683,9 @@ static int build_rank_map(sc_ctx *ctx, const uint32_t *uid, const uint32_t *n_pt
     return 0;
 }
 
-static int require_ready(sc_ctx *ctx, const char *who) {
-    if (!ctx) return fail(ctx, std::string(who) + ": NULL ctx");
+static int require_ready(sc_ctx *ctx, const char *who, bool consumes_unpack = false) {
+    CKR(enter(ctx, who, consumes_unpack));
     if (!ctx->params_set) return fail(ctx, std::string(who) + ": sc_set_params has not been called");
-    cudaError_t e = cudaSetDevice(ctx->device);
-    if (e != cudaSuccess) return fail(ctx, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
     return 0;
 }
 
@@ -905,7 +894,7 @@ static int enqueue_forces(sc_ctx *ctx, const uint32_t *noise_off) {
 }
 
 extern "C" int sc_step(sc_ctx *ctx) {
-    CKR(require_ready(ctx, "sc_step"));
+    CKR(require_ready(ctx, "sc_step", true));
     if (ctx->in_step) return fail(ctx, "sc_step: a split step is open");
     if (ctx->noise_mode == SC_NOISE_HOST && ctx->hp.collider_noise_level != 0.0)
         return fail(ctx, "sc_step: SC_NOISE_HOST needs sc_step_begin / sc_step_finish");
@@ -919,7 +908,7 @@ extern "C" int sc_step_n(sc_ctx *ctx, int nsteps) {
 }
 
 extern "C" int sc_step_begin(sc_ctx *ctx, int64_t *n_particles, int64_t *n_pairs) {
-    CKR(require_ready(ctx, "sc_step_begin"));
+    CKR(require_ready(ctx, "sc_step_begin", true));
     if (ctx->in_step) return fail(ctx, "sc_step_begin: a split step is already open");
     CKR(enqueue_search<true>(ctx));
     ctx->in_step = true;
@@ -991,8 +980,7 @@ static int ensure_rank_for_current(sc_ctx *ctx) {
 }
 
 extern "C" int sc_get_state(sc_ctx *ctx, double *pos, double *vel, double *pressure, int64_t cap, int64_t *n_out) {
-    if (!ctx) return fail(ctx, "sc_get_state: NULL ctx");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_get_state"));
     if (ctx->in_step) return fail(ctx, "sc_get_state: inside a split step");
     CKR(no_neighbors(ctx, "sc_get_state"));
     CKR(sync_count(ctx));
@@ -1034,8 +1022,7 @@ extern "C" int sc_get_state(sc_ctx *ctx, double *pos, double *vel, double *press
 }
 
 extern "C" int sc_get_uids(sc_ctx *ctx, uint32_t *uid, int64_t cap, int64_t *n_out) {
-    if (!ctx) return fail(ctx, "sc_get_uids: NULL ctx");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_get_uids"));
     if (ctx->in_step) return fail(ctx, "sc_get_uids: inside a split step");
     CKR(no_neighbors(ctx, "sc_get_uids"));
     CKR(sync_count(ctx));
@@ -1053,8 +1040,7 @@ extern "C" int sc_get_uids(sc_ctx *ctx, uint32_t *uid, int64_t cap, int64_t *n_o
 
 // ---- taps --------------------------------------------------------------------------------------------------
 static int tap_prologue(sc_ctx *ctx, const char *who, int64_t cap, int64_t *n_out) {
-    if (!ctx) return fail(ctx, std::string(who) + ": NULL ctx");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, who));
     if (!ctx->srt_valid) return fail(ctx, std::string(who) + ": no search state (call sc_step or sc_step_begin first)");
     CKR(no_neighbors(ctx, who));
     uint32_t total = 0;
@@ -1149,16 +1135,13 @@ extern "C" int sc_get_wall_counts(sc_ctx *ctx, int32_t *counts, int64_t cap) {
 // ---- standalone layer-2 ops ----------------------------------------------------------------------------------
 extern "C" int sc_detect_particle_collisions(sc_ctx *parent, const double *particles, int64_t P, double diameter,
                                              int64_t *rows_sorted, int64_t *order, int32_t *counts, int32_t *idx) {
-    sc_ctx *ctx = parent;
-    if (!parent) return fail(parent, "sc_detect_particle_collisions: NULL ctx");
+    CKR(enter(parent, "sc_detect_particle_collisions"));
     if (P < 0 || !(diameter > 0)) return fail(parent, "sc_detect_particle_collisions: bad arguments");
     if (P == 0) return 0;
-    CK(cudaSetDevice(parent->device));
     // a private context keeps the caller's simulation state untouched
     sc_ctx *t = nullptr;
     if (sc_create(parent->device, SC_PRECISION_F64, P, nullptr, &t)) return fail(parent, g_create_error);
     auto bail = [&](int rc) { if (rc) parent->err = t->err; sc_destroy(t); return rc; };
-    ctx = t;
     int rc = 0;
     do {
         t->hp = sc_params{}; t->hp.particle_radius = diameter / 2; t->params_set = true;
@@ -1191,11 +1174,10 @@ extern "C" int sc_detect_particle_collisions(sc_ctx *parent, const double *parti
 
 extern "C" int sc_points_to_segments_distance(sc_ctx *ctx, const double *p, int64_t P, const double *segments, int S,
                                               double *nearest, double *dist) {
-    if (!ctx) return fail(ctx, "sc_points_to_segments_distance: NULL ctx");
+    CKR(enter(ctx, "sc_points_to_segments_distance"));
     if (P < 0 || S < 0) return fail(ctx, "sc_points_to_segments_distance: bad arguments");
     if (P == 0 || S == 0) return 0;
     if (P * (int64_t)S > ((int64_t)1 << 31) - 1) return fail(ctx, "sc_points_to_segments_distance: P*S too large");
-    CK(cudaSetDevice(ctx->device));
     double2 *dp = nullptr; double *ds = nullptr, *dn = nullptr, *dd = nullptr;
     CK(cudaMalloc((void **)&dp, sizeof(double2) * (size_t)P));
     CK(cudaMalloc((void **)&ds, sizeof(double) * 4 * (size_t)S));
@@ -1216,8 +1198,8 @@ extern "C" int sc_points_to_segments_distance(sc_ctx *ctx, const double *p, int6
 // directed pairs sum(K_i) of the last tick over the particles this context holds (ghosts included), = the number of
 // pair records the density kernel handed to the force kernel.  Synchronises.
 extern "C" int sc_last_pair_count(sc_ctx *ctx, int64_t *n_pairs) {
-    if (!ctx || !n_pairs) return fail(ctx, "sc_last_pair_count: NULL argument");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_last_pair_count"));
+    if (!n_pairs) return fail(ctx, "sc_last_pair_count: NULL argument");
     if (!ctx->srt_valid) { *n_pairs = 0; return 0; }
     CK(cudaMemsetAsync(&ctx->cnt->n_pairs, 0, sizeof(uint32_t), ctx->stream));
     if (ctx->n_host > 0) {
@@ -1273,8 +1255,7 @@ extern "C" int64_t sc_debug_untiled_blocks(sc_ctx *ctx) {
 
 // ---- ForceMonitor (utils/force_monitor.py) ------------------------------------------------------------------------
 extern "C" int sc_set_monitor(sc_ctx *ctx, int on) {
-    if (!ctx) return fail(ctx, "sc_set_monitor: NULL ctx");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_set_monitor"));
     if (on && !ctx->monitor) {
         CKR(dev_alloc(ctx, &ctx->monitor, 8));
         CK(cudaMemsetAsync(ctx->monitor, 0, sizeof(double) * 8, ctx->stream));
@@ -1284,8 +1265,8 @@ extern "C" int sc_set_monitor(sc_ctx *ctx, int on) {
 }
 
 extern "C" int sc_get_monitor(sc_ctx *ctx, double *sum_dv, int64_t *n) {
-    if (!ctx || !sum_dv) return fail(ctx, "sc_get_monitor: NULL argument");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_get_monitor"));
+    if (!sum_dv) return fail(ctx, "sc_get_monitor: NULL argument");
     if (!ctx->monitor) return fail(ctx, "sc_get_monitor: sc_set_monitor(ctx, 1) has not been called");
     double h[8];
     CK(cudaMemcpyAsync(h, ctx->monitor, sizeof(h), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1324,7 +1305,7 @@ static int dist_ready(sc_ctx *ctx, const char *who) {
     CKR(require_ready(ctx, who));
     if (!ctx->dist_on) return fail(ctx, std::string(who) + ": sc_dist_configure has not been called");
     if (ctx->in_step) return fail(ctx, std::string(who) + ": inside a split step");
-    return flush_pending_unpack(ctx);
+    return 0;
 }
 
 extern "C" int64_t sc_dist_wire_bytes(int64_t wire_capacity) {
@@ -1333,8 +1314,7 @@ extern "C" int64_t sc_dist_wire_bytes(int64_t wire_capacity) {
 
 extern "C" int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_lo, int64_t row_hi, int halo_rows,
                                  int64_t wire_capacity) {
-    if (!ctx) return fail(ctx, "sc_dist_configure: NULL ctx");
-    CK(cudaSetDevice(ctx->device));
+    CKR(enter(ctx, "sc_dist_configure"));
     if (nranks < 1 || rank < 0 || rank >= nranks) return fail(ctx, "sc_dist_configure: bad rank");
     if (halo_rows < 1) return fail(ctx, "sc_dist_configure: halo_rows must be >= 1");
     if (wire_capacity < 1 || wire_capacity > ctx->cap) return fail(ctx, "sc_dist_configure: bad wire capacity");
@@ -1347,8 +1327,8 @@ extern "C" int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_
     ctx->dist.has_lo = rank > 0; ctx->dist.has_hi = rank < nranks - 1;
     ctx->dist.cap = (uint32_t)wire_capacity;
     if (!ctx->wire_dummy) {
-        CKR(dev_alloc(ctx, &ctx->wire_dummy, 4));
-        CK(cudaMemsetAsync(ctx->wire_dummy, 0, sizeof(WireHeader) * 4, ctx->stream));
+        CKR(dev_alloc(ctx, &ctx->wire_dummy, 3));
+        CK(cudaMemsetAsync(ctx->wire_dummy, 0, sizeof(WireHeader) * 3, ctx->stream));
     }
     ctx->dist_on = true;
     if (ctx->params_set) {
@@ -1400,11 +1380,7 @@ static uint32_t work_base() {
 extern "C" int sc_dist_row_histogram(sc_ctx *ctx, int64_t row0, int64_t nrows, uint64_t *hist) {
     CKR(dist_ready(ctx, "sc_dist_row_histogram"));
     if (nrows < 1 || nrows > (1 << 24) || !hist) return fail(ctx, "sc_dist_row_histogram: bad arguments");
-    if (ctx->carry_count) {
-        ProfScope ps(ctx, SLOT_END);
-        k_end_tick<<<1, 1, 0, ctx->stream>>>(ctx->cnt, ctx->cell_start + ctx->grid.ncells);
-        ctx->carry_count = false;
-    }
+    refresh_count(ctx);
     unsigned long long *d_hist = nullptr;
     CK(cudaMalloc((void **)&d_hist, sizeof(unsigned long long) * (size_t)nrows));
     CK(cudaMemsetAsync(d_hist, 0, sizeof(unsigned long long) * (size_t)nrows, ctx->stream));
@@ -1413,12 +1389,8 @@ extern "C" int sc_dist_row_histogram(sc_ctx *ctx, int64_t row0, int64_t nrows, u
     const uint8_t *pc = ctx->rows_valid ? ctx->pair_cnt : nullptr;
     if (n > 0) {
         ProfScope ps(ctx, SLOT_IO);
-        if (ctx->precision == SC_PRECISION_F64)
-            k_dist_row_hist<double><<<blocks_for(n), SC_BLOCK, 0, ctx->stream>>>(&ctx->cnt->n, ctx->grid, ctx->pos_cur,
-                                                                             ctx->uid_cur, pc, row0, (int)nrows, d_hist, work_base());
-        else
-            k_dist_row_hist<float><<<blocks_for(n), SC_BLOCK, 0, ctx->stream>>>(&ctx->cnt->n, ctx->grid, ctx->pos_cur,
-                                                                            ctx->uid_cur, pc, row0, (int)nrows, d_hist, work_base());
+        k_dist_row_hist<<<blocks_for(n), SC_BLOCK, 0, ctx->stream>>>(&ctx->cnt->n, ctx->grid, ctx->pos_cur, ctx->uid_cur, pc,
+                                                                     row0, (int)nrows, d_hist, work_base());
     }
     CK(cudaMemcpyAsync(hist, d_hist, sizeof(uint64_t) * (size_t)nrows, cudaMemcpyDeviceToHost, ctx->stream));
     CK(stream_sync(ctx));
@@ -1436,7 +1408,7 @@ static int enqueue_pack(sc_ctx *ctx, const char *who, void *send_lo_dev, void *s
         return fail(ctx, std::string(who) + ": a neighbor exists but its peer pointers are NULL");
     WireHeader *lo = send_lo_dev ? (WireHeader *)send_lo_dev : ctx->wire_dummy;
     WireHeader *hi = send_hi_dev ? (WireHeader *)send_hi_dev : ctx->wire_dummy + 1;
-    if (lo != ctx->send_lo || hi != ctx->send_hi) {  // first use of these buffers: arm them (later k_dist_unpack does)
+    if (lo != ctx->send_lo || hi != ctx->send_hi) {  // first use of these buffers: arm them (later the pre-pass does)
         ProfScope ps(ctx, SLOT_IO);
         k_wire_reset<<<1, 1, 0, ctx->stream>>>(lo, hi);
         ctx->send_lo = lo; ctx->send_hi = hi;
@@ -1470,14 +1442,13 @@ static int enqueue_pack(sc_ctx *ctx, const char *who, void *send_lo_dev, void *s
         if (ctx->dist.has_lo) { plo.peer_hdr = (WireHeader *)peer_recv_lo; plo.recs = reinterpret_cast<WireRec *>(plo.peer_hdr + 1); plo.peer_flag = (uint32_t *)peer_flag_lo; }
         if (ctx->dist.has_hi) { phi.peer_hdr = (WireHeader *)peer_recv_hi; phi.recs = reinterpret_cast<WireRec *>(phi.peer_hdr + 1); phi.peer_flag = (uint32_t *)peer_flag_hi; }
     }
-    uint32_t *done = reinterpret_cast<uint32_t *>(ctx->wire_dummy + 3);  // "blocks done" counter of the fused kernel
+    uint32_t *done = &ctx->wire_dummy[2].count;  // "blocks done" counter of the direct kernel
     if (launch_n > 0) {
         ProfScope ps(ctx, SLOT_DIST_PACK);
         const dim3 grid(std::min<unsigned>(blocks_for(launch_n), 2 * 148)), block(SC_BLOCK);  // grid-stride: few, fat blocks
-        const bool pdl = dist_pdl_mask() & 1;
 #define SC_PACK(REAL, DIRECT)                                                                                        \
-        CK(launch_maybe_pdl(pdl, k_dist_pack<REAL, DIRECT>, grid, block, ctx->stream, ctx->cnt, n_in, g, ctx->dist, R,   \
-                            ctx->pos_cur, (const Vec2<REAL>::type *)ctx->vel_cur, ctx->uid_cur, plo, phi, done, value))
+        CK(launch_pdl(k_dist_pack<REAL, DIRECT>, grid, block, ctx->stream, ctx->cnt, n_in, g, ctx->dist, R,              \
+                      ctx->pos_cur, (const Vec2<REAL>::type *)ctx->vel_cur, ctx->uid_cur, plo, phi, done, value))
         if (ctx->precision == SC_PRECISION_F64) { if (direct) SC_PACK(double, true); else SC_PACK(double, false); }
         else { if (direct) SC_PACK(float, true); else SC_PACK(float, false); }
 #undef SC_PACK
@@ -1498,52 +1469,13 @@ extern "C" int sc_dist_pack_push(sc_ctx *ctx, void *send_lo_dev, void *peer_recv
                         peer_recv_hi_dev, peer_flag_hi_dev, true, value);
 }
 
-static int launch_unpack(sc_ctx *ctx, const void *recv_lo, const void *flag_lo, const void *recv_hi,
-                         const void *flag_hi, uint32_t value) {
-    UnpackSide lo{ctx->dist.has_lo ? (const WireHeader *)recv_lo : nullptr, (const uint32_t *)flag_lo};
-    UnpackSide hi{ctx->dist.has_hi ? (const WireHeader *)recv_hi : nullptr, (const uint32_t *)flag_hi};
-    if (lo.hdr || hi.hdr) {
-        ProfScope ps(ctx, SLOT_DIST_UNPACK);
-        const dim3 grid(std::min<unsigned>(blocks_for(ctx->dist.cap), 74), 2);  // grid-stride
-        if (ctx->precision == SC_PRECISION_F64)
-            CK(launch_maybe_pdl(dist_pdl_mask() & 4, k_dist_unpack<double>, grid, dim3(SC_BLOCK), ctx->stream,
-                lo, hi, value, ctx->dist.cap, ctx->pos_cur, (double2 *)ctx->vel_cur, ctx->uid_cur, &ctx->cnt->n,
-                (const uint32_t *)&ctx->cnt->n_split, (uint32_t)ctx->cap, &ctx->cnt->overflow, ctx->send_lo ? ctx->send_lo : ctx->wire_dummy,
-                ctx->send_hi ? ctx->send_hi : ctx->wire_dummy + 1));
-        else
-            CK(launch_maybe_pdl(dist_pdl_mask() & 4, k_dist_unpack<float>, grid, dim3(SC_BLOCK), ctx->stream,
-                lo, hi, value, ctx->dist.cap, ctx->pos_cur, (float2 *)ctx->vel_cur, ctx->uid_cur, &ctx->cnt->n,
-                (const uint32_t *)&ctx->cnt->n_split, (uint32_t)ctx->cap, &ctx->cnt->overflow, ctx->send_lo ? ctx->send_lo : ctx->wire_dummy,
-                ctx->send_hi ? ctx->send_hi : ctx->wire_dummy + 1));
-    }
-    CK(cudaGetLastError());
-    return 0;
-}
-
-// a deferred unpack that the step has not consumed yet (somebody asks for the state between unpack and step)
-static int flush_pending_unpack(sc_ctx *ctx) {
-    if (!ctx->pend.on) return 0;
-    ctx->pend.on = false;
-    return launch_unpack(ctx, ctx->pend.recv_lo, ctx->pend.flag_lo, ctx->pend.recv_hi, ctx->pend.flag_hi, ctx->pend.value);
-}
-
-static bool defer_unpack() {
-    // SC_DIST_DEFER=0 (developer switch): launch k_dist_unpack where sc_dist_unpack is called (A/B timing)
-    static int v = -1;
-    if (v < 0) { const char *e = getenv("SC_DIST_DEFER"); v = e ? atoi(e) : 1; }
-    return v != 0;
-}
-
-static int enqueue_unpack(sc_ctx *ctx, const void *recv_lo, const void *flag_lo, const void *recv_hi,
-                          const void *flag_hi, uint32_t value) {
-    CKR(flush_pending_unpack(ctx));
-    if (defer_unpack()) {
-        ctx->pend.on = true;
-        ctx->pend.recv_lo = recv_lo; ctx->pend.flag_lo = flag_lo; ctx->pend.recv_hi = recv_hi; ctx->pend.flag_hi = flag_hi;
-        ctx->pend.value = value;
-    } else {
-        CKR(launch_unpack(ctx, recv_lo, flag_lo, recv_hi, flag_hi, value));
-    }
+// The unpack is only recorded: the next step's pre-pass appends the records (PrepassUnpack) and enter() holds every
+// other call off until then.
+static int record_unpack(sc_ctx *ctx, const void *recv_lo, const void *flag_lo, const void *recv_hi, const void *flag_hi,
+                         uint32_t value) {
+    ctx->pend.on = true;
+    ctx->pend.recv_lo = recv_lo; ctx->pend.flag_lo = flag_lo; ctx->pend.recv_hi = recv_hi; ctx->pend.flag_hi = flag_hi;
+    ctx->pend.value = value;
     // the live count (owned + ghosts) is only known on the device: launch over the whole capacity, kernels exit early
     ctx->n_host = ctx->cap;
     ctx->n_exact = false;
@@ -1552,46 +1484,20 @@ static int enqueue_unpack(sc_ctx *ctx, const void *recv_lo, const void *flag_lo,
 
 extern "C" int sc_dist_unpack(sc_ctx *ctx, const void *recv_lo_dev, const void *recv_hi_dev) {
     CKR(dist_ready(ctx, "sc_dist_unpack"));
-    return enqueue_unpack(ctx, recv_lo_dev, nullptr, recv_hi_dev, nullptr, 0);
+    return record_unpack(ctx, recv_lo_dev, nullptr, recv_hi_dev, nullptr, 0);
 }
 
 extern "C" int sc_dist_unpack_flagged(sc_ctx *ctx, const void *recv_lo_dev, const void *flag_lo_dev,
                                       const void *recv_hi_dev, const void *flag_hi_dev, uint32_t value) {
     CKR(dist_ready(ctx, "sc_dist_unpack_flagged"));
-    return enqueue_unpack(ctx, recv_lo_dev, flag_lo_dev, recv_hi_dev, flag_hi_dev, value);
+    return record_unpack(ctx, recv_lo_dev, flag_lo_dev, recv_hi_dev, flag_hi_dev, value);
 }
 
-extern "C" int sc_dist_push(sc_ctx *ctx, const void *send_lo_dev, void *peer_recv_lo_dev, void *peer_flag_lo_dev,
-                            const void *send_hi_dev, void *peer_recv_hi_dev, void *peer_flag_hi_dev, uint32_t value) {
-    CKR(dist_ready(ctx, "sc_dist_push"));
-    uint32_t *done = reinterpret_cast<uint32_t *>(ctx->wire_dummy + 2);  // "blocks done" counters, one per direction
-    PushSide lo{nullptr, nullptr, nullptr, done}, hi{nullptr, nullptr, nullptr, done + 1};
-    if (ctx->dist.has_lo) {
-        if (!send_lo_dev || !peer_recv_lo_dev || !peer_flag_lo_dev) return fail(ctx, "sc_dist_push: NULL lower buffer");
-        lo.src = (const WireHeader *)send_lo_dev; lo.peer_dst = peer_recv_lo_dev; lo.peer_flag = (uint32_t *)peer_flag_lo_dev;
-    }
-    if (ctx->dist.has_hi) {
-        if (!send_hi_dev || !peer_recv_hi_dev || !peer_flag_hi_dev) return fail(ctx, "sc_dist_push: NULL upper buffer");
-        hi.src = (const WireHeader *)send_hi_dev; hi.peer_dst = peer_recv_hi_dev; hi.peer_flag = (uint32_t *)peer_flag_hi_dev;
-    }
-    if (!lo.src && !hi.src) return 0;
-    ProfScope ps(ctx, SLOT_DIST_PUSH);
-    const size_t bytes = sizeof(WireHeader) + (size_t)ctx->dist.cap * sizeof(WireRec);
-    const unsigned nb = (unsigned)std::min<size_t>((bytes / 16 + SC_BLOCK - 1) / SC_BLOCK, 64);
-    CK(launch_maybe_pdl(dist_pdl_mask() & 2, k_wire_push, dim3(nb, 2), dim3(SC_BLOCK), ctx->stream, lo, hi, ctx->dist.cap, value));
-    CK(cudaGetLastError());
-    return 0;
-}
-
-// NOTE: unpack's kernels clamp the appended count on overflow only by flagging; cnt->n may exceed cap by the number
-// of dropped records, every kernel bounds its index by the arrays' capacity through n_host <= cap.
+// NOTE: the unpacking pre-pass clamps the appended count on overflow only by flagging; cnt->n may exceed cap by the
+// number of dropped records, every kernel bounds its index by the arrays' capacity through n_host <= cap.
 extern "C" int sc_dist_get_owned(sc_ctx *ctx, double *pos, double *vel, uint32_t *uid, int64_t cap, int64_t *n_out) {
     CKR(dist_ready(ctx, "sc_dist_get_owned"));
-    if (ctx->carry_count) {
-        ProfScope ps(ctx, SLOT_END);
-        k_end_tick<<<1, 1, 0, ctx->stream>>>(ctx->cnt, ctx->cell_start + ctx->grid.ncells);
-        ctx->carry_count = false;
-    }
+    refresh_count(ctx);
     CK(cudaMemsetAsync(&ctx->cnt->n_tmp, 0, sizeof(uint32_t), ctx->stream));
     const int64_t n = ctx->n_host;
     if (n > 0) {

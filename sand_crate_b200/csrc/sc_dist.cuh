@@ -1,4 +1,5 @@
-// sc_dist.cuh - strip decomposition across GPUs: pack / unpack kernels of the per-tick boundary exchange.
+// sc_dist.cuh - strip decomposition across GPUs: the pack kernel of the per-tick boundary exchange (the unpack is done
+// by the step's pre-pass, k_prepass<..., true> in sc_sort.cuh), the owned-particle readback and the re-cut histogram.
 //
 // The reference's own neighbor search is a 1-D strip decomposition in y with strip height one diameter
 // (collision_detector.py:10-31, 124-128); the same rows are the multi-GPU partition unit.  Rank k owns the cell rows
@@ -54,9 +55,9 @@ __device__ __forceinline__ void wire_store(WireHeader *h, WireRec *recs, uint32_
 //   last tick's ghost      -> killed: its x becomes +inf, so this tick's remove_particles pass (k_prepass) drops it
 //   row left the strip     -> MIGRANT record for the neighbor; stays here, re-tagged as a ghost, for this tick
 //   owned, near a cut      -> HALO record(s)
-// n_in_ptr = live count left by the previous tick (its scan total) or cnt->n; it is copied to cnt->n, where the
-// unpack kernel appends what the neighbors send.  The send headers' counts are zero on entry (k_dist_unpack re-arms
-// them once the previous tick's buffers have left).
+// n_in_ptr = live count left by the previous tick (its scan total) or cnt->n; it is copied to cnt->n and cnt->n_split,
+// behind which the step's pre-pass appends what the neighbors send.  The send headers' counts are zero on entry (the
+// pre-pass re-arms them once the previous tick's buffers have left).
 //
 // Only the rows near a cut can hold any of the three.  The arrays are in the last tick's sorted order (cell rows
 // ascending), so those rows are two index ranges, [0, A) and [B, n), read off the last tick's cell boundaries
@@ -66,7 +67,7 @@ __device__ __forceinline__ void wire_store(WireHeader *h, WireRec *recs, uint32_
 // kDirect (the NVLink transport): the records are written straight into the neighbor's receive buffer through a
 // peer-mapped pointer - pack and transfer are ONE kernel, the bytes cross NVLink as they are produced - and the last
 // block to finish publishes the record count and raises the neighbor's flag (release, system scope); the neighbor's
-// unpack kernel, running on its own GPU, acquires it.
+// pre-pass, running on its own GPU, acquires it.
 struct PackRange {
     const uint32_t *cell_start;  // last tick's cell boundaries, or NULL: cover all particles
     uint32_t cell_a, cell_b;     // first cell of the first row above the lower boundary zone / of the upper boundary zone
@@ -155,47 +156,6 @@ k_dist_pack(Counters *cnt, const uint32_t *n_in_ptr, Grid g, DistCfg D, PackRang
     }
 }
 
-// both neighbors' buffers in one launch (blockIdx.y = side).  With the direct NVLink transport every block first
-// waits for BOTH flags to reach `value` (raised by the neighbors' pack kernels, which run on other GPUs).  Where a record
-// lands is a pure function of its position in its buffer - the lower neighbor's records directly behind the particles
-// this rank already held (*n_split, left there by k_dist_pack), the upper neighbor's behind those - so there is no atomic
-// on the particle counter (one per record meant ~25 000 serialized operations on one address per tick).
-template <typename Real>
-__global__ void __launch_bounds__(SC_BLOCK)
-k_dist_unpack(UnpackSide lo, UnpackSide hi, uint32_t value, uint32_t wire_cap, double2 *pos,
-              typename Vec2<Real>::type *vel, uint32_t *uid, uint32_t *n, const uint32_t *n_split,
-              uint32_t cap, uint32_t *overflow, WireHeader *send_lo, WireHeader *send_hi) {
-    pdl_enter();
-    // this tick's send buffers have left (stream order): re-arm their counts for the next k_dist_pack; the sticky
-    // overflow / too_far marks stay for sc_dist_status
-    if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) { send_lo->count = 0u; send_hi->count = 0u; }
-    if (threadIdx.x == 0) {
-        if (lo.hdr && lo.flag) while ((int)(ld_acquire_sys(lo.flag) - value) < 0) __nanosleep(64);
-        if (hi.hdr && hi.flag) while ((int)(ld_acquire_sys(hi.flag) - value) < 0) __nanosleep(64);
-    }
-    __syncthreads();
-    const uint32_t c_lo = lo.hdr ? (lo.hdr->count < wire_cap ? lo.hdr->count : wire_cap) : 0u;
-    const uint32_t c_hi = hi.hdr ? (hi.hdr->count < wire_cap ? hi.hdr->count : wire_cap) : 0u;
-    const uint32_t base = *n_split;
-    if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) {
-        *n = base + c_lo + c_hi;  // k_prepass clamps it to the capacity and raises the overflow flag
-        if (base + c_lo + c_hi > cap) *overflow = 1u;
-    }
-    const UnpackSide side = blockIdx.y ? hi : lo;
-    if (!side.hdr) return;
-    const uint32_t count = blockIdx.y ? c_hi : c_lo;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < count; i += gridDim.x * blockDim.x) {
-        const uint32_t k = base + (blockIdx.y ? c_lo : 0u) + i;
-        if (k >= cap) return;
-        const WireRec r = reinterpret_cast<const WireRec *>(side.hdr + 1)[i];
-        pos[k] = make_double2(r.px, r.py);
-        typename Vec2<Real>::type v;
-        v.x = (Real)r.vx; v.y = (Real)r.vy;
-        vel[k] = v;
-        uid[k] = r.kind == SC_WIRE_HALO ? (r.uid | SC_GHOST_BIT) : r.uid;
-    }
-}
-
 // owned particles (no ghosts) compacted into staging arrays for readback; order is arbitrary, uids identify rows
 template <typename Real>
 __global__ void __launch_bounds__(SC_BLOCK)
@@ -214,36 +174,6 @@ k_dist_collect_owned(const uint32_t *n_ptr, const double2 *pos,
     uid_out[k] = u;
 }
 
-// Direct NVLink transport: copies the used part of a packed wire buffer (header + count records) into the neighbor's
-// receive buffer through a peer-mapped pointer (torch symmetric memory), then raises the neighbor's flag: every block
-// fences its stores to system scope and the last block to finish publishes `value` (the tick number, monotonic,
-// so flags are never reset).  The receiver's unpack kernel spins on the flag - the two kernels run on different
-// GPUs, so neither waits for a launch on its own device.
-struct PushSide { const WireHeader *src; void *peer_dst; uint32_t *peer_flag; uint32_t *done; };
-
-__global__ void __launch_bounds__(SC_BLOCK)
-k_wire_push(PushSide lo, PushSide hi, uint32_t cap, uint32_t value) {
-    pdl_enter();
-    const PushSide side = blockIdx.y ? hi : lo;
-    if (!side.src) return;
-    const uint32_t count = side.src->count < cap ? side.src->count : cap;
-    const size_t bytes = sizeof(WireHeader) + (size_t)count * sizeof(WireRec);
-    const size_t chunks = (bytes + 15) / 16;
-    const uint4 *s4 = reinterpret_cast<const uint4 *>(side.src);
-    uint4 *d4 = reinterpret_cast<uint4 *>(side.peer_dst);
-    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < chunks; i += (size_t)gridDim.x * blockDim.x)
-        d4[i] = s4[i];
-    __threadfence_system();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        const uint32_t prev = atomicAdd(side.done, 1u);
-        if (prev == gridDim.x - 1) {
-            *side.done = 0u;
-            st_release_sys(side.peer_flag, value);
-        }
-    }
-}
-
 // per-row WORK of the owned particles (input of the partition re-cut): hist[row - row0], rows outside are clamped.
 // A particle weighs work_base + K_i, K_i = its directed pairs of the last tick: the pair kernels are two thirds of a tick,
 // their cost grows with K, and K is anything but uniform - the bottom strip of the settled 64M column holds 10.5 pairs
@@ -257,7 +187,6 @@ k_wire_push(PushSide lo, PushSide hi, uint32_t cap, uint32_t value) {
 // summed value) and issues one global atomic per row it touched - instead of one per particle, 32M of them on a few
 // dozen hot addresses in the 64M scene (8 ms; profiles/r3f_*).  Rows outside the window fall back to global atomics.
 #define SC_HIST_WIN 64
-template <typename Real>
 __global__ void __launch_bounds__(SC_BLOCK)
 k_dist_row_hist(const uint32_t *n_ptr, Grid g, const double2 *pos,
                 const uint32_t *uid, const uint8_t *pair_cnt, long long row0, int nrows, unsigned long long *hist,

@@ -71,25 +71,15 @@ def partition_rows(rows: np.ndarray, nranks: int, halo_rows: int = HALO_ROWS) ->
     least 2 * halo_rows high."""
     if nranks == 1:
         return [INT64_MIN, INT64_MAX]
-    lo, hi = int(rows.min()), int(rows.max())
-    hist = np.bincount(rows - lo, minlength=hi - lo + 1)
-    cum = np.cumsum(hist)
-    cuts = [INT64_MIN]
-    prev = lo
-    for k in range(1, nranks):
-        target = cum[-1] * k / nranks
-        r = lo + int(np.searchsorted(cum, target, side="left")) + 1  # first row of rank k
-        r = max(r, prev + 2 * halo_rows)
-        cuts.append(r)
-        prev = r
-    cuts.append(INT64_MAX)
-    if cuts[-2] + 2 * halo_rows > hi + 1 and nranks > 1:
-        raise ValueError(f"scene has too few cell rows ({hi - lo + 1}) for {nranks} strips of >= {2 * halo_rows} rows")
-    return cuts
+    lo = int(rows.min())
+    return partition_histogram(np.bincount(rows - lo), lo, nranks, halo_rows)
 
 
 def cuts_from_histogram(hist: np.ndarray, row0: int, nranks: int, halo_rows: int = HALO_ROWS) -> list[int]:
-    """The same equal-count cuts as `partition_rows`, from a per-row particle histogram starting at row `row0`."""
+    """Equal-weight cuts from a per-row histogram (`hist[k]` = weight of row `row0 + k`): cut k is the row after the
+    one where the cumulative weight reaches k / nranks of the total, and at least 2 * halo_rows above the previous cut.
+    The first cut's floor is `row0 + 2 * halo_rows`, so the histogram is used as given: trimming its empty end rows
+    would move that floor."""
     if nranks == 1:
         return [INT64_MIN, INT64_MAX]
     cum = np.cumsum(hist.astype(np.int64))
@@ -105,7 +95,8 @@ def cuts_from_histogram(hist: np.ndarray, row0: int, nranks: int, halo_rows: int
 
 
 def partition_histogram(hist: np.ndarray, row0: int, nranks: int, halo_rows: int = HALO_ROWS) -> list[int]:
-    """`partition_rows` from a per-row histogram (`hist[k]` = particles in row `row0 + k`)."""
+    """`cuts_from_histogram` over the occupied rows of `hist` (`hist[k]` = particles in row `row0 + k`); raises if
+    they are too few for nranks strips of at least 2 * halo_rows rows."""
     nz = np.nonzero(hist)[0]
     lo, hi = row0 + int(nz[0]), row0 + int(nz[-1])
     cuts = cuts_from_histogram(hist[nz[0]:nz[-1] + 1], lo, nranks, halo_rows)

@@ -605,6 +605,52 @@ def test_recut_histogram_counts_every_owned_particle_once():
     assert narrow.sum() == hist.sum() and np.array_equal(narrow[1:-1], hist[101:129])
 
 
+def test_pending_unpack_admits_only_the_step():
+    """sc_dist_unpack only records the receive buffers; the next step's pre-pass appends the records.  In between, the
+    particle arrays and the device count lack them, so calls that read or change the state are refused - and the step
+    then appends the neighbor's migrant as an owned particle and its halos as ghosts."""
+    import torch
+    from sand_crate_b200.strips import HALO_ROWS, INT64_MIN
+    world, pos, vel = dam_break(4000, height=0.4)
+    pos = pos - [0.0, 0.5]      # the column (y in 0.58 .. 0.99) lifted, so the neighbor's rows above it lie in the box
+    c = world.coefficients
+    r, d = c["particle_radius"], 2 * c["particle_radius"]
+    ctx = _lib.Context(len(pos) + 1024, _lib.PRECISION_F64)
+    ctx.set_params(**{k: float(c[k]) for k in _lib.PARAM_FIELDS[:9]},
+                   gravity_x=float(c["gravity"][0]), gravity_y=float(c["gravity"][1]))
+    seg = np.array(world.rigid_bodies[0]["fixed"]["segments"], dtype=np.float64)
+    ctx.set_walls(seg, [len(seg)], np.zeros((1, 5)))
+    ctx.set_noise(_lib.NOISE_COUNTER, 3)
+    ctx.set_state_uids(pos, vel, np.arange(len(pos), dtype=np.uint32))
+    row_hi = int(np.floor(pos[:, 1] / d).max()) + 20      # an upper neighbor far above every particle, no lower one
+    assert (row_hi + 2) * d < 1
+    wire_cap = 256
+    ctx.dist_configure(0, 2, INT64_MIN, row_hi, HALO_ROWS, wire_cap)
+    ctx.step()
+    p0, _, uid0 = ctx.dist_get_owned()
+    removed = int(((p0 < -r) | (p0 > 1 + r)).any(axis=1).sum())   # what the next step's removal pass drops
+    nbytes = _lib.wire_bytes(wire_cap)
+    rec = np.dtype([("px", "f8"), ("py", "f8"), ("vx", "f8"), ("vy", "f8"), ("uid", "u4"), ("kind", "u4")])
+    recs = np.array([(0.3, (row_hi - 2 + 0.5) * d, 0.0, 0.0, 1_000_000, 0),    # MIGRANT into this strip
+                     (0.6, (row_hi + 0.5) * d, 0.0, 0.0, 1_000_001, 1),        # HALO rows of the neighbor
+                     (0.7, (row_hi + 1.5) * d, 0.0, 0.0, 1_000_002, 1)], dtype=rec)
+    raw = np.zeros(nbytes, np.uint8)
+    raw[:16].view(np.uint32)[:] = [len(recs), 0, 0, 0]
+    raw[16:16 + rec.itemsize * len(recs)].view(rec)[:] = recs
+    send_hi, recv_hi = torch.zeros(nbytes, dtype=torch.uint8, device="cuda"), torch.from_numpy(raw).cuda()
+    torch.cuda.synchronize()                              # written on torch's stream, used on the context's
+    ctx.dist_pack(None, send_hi)
+    ctx.dist_unpack(None, recv_hi)
+    for call in (ctx.particle_count, lambda: ctx.dist_status(None, send_hi), ctx.dist_get_owned,
+                 lambda: ctx.set_state_uids(pos, vel, np.arange(len(pos), dtype=np.uint32))):
+        with pytest.raises(_lib.SandCrateError, match="unpack"):
+            call()
+    ctx.step()
+    _, _, uid1 = ctx.dist_get_owned()
+    assert 1_000_000 in uid1 and len(uid1) == len(uid0) - removed + 1
+    assert ctx.dist_status()["n_local"] == len(uid0) - removed + 3
+
+
 # ---- multi-GPU: strip decomposition over NCCL (needs >= 2 GPUs; skipped on a 1-GPU box) -------------------------
 def test_strips_two_gpus_bit_identical_to_single_gpu():
     import os
