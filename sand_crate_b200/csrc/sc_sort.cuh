@@ -282,13 +282,17 @@ k_rank_gather(Grid g, const uint32_t *cell_start, const uint32_t *tmpidx,
     const typename Vec2<Real>::type v_own = vel[i];
     const bool touching = (wall_bits[i >> 5] >> (i & 31)) & 1u;
     const uint32_t um = u & 0x7FFFFFFFu;  // ties are broken by identity; bit 31 only marks a ghost copy
+    // Two records of one identity at one x never meet in a correct run, but if they do (a uid handed to set_state_uids
+    // twice, a strip exchange that keeps a migrant or a ghost it should drop) the array index decides: the ranks must
+    // stay a permutation of the cell.  Two equal ranks would leave a sorted slot unwritten, and the pair kernels would
+    // then walk the cell neighborhood of whatever stale cell key that slot held - outside the arrays.
     uint32_t rank = 0;
     for (uint32_t m = beg; m < end; ++m) {
         if (m == t) continue;
         const uint32_t j = tmpidx[m];
         const double xj = pos[j].x;
         const uint32_t uj = uid[j] & 0x7FFFFFFFu;
-        rank += (x_less(xj, p.x) || (!x_less(p.x, xj) && uj < um)) ? 1u : 0u;
+        rank += (x_less(xj, p.x) || (!x_less(p.x, xj) && (uj < um || (uj == um && j < i)))) ? 1u : 0u;
     }
     const uint32_t f = beg + rank;
     pos_s[f] = p;
