@@ -55,13 +55,20 @@ struct sc_ctx {
     BlockDesc *blk_desc = nullptr;    // mixed mode: per block of SC_TILE sorted particles, its three windows
     void *vel_cur = nullptr, *vel_srt = nullptr;
     uint32_t *uid_cur = nullptr, *uid_srt = nullptr;
-    uint32_t *cell_key = nullptr, *cell_key_srt = nullptr, *slot = nullptr, *tmpidx = nullptr;
-    // The cell grid and the wall bitmaps are double buffered by tick parity: a tick's force kernel clears the OTHER set
-    // for the next tick (end_of_tick, sc_common.cuh), so a tick does not open with a clearing launch.  cell_start /
-    // wall_bits_* always point at the set of the last search (the taps read them).
-    uint32_t *cell_bufs[2] = {nullptr, nullptr}, *cell_start = nullptr; size_t cell_cap = 0;
+    uint32_t *cell_key = nullptr, *cell_key_srt = nullptr, *tmpidx = nullptr;
+    // One cell-count grid and one cell_start array (+ the live count at [ncells]).  The counts are zero between ticks:
+    // k_place takes each one back down (sc_sort.cuh).  cell_start holds the last search's boundaries until the next
+    // tick's scan (the taps and the strip pack read them).
+    uint32_t *cell_count = nullptr, *cell_start = nullptr; size_t cell_cap = 0;
+    // The wall bitmaps, side list and its counter are double buffered by tick parity: the force kernel of one tick may
+    // fill the next tick's (NextKeys) while it reads its own.  wall_bits_* / wall_pre point at the last search's set.
     int par = 0;
-    bool next_clean = false;  // the other set has been cleared by the last force kernel
+    bool next_clean = false;  // the next tick finds the grid, its wall set and the scan descriptors cleared
+    // The last force kernel ran the next tick's key pass (NextKeys, sc_pair.cuh) and nothing since changed what the keys
+    // depend on: the next tick launches no k_prepass.  pos_cur then holds the positions AFTER the next tick's hard-wall
+    // fix (the readback undoes it: k_scatter_pos), and drop_keys() takes it all back when a call invalidates it.
+    bool next_keyed = false;
+    bool keys_dropped = true;  // a call since the last step invalidated the keys: this step's force kernel computes none
     unsigned long long *bsum = nullptr; size_t bsum_cap = 0;    // cell scan: tile descriptors, [0] = ticket
     unsigned long long *bsum2 = nullptr; size_t bsum2_cap = 0;  // the same for every other scan (readback maps)
     void *ps = nullptr;               // PS<Real>[cap]: pressure + surface normal of the sorted set
@@ -69,7 +76,7 @@ struct sc_ctx {
     uint32_t *pair_off = nullptr; uint8_t *pair_cnt = nullptr;
     uint32_t *wbits_cur[2] = {nullptr, nullptr}, *wbits_srt[2] = {nullptr, nullptr};
     uint32_t *wall_bits_cur = nullptr, *wall_bits_srt = nullptr, *wall_slot_cur = nullptr, *wall_slot_srt = nullptr;
-    double2 *wall_pre = nullptr;
+    double2 *wall_pre_buf[2] = {nullptr, nullptr}, *wall_pre = nullptr;
     Counters *cnt = nullptr;
     uint32_t *rank_of_uid = nullptr; size_t uid_cap = 0;
     uint32_t next_uid = 0;
@@ -226,14 +233,14 @@ static int setup_grid(sc_ctx *ctx, double d, int row_min, int row_max, int col_m
     g.ncells = (uint32_t)(nrows * ncols);
     const size_t need = (size_t)g.ncells + 8;  // + the live count at [ncells]; bulk copies read whole 16-byte groups
     if (need > ctx->cell_cap) {
-        for (int q = 0; q < 2; ++q) {
-            if (ctx->cell_bufs[q]) CK(cudaFree(ctx->cell_bufs[q]));
-            CKR(dev_alloc(ctx, &ctx->cell_bufs[q], need));
-        }
+        if (ctx->cell_count) CK(cudaFree(ctx->cell_count));
+        if (ctx->cell_start) CK(cudaFree(ctx->cell_start));
+        CKR(dev_alloc(ctx, &ctx->cell_count, need));
+        CKR(dev_alloc(ctx, &ctx->cell_start, need));
         ctx->cell_cap = need;
     }
-    ctx->cell_start = ctx->cell_bufs[ctx->par];
     ctx->next_clean = false;  // a new grid: the next tick clears it itself
+    ctx->next_keyed = false;  // (every caller has dropped the keys first: drop_keys)
     const size_t nb = (size_t)(g.ncells + SC_SCAN_TILE - 1) / SC_SCAN_TILE + 2;
     const size_t nb2 = (size_t)(ctx->cap + SC_SCAN_TILE - 1) / SC_SCAN_TILE + 2;
     const size_t needb = nb > nb2 ? nb : nb2;
@@ -288,6 +295,34 @@ static int refresh_dev_params(sc_ctx *ctx) {
     return 0;
 }
 
+// k_begin_tick over the cell-count grid and the wall set of tick parity `q` (see there for `carry` and `restore`)
+static int launch_clear(sc_ctx *ctx, int q, const uint32_t *carry, KeyRestore restore) {
+    const Grid &g = ctx->grid;
+    ProfScope ps(ctx, SLOT_CLEAR);
+    const uint32_t words = (uint32_t)(ctx->cap / 32 + 1);
+    const unsigned nb = (unsigned)std::min<int64_t>(((int64_t)g.ncells / 4 + SC_BLOCK - 1) / SC_BLOCK + 1, 148 * 16);
+    const uint32_t scan_words = (g.ncells + SC_SCAN_TILE - 1) / SC_SCAN_TILE + 1;  // ticket + descriptors
+    CK(launch_pdl(k_begin_tick, dim3(nb), dim3(SC_BLOCK), ctx->stream, ctx->cnt, ctx->cell_count, g.ncells, carry,
+                  ctx->wbits_cur[q], ctx->wbits_srt[q], words, ctx->bsum, scan_words, (uint32_t)ctx->cap, restore));
+    return 0;
+}
+
+// Called by every entry point that changes what the next tick's keys depend on - the particle state and count, the
+// walls, the parameters, the cell grid, the strip exchange - before it changes anything.  If the last force kernel
+// already ran the next tick's key pass (next_keyed), its work is taken back: positions from before its hard-wall fix,
+// counts and the next tick's wall set zeroed (one launch).  The next tick then runs its own pre-pass, and its force
+// kernel computes no keys for the tick after (keys_dropped): a scene that changes its walls every tick (a moving
+// paddle) would otherwise pay for keys and their clearing every tick only to throw them away.
+static int drop_keys(sc_ctx *ctx) {
+    ctx->keys_dropped = true;
+    if (!ctx->next_keyed) return 0;
+    ctx->next_keyed = false;
+    const int q = ctx->par ^ 1;
+    CKR(launch_clear(ctx, q, nullptr, KeyRestore{ctx->pos_cur, ctx->wall_slot_cur, ctx->wall_pre_buf[q]}));
+    ctx->next_clean = true;
+    return 0;
+}
+
 extern "C" int sc_version(void) { return 1; }
 
 extern "C" const char *sc_last_error(const sc_ctx *ctx) { return ctx ? ctx->err.c_str() : g_create_error.c_str(); }
@@ -324,7 +359,7 @@ extern "C" int sc_create(int device, int precision, int64_t capacity, void *stre
     rc |= dev_alloc(c, (char **)&c->vel_cur, n * 2 * rs); rc |= dev_alloc(c, (char **)&c->vel_srt, n * 2 * rs);
     rc |= dev_alloc(c, &c->uid_cur, n); rc |= dev_alloc(c, &c->uid_srt, n);
     rc |= dev_alloc(c, &c->cell_key, n); rc |= dev_alloc(c, &c->cell_key_srt, n);
-    rc |= dev_alloc(c, &c->slot, n); rc |= dev_alloc(c, &c->tmpidx, n);
+    rc |= dev_alloc(c, &c->tmpidx, n);
     rc |= dev_alloc(c, &c->rel_srt, n);
     if (precision == SC_PRECISION_MIXED) {
         rc |= dev_alloc(c, &c->rec_srt, n);
@@ -341,7 +376,8 @@ extern "C" int sc_create(int device, int precision, int64_t capacity, void *stre
     for (int q = 0; q < 2; ++q) { rc |= dev_alloc(c, &c->wbits_cur[q], n / 32 + 1); rc |= dev_alloc(c, &c->wbits_srt[q], n / 32 + 1); }
     c->wall_bits_cur = c->wbits_cur[0]; c->wall_bits_srt = c->wbits_srt[0];
     rc |= dev_alloc(c, &c->wall_slot_cur, n); rc |= dev_alloc(c, &c->wall_slot_srt, n);
-    rc |= dev_alloc(c, &c->wall_pre, n);
+    rc |= dev_alloc(c, &c->wall_pre_buf[0], n); rc |= dev_alloc(c, &c->wall_pre_buf[1], n);
+    c->wall_pre = c->wall_pre_buf[0];
     rc |= dev_alloc(c, &c->cnt, 1);
     rc |= dev_alloc(c, &c->count_by_rank, n + 1);
     rc |= dev_alloc(c, &c->stage2, n); rc |= dev_alloc(c, &c->stage1, n);
@@ -357,8 +393,8 @@ extern "C" void sc_destroy(sc_ctx *c) {
     cudaSetDevice(c->device);
     cudaStreamSynchronize(c->stream);
     void *ptrs[] = {c->pos_cur, c->pos_srt, c->vel_cur, c->vel_srt, c->uid_cur, c->uid_srt, c->cell_key,
-                    c->cell_key_srt, c->slot, c->tmpidx, c->cell_bufs[0], c->cell_bufs[1], c->bsum, c->bsum2, c->rel_srt, c->rec_srt, c->blk_desc, c->ps, c->pair_j, c->pair_n, c->pair_off, c->pair_cnt,
-                    c->wbits_cur[0], c->wbits_cur[1], c->wbits_srt[0], c->wbits_srt[1], c->wall_slot_cur, c->wall_slot_srt, c->wall_pre, c->cnt,
+                    c->cell_key_srt, c->tmpidx, c->cell_count, c->cell_start, c->bsum, c->bsum2, c->rel_srt, c->rec_srt, c->blk_desc, c->ps, c->pair_j, c->pair_n, c->pair_off, c->pair_cnt,
+                    c->wbits_cur[0], c->wbits_cur[1], c->wbits_srt[0], c->wbits_srt[1], c->wall_slot_cur, c->wall_slot_srt, c->wall_pre_buf[0], c->wall_pre_buf[1], c->cnt,
                     c->rank_of_uid, c->count_by_rank, c->list_sorted, c->noise_dev, c->stage2, c->stage1, c->wire_dummy, c->monitor};
     for (void *p : ptrs) if (p) cudaFree(p);
     for (auto &p : c->pending) { cudaEventDestroy(p.e0); cudaEventDestroy(p.e1); }
@@ -373,6 +409,8 @@ extern "C" int sc_set_params(sc_ctx *ctx, const sc_params *p) {
     if (!(p->particle_radius > 0) || !(p->dt == p->dt)) return fail(ctx, "sc_set_params: particle_radius must be > 0");
     const bool regrid = !ctx->params_set || p->particle_radius != ctx->hp.particle_radius;
     if (regrid && ctx->in_step) return fail(ctx, "sc_set_params: radius change inside a split step");
+    // the same bytes again (a Crate pushes its coefficients every tick) leave the next tick's keys valid
+    if (!ctx->params_set || std::memcmp(p, &ctx->hp, sizeof(sc_params)) != 0) CKR(drop_keys(ctx));
     if (regrid && ctx->params_set) CKR(sync_count(ctx));  // the live count sits in the old cell array's tail
     ctx->hp = *p;
     refresh_dev_params(ctx);
@@ -457,6 +495,16 @@ extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const in
     if (nbodies < 0 || nbodies > SC_MAX_BODIES) return fail(ctx, "sc_set_walls: more than SC_MAX_BODIES bodies");
     if (!ctx->params_set) return fail(ctx, "sc_set_walls: call sc_set_params first (padding needs the radius)");
     WallParams &w = ctx->walls;
+    {   // the same walls again (a Crate pushes them every tick) leave the next tick's keys valid; moving ones do not
+        bool same = ctx->walls_set && S == w.S && nbodies == w.nbodies &&
+                    (S == 0 || std::memcmp(&w.seg[0][0], segments, sizeof(double) * 4 * (size_t)S) == 0);
+        int k = 0;
+        for (int b = 0; same && b < nbodies; ++b) {
+            same = std::memcmp(w.kin[b], body_kin + 5 * b, sizeof(double) * 5) == 0;
+            for (int q = 0; same && q < body_len[b]; ++q, ++k) same = k < S && w.seg_body[k] == b;
+        }
+        if (!same || k != S) CKR(drop_keys(ctx));
+    }
     w.S = S; w.nbodies = nbodies;
     int k = 0;
     for (int b = 0; b < nbodies; ++b) {
@@ -536,6 +584,7 @@ static int upload_particles(sc_ctx *ctx, const double *pos, const double *vel, i
 
 extern "C" int sc_set_state(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
     CKR(enter(ctx, "sc_set_state"));
+    CKR(drop_keys(ctx));
     if (n < 0 || n > ctx->cap) return fail(ctx, "sc_set_state: n exceeds capacity");
     if (ctx->in_step) return fail(ctx, "sc_set_state: inside a split step");
     ctx->next_uid = 0;
@@ -564,6 +613,7 @@ extern "C" int sc_set_state_uids(sc_ctx *ctx, const double *pos, const double *v
 
 extern "C" int sc_append_particles(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
     CKR(enter(ctx, "sc_append_particles"));
+    CKR(drop_keys(ctx));
     if (ctx->in_step) return fail(ctx, "sc_append_particles: inside a split step");
     if (n < 0) return fail(ctx, "sc_append_particles: n < 0");
     CKR(sync_count(ctx));
@@ -600,6 +650,7 @@ extern "C" int sc_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsou
         total += S.n;
     }
     if (!E.nsrc) return 0;
+    CKR(drop_keys(ctx));  // the new particles have no keys
     if ((uint64_t)ctx->next_uid + total >= (uint64_t)SC_GHOST_BIT)
         return fail(ctx, "particle identities exhausted (2^31 particles created in this context)");
     refresh_count(ctx);
@@ -642,10 +693,11 @@ extern "C" int sc_particle_count(sc_ctx *ctx, int64_t *n) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// In-place exclusive scan of a[0..n), total to a[n].  `pre_cleared`: the descriptors were zeroed by k_begin_tick.
-static int exclusive_scan(sc_ctx *ctx, uint32_t *a, uint32_t n, int slot, bool pre_cleared = false) {
+// Exclusive scan of in[0..n) to out[0..n), total to out[n] (in == out: in place).  `pre_cleared`: the descriptors were
+// zeroed by k_begin_tick / the last force kernel.
+static int exclusive_scan(sc_ctx *ctx, const uint32_t *in, uint32_t *out, uint32_t n, int slot, bool pre_cleared = false) {
     const unsigned nb = (n + SC_SCAN_TILE - 1) / SC_SCAN_TILE;
-    if (nb == 0) { CK(cudaMemsetAsync(a, 0, sizeof(uint32_t), ctx->stream)); return 0; }
+    if (nb == 0) { CK(cudaMemsetAsync(out, 0, sizeof(uint32_t), ctx->stream)); return 0; }
     // the cell scan's descriptors (bsum) are kept zeroed from tick to tick by the force kernel; every other scan uses
     // its own set and zeroes it here
     unsigned long long *&desc = pre_cleared ? ctx->bsum : ctx->bsum2;
@@ -659,7 +711,7 @@ static int exclusive_scan(sc_ctx *ctx, uint32_t *a, uint32_t n, int slot, bool p
     }
     if (!pre_cleared) CK(cudaMemsetAsync(desc, 0, sizeof(unsigned long long) * ((size_t)nb + 1), ctx->stream));
     ProfScope ps(ctx, slot);
-    CK(launch_pdl(k_scan_lookback, dim3(nb), dim3(SC_SCAN_THREADS), ctx->stream, a, n, desc + 1, (uint32_t *)desc));
+    CK(launch_pdl(k_scan_lookback, dim3(nb), dim3(SC_SCAN_THREADS), ctx->stream, in, out, n, desc + 1, (uint32_t *)desc));
     return 0;
 }
 
@@ -679,7 +731,7 @@ static int build_rank_map(sc_ctx *ctx, const uint32_t *uid, const uint32_t *n_pt
         ProfScope ps(ctx, SLOT_RANKMAP);
         k_mark_alive<<<blocks_for(ctx->n_host), SC_BLOCK, 0, ctx->stream>>>(n_ptr, uid, ctx->rank_of_uid);
     }
-    CKR(exclusive_scan(ctx, ctx->rank_of_uid, ctx->next_uid, SLOT_RANKMAP));
+    CKR(exclusive_scan(ctx, ctx->rank_of_uid, ctx->rank_of_uid, ctx->next_uid, SLOT_RANKMAP));
     return 0;
 }
 
@@ -689,26 +741,28 @@ static int require_ready(sc_ctx *ctx, const char *who, bool consumes_unpack = fa
     return 0;
 }
 
+// where the key pass of a tick of parity `q` writes (key_particle, sc_common.cuh)
+static KeyOut key_out(sc_ctx *ctx, int q) {
+    return KeyOut{ctx->cell_key, ctx->cell_count, ctx->wbits_cur[q], ctx->wall_slot_cur, &ctx->cnt->n_wall[q],
+                  ctx->pos_cur, ctx->wall_pre_buf[q]};
+}
+
 // remove -> walls -> keys -> sort -> gather
 template <bool kStep> static int enqueue_search(sc_ctx *ctx) {
     const int64_t n = ctx->n_host;
     const Grid &g = ctx->grid;
-    // this tick's buffer set: the one the previous tick's force kernel cleared
+    // this tick's wall set: the one the previous tick's density kernel cleared (and its force kernel may have filled)
     ctx->par ^= 1;
-    ctx->cell_start = ctx->cell_bufs[ctx->par];
     ctx->wall_bits_cur = ctx->wbits_cur[ctx->par];
     ctx->wall_bits_srt = ctx->wbits_srt[ctx->par];
-    if (!ctx->next_clean) {  // cold start: first tick of the context / first after the grid was rebuilt
-        ProfScope ps(ctx, SLOT_CLEAR);
-        const uint32_t words = (uint32_t)(ctx->cap / 32 + 1);
-        const unsigned nb = (unsigned)std::min<int64_t>(((int64_t)g.ncells / 4 + SC_BLOCK - 1) / SC_BLOCK + 1, 148 * 16);
-        const uint32_t scan_words = (g.ncells + SC_SCAN_TILE - 1) / SC_SCAN_TILE + 1;  // ticket + descriptors
-        CK(launch_pdl(k_begin_tick, dim3(nb), dim3(SC_BLOCK), ctx->stream, ctx->cnt, ctx->cell_start, g.ncells,
-                      ctx->carry_count ? 1 : 0, ctx->wall_bits_cur, ctx->wall_bits_srt, words, ctx->bsum, scan_words,
-                      (uint32_t)ctx->cap));
+    ctx->wall_pre = ctx->wall_pre_buf[ctx->par];
+    const bool keyed = kStep && ctx->next_keyed;  // the previous tick's force kernel did this tick's pre-pass
+    if (!ctx->next_clean && !keyed) {  // cold start: first tick of the context / first after the grid was rebuilt
+        CKR(launch_clear(ctx, ctx->par, ctx->carry_count ? ctx->cell_start + g.ncells : nullptr, KeyRestore{}));
         ctx->carry_count = false;
     }
     ctx->next_clean = false;
+    ctx->next_keyed = false;
     // strips: a recorded (deferred) unpack is carried out by the pre-pass itself (PrepassUnpack, sc_common.cuh)
     PrepassUnpack U{};
     if (ctx->pend.on) {
@@ -722,32 +776,31 @@ template <bool kStep> static int enqueue_search(sc_ctx *ctx) {
         if (!U.lo.hdr && !U.hi.hdr) U.on = 0;
         ctx->pend.on = false;
     }
-    if (n > 0) {
+    if (n > 0 && !keyed) {
         ProfScope ps(ctx, SLOT_PREPASS);
         auto go = [&](auto kernel) {
             return launch_pdl(kernel, dim3(blocks_for((n + SC_PREPASS_ILP - 1) / SC_PREPASS_ILP)), dim3(SC_BLOCK),
-                              ctx->stream, ctx->cnt, g, ctx->dp, ctx->walls, ctx->pos_cur, ctx->cell_key, ctx->slot,
-                              ctx->cell_start, ctx->wall_bits_cur, ctx->wall_slot_cur, ctx->wall_pre, (uint32_t)ctx->cap, U);
+                              ctx->stream, ctx->cnt, g, ctx->dp, ctx->walls, key_out(ctx, ctx->par), (uint32_t)ctx->cap, U);
         };
         CK(U.on ? go(k_prepass<kStep, true>) : go(k_prepass<kStep, false>));
     }
-    CKR(exclusive_scan(ctx, ctx->cell_start, g.ncells, SLOT_SCAN, true));
+    CKR(exclusive_scan(ctx, ctx->cell_count, ctx->cell_start, g.ncells, SLOT_SCAN, true));
     if (n > 0) {
         {
             ProfScope ps(ctx, SLOT_PLACE);
             CK(launch_pdl(k_place, dim3(blocks_for((n + SC_PLACE_ILP - 1) / SC_PLACE_ILP)), dim3(SC_BLOCK), ctx->stream,
-                          (const Counters *)ctx->cnt, (const uint32_t *)ctx->cell_key, (const uint32_t *)ctx->slot,
+                          (const Counters *)ctx->cnt, (const uint32_t *)ctx->cell_key, ctx->cell_count,
                           (const uint32_t *)ctx->cell_start, ctx->tmpidx, (uint32_t)ctx->cap));
         }
         ProfScope ps(ctx, SLOT_RANK_GATHER);
         if (ctx->precision == SC_PRECISION_F64)
             CK(launch_pdl(k_rank_gather<double>, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream,
-                g, ctx->cell_start, ctx->tmpidx, ctx->cell_key, ctx->pos_cur, (const double2 *)ctx->vel_cur,
+                ctx->cnt, g, ctx->cell_start, ctx->tmpidx, ctx->cell_key, ctx->pos_cur, (const double2 *)ctx->vel_cur,
                 ctx->uid_cur, ctx->wall_bits_cur, ctx->wall_slot_cur, ctx->pos_srt, ctx->rel_srt, (double2 *)ctx->vel_srt,
                 ctx->uid_srt, ctx->cell_key_srt, ctx->wall_bits_srt, ctx->wall_slot_srt, (float4 *)nullptr, (BlockDesc *)nullptr));
         else
             CK(launch_pdl(k_rank_gather<float>, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream,
-                g, ctx->cell_start, ctx->tmpidx, ctx->cell_key, ctx->pos_cur, (const float2 *)ctx->vel_cur,
+                ctx->cnt, g, ctx->cell_start, ctx->tmpidx, ctx->cell_key, ctx->pos_cur, (const float2 *)ctx->vel_cur,
                 ctx->uid_cur, ctx->wall_bits_cur, ctx->wall_slot_cur, ctx->pos_srt, ctx->rel_srt, (float2 *)ctx->vel_srt,
                 ctx->uid_srt, ctx->cell_key_srt, ctx->wall_bits_srt, ctx->wall_slot_srt, ctx->rec_srt, ctx->blk_desc));
     }
@@ -782,6 +835,12 @@ static int enqueue_count(sc_ctx *ctx, const uint32_t *uid, bool want_lists) {
     return 0;
 }
 
+// what this tick's density kernel clears for the next tick (NextWallClear, sc_common.cuh)
+static NextWallClear next_wall_clear(sc_ctx *ctx) {
+    const int o = ctx->par ^ 1;
+    return NextWallClear{ctx->wbits_cur[o], ctx->wbits_srt[o], (uint32_t)(ctx->cap / 32 + 1), &ctx->cnt->n_wall[o]};
+}
+
 template <typename Real>
 static int launch_density(sc_ctx *ctx, const Grid &g, const DevParams &dp, const uint32_t *noise_off, int64_t n) {
     typedef typename Vec2<Real>::type R2;
@@ -789,7 +848,7 @@ static int launch_density(sc_ctx *ctx, const Grid &g, const DevParams &dp, const
         return launch_pdl(kernel, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream, ctx->cnt, g, dp, ctx->cell_start,
                           ctx->pos_srt, ctx->rel_srt, ctx->cell_key_srt, ctx->uid_srt, ctx->noise_dev, noise_off,
                           ctx->rank_of_uid, ctx->pair_j, (R2 *)ctx->pair_n, ctx->pair_off, ctx->pair_cnt,
-                          (PS<Real> *)ctx->ps);
+                          (PS<Real> *)ctx->ps, next_wall_clear(ctx));
     };
     cudaError_t e;
     if (dp.noise_mode == SC_NOISE_HOST) e = go(k_density<Real, SC_NOISE_HOST>);
@@ -799,19 +858,23 @@ static int launch_density(sc_ctx *ctx, const Grid &g, const DevParams &dp, const
     return 0;
 }
 
-// what this tick's force kernel clears for the next tick (TickDuty, sc_common.cuh)
+// what this tick's force kernel does for the next tick (TickDuty, sc_common.cuh), and the next tick's key pass when
+// `keys` (NextKeys, sc_pair.cuh)
 static TickDuty tick_duty(sc_ctx *ctx) {
     TickDuty d;
-    const int o = ctx->par ^ 1;
-    d.cells = ctx->cell_bufs[o]; d.ncells = ctx->grid.ncells;
-    d.bits_a = ctx->wbits_cur[o]; d.bits_b = ctx->wbits_srt[o]; d.nbits = (uint32_t)(ctx->cap / 32 + 1);
     d.scan_desc = ctx->bsum; d.scan_words = (ctx->grid.ncells + SC_SCAN_TILE - 1) / SC_SCAN_TILE + 1;
     d.cnt = ctx->cnt;
     return d;
 }
+static NextKeys next_keys(sc_ctx *ctx, bool keys) {
+    NextKeys k{};
+    k.g = ctx->grid;
+    if (keys) k.out = key_out(ctx, ctx->par ^ 1);
+    return k;
+}
 
 template <typename Real>
-static int launch_force(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n) {
+static int launch_force(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n, bool keys) {
     typedef typename Vec2<Real>::type R2;
     if (ctx->monitor_on) CK(cudaMemsetAsync(ctx->monitor, 0, sizeof(double) * 8, ctx->stream));
     ProfScope ps(ctx, SLOT_FORCE);
@@ -822,21 +885,22 @@ static int launch_force(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr,
         return launch_pdl(kernel, dim3(nb), dim3(nt), ctx->stream, n_ptr, dp, ctx->walls, ctx->pos_srt,
                           (const R2 *)ctx->vel_srt, ctx->pair_j, (const R2 *)ctx->pair_n, ctx->pair_off, ctx->pair_cnt,
                           (const PS<Real> *)ctx->ps, ctx->wall_bits_srt, ctx->wall_slot_srt, ctx->wall_pre,
-                          ctx->pos_cur, (R2 *)ctx->vel_cur, ctx->monitor, tick_duty(ctx));
+                          ctx->pos_cur, (R2 *)ctx->vel_cur, ctx->monitor, tick_duty(ctx), next_keys(ctx, keys));
     };
     CK(ctx->monitor_on ? go(k_force<Real, true>) : go(k_force<Real, false>));
     return 0;
 }
 
 // mixed precision with device-side noise: K5 on the same blocks and windows as K4 (sc_tile.cuh)
-static int launch_force_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n) {
+static int launch_force_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n, bool keys) {
     if (ctx->monitor_on) CK(cudaMemsetAsync(ctx->monitor, 0, sizeof(double) * 8, ctx->stream));
     ProfScope ps(ctx, SLOT_FORCE);
     auto go = [&](auto kernel) {
         return launch_pdl(kernel, dim3((unsigned)((n + SC_TILE - 1) / SC_TILE)), dim3(SC_TILE), ctx->stream, n_ptr, dp,
                           ctx->walls, ctx->blk_desc, ctx->pos_srt, (const float2 *)ctx->vel_srt, (const uint2 *)ctx->pair_n,
                           ctx->pair_cnt, (const PS<float> *)ctx->ps, ctx->wall_bits_srt, ctx->wall_slot_srt,
-                          ctx->wall_pre, ctx->pos_cur, (float2 *)ctx->vel_cur, ctx->monitor, tick_duty(ctx));
+                          ctx->wall_pre, ctx->pos_cur, (float2 *)ctx->vel_cur, ctx->monitor, tick_duty(ctx),
+                          next_keys(ctx, keys));
     };
     CK(ctx->monitor_on ? go(k_force_tile<true>) : go(k_force_tile<false>));
     return 0;
@@ -847,7 +911,7 @@ static int launch_density_tile(sc_ctx *ctx, const Grid &g, const DevParams &dp, 
     auto go = [&](auto kernel) {
         return launch_pdl(kernel, dim3((unsigned)((n + SC_TILE - 1) / SC_TILE)), dim3(SC_TILE), ctx->stream, ctx->cnt, g, dp,
                           ctx->cell_start, ctx->blk_desc, ctx->pos_srt, ctx->rec_srt, ctx->cell_key_srt, (uint2 *)ctx->pair_n,
-                          ctx->pair_cnt, (PS<float> *)ctx->ps);
+                          ctx->pair_cnt, (PS<float> *)ctx->ps, next_wall_clear(ctx));
     };
     CK(dp.noise_mode == SC_NOISE_COUNTER ? go(k_density_tile<SC_NOISE_COUNTER>) : go(k_density_tile<SC_NOISE_NONE>));
     return 0;
@@ -861,29 +925,34 @@ static int enqueue_forces(sc_ctx *ctx, const uint32_t *noise_off) {
                                                                                              : ctx->noise_mode;
     dp.tick_key = tick_key(ctx->seed, ctx->tick);
     const uint32_t *n_ptr = ctx->cell_start + g.ncells;
+    // the force kernel runs the next tick's key pass (NextKeys) unless a call since the last step changed what the keys
+    // depend on (drop_keys) or this is a strip, whose exchange changes the particle set between the ticks
+    const bool keys = n > 0 && !ctx->keys_dropped && !ctx->dist_on;
     if (n > 0) {
         if (ctx->precision == SC_PRECISION_F64) {
             {
                 ProfScope ps(ctx, SLOT_DENSITY);
                 CKR(launch_density<double>(ctx, g, dp, noise_off, n));
             }
-            CKR(launch_force<double>(ctx, dp, n_ptr, n));
+            CKR(launch_force<double>(ctx, dp, n_ptr, n, keys));
         } else if (dp.noise_mode == SC_NOISE_HOST || (ctx->pair_mode == 0)) {
             {
                 ProfScope ps(ctx, SLOT_DENSITY);
                 CKR(launch_density<float>(ctx, g, dp, noise_off, n));
             }
-            CKR(launch_force<float>(ctx, dp, n_ptr, n));
+            CKR(launch_force<float>(ctx, dp, n_ptr, n, keys));
         } else {
             {
                 ProfScope ps(ctx, SLOT_DENSITY);
                 CKR(launch_density_tile(ctx, g, dp, n));
             }
-            CKR(launch_force_tile(ctx, dp, n_ptr, n));
+            CKR(launch_force_tile(ctx, dp, n_ptr, n, keys));
         }
     }
-    if (n > 0) { ctx->next_clean = true; ctx->carry_count = false; }  // the force kernel carried the count and cleared the other set
+    // the force kernel carried the count; the density kernel cleared the next tick's wall set, k_place the counts
+    if (n > 0) { ctx->next_clean = !keys; ctx->next_keyed = keys; ctx->carry_count = false; }
     else ctx->carry_count = true;  // nothing ran: cnt->n is refreshed by the next cold start or by sync_count
+    ctx->keys_dropped = false;
     CK(cudaGetLastError());
     // the new state (pos_cur, vel_cur) is in this tick's sorted order, whose uids are uid_srt
     uint32_t *t = ctx->uid_cur; ctx->uid_cur = ctx->uid_srt; ctx->uid_srt = t;
@@ -942,7 +1011,7 @@ extern "C" int sc_step_finish(sc_ctx *ctx, const double *noise) {
         }
         if (need) CK(cudaMemcpyAsync(ctx->noise_dev, noise, sizeof(double) * need, cudaMemcpyHostToDevice, ctx->stream));
         // CSR offsets in original index order (crate.py:165: `for particle_index in range(self.particle_count)`)
-        CKR(exclusive_scan(ctx, ctx->count_by_rank, (uint32_t)ctx->n_host, SLOT_COUNT));
+        CKR(exclusive_scan(ctx, ctx->count_by_rank, ctx->count_by_rank, (uint32_t)ctx->n_host, SLOT_COUNT));
         noise_off = ctx->count_by_rank;
         ctx->lists_valid = false;
     }
@@ -992,8 +1061,11 @@ extern "C" int sc_get_state(sc_ctx *ctx, double *pos, double *vel, double *press
     const uint32_t *n_ptr = &ctx->cnt->n;
     const unsigned nb = blocks_for(n);
     if (pos) {
+        const int q = ctx->par ^ 1;  // the wall set the next tick's key pass filled, if it ran (next_keyed)
         { ProfScope ps(ctx, SLOT_IO);
-          k_scatter_vec2<double2><<<nb, SC_BLOCK, 0, ctx->stream>>>(n_ptr, ctx->uid_cur, ctx->rank_of_uid, ctx->pos_cur, ctx->stage2); }
+          k_scatter_pos<<<nb, SC_BLOCK, 0, ctx->stream>>>(n_ptr, ctx->uid_cur, ctx->rank_of_uid, ctx->pos_cur,
+                                                          ctx->next_keyed ? ctx->wbits_cur[q] : nullptr, ctx->wall_slot_cur,
+                                                          ctx->wall_pre_buf[q], ctx->stage2); }
         CK(cudaMemcpyAsync(pos, ctx->stage2, sizeof(double2) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     }
     if (vel) {
@@ -1219,6 +1291,7 @@ extern "C" int sc_last_pair_count(sc_ctx *ctx, int64_t *n_pairs) {
 extern "C" double sc_debug_rerun(sc_ctx *ctx, int which, int reps) {
     if (!ctx || !ctx->srt_valid) return -1.0;
     cudaSetDevice(ctx->device);
+    if (drop_keys(ctx)) return -1.0;  // the force kernel re-run below computes no keys, and its own must not be counted twice
     DevParams dp = ctx->dp;
     dp.noise_mode = ctx->noise_mode;
     dp.tick_key = tick_key(ctx->seed, ctx->tick - 1);
@@ -1231,8 +1304,8 @@ extern "C" double sc_debug_rerun(sc_ctx *ctx, int which, int reps) {
         cudaEventRecord(e0, ctx->stream);
         const bool tiled = ctx->pair_mode != 0 && dp.noise_mode != SC_NOISE_HOST;
         if (which == 4) { if (tiled) launch_density_tile(ctx, ctx->grid, dp, n); else launch_density<float>(ctx, ctx->grid, dp, nullptr, n); }
-        else if (tiled) launch_force_tile(ctx, dp, ctx->cell_start + ctx->grid.ncells, n);
-        else launch_force<float>(ctx, dp, ctx->cell_start + ctx->grid.ncells, n);
+        else if (tiled) launch_force_tile(ctx, dp, ctx->cell_start + ctx->grid.ncells, n, false);
+        else launch_force<float>(ctx, dp, ctx->cell_start + ctx->grid.ncells, n, false);
         cudaEventRecord(e1, ctx->stream);
         cudaEventSynchronize(e1);
         float ms = 0;
@@ -1315,6 +1388,7 @@ extern "C" int64_t sc_dist_wire_bytes(int64_t wire_capacity) {
 extern "C" int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_lo, int64_t row_hi, int halo_rows,
                                  int64_t wire_capacity) {
     CKR(enter(ctx, "sc_dist_configure"));
+    CKR(drop_keys(ctx));
     if (nranks < 1 || rank < 0 || rank >= nranks) return fail(ctx, "sc_dist_configure: bad rank");
     if (halo_rows < 1) return fail(ctx, "sc_dist_configure: halo_rows must be >= 1");
     if (wire_capacity < 1 || wire_capacity > ctx->cap) return fail(ctx, "sc_dist_configure: bad wire capacity");
@@ -1340,6 +1414,7 @@ extern "C" int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_
 
 extern "C" int sc_dist_set_rows(sc_ctx *ctx, int64_t row_lo, int64_t row_hi) {
     CKR(dist_ready(ctx, "sc_dist_set_rows"));
+    CKR(drop_keys(ctx));
     if (ctx->dist.has_lo && ctx->dist.has_hi && row_hi - row_lo < 2 * (int64_t)ctx->dist.halo)
         return fail(ctx, "sc_dist_set_rows: a strip must be at least 2 * halo_rows high");
     ctx->dist.row_lo = row_lo; ctx->dist.row_hi = row_hi;
@@ -1402,6 +1477,7 @@ extern "C" int sc_dist_row_histogram(sc_ctx *ctx, int64_t row0, int64_t nrows, u
 static int enqueue_pack(sc_ctx *ctx, const char *who, void *send_lo_dev, void *send_hi_dev, void *peer_recv_lo,
                         void *peer_flag_lo, void *peer_recv_hi, void *peer_flag_hi, bool direct, uint32_t value) {
     CKR(dist_ready(ctx, who));
+    CKR(drop_keys(ctx));
     if ((ctx->dist.has_lo && !send_lo_dev) || (ctx->dist.has_hi && !send_hi_dev))
         return fail(ctx, std::string(who) + ": a neighbor exists but its send buffer is NULL");
     if (direct && ((ctx->dist.has_lo && (!peer_recv_lo || !peer_flag_lo)) || (ctx->dist.has_hi && (!peer_recv_hi || !peer_flag_hi))))
@@ -1473,6 +1549,7 @@ extern "C" int sc_dist_pack_push(sc_ctx *ctx, void *send_lo_dev, void *peer_recv
 // other call off until then.
 static int record_unpack(sc_ctx *ctx, const void *recv_lo, const void *flag_lo, const void *recv_hi, const void *flag_hi,
                          uint32_t value) {
+    CKR(drop_keys(ctx));
     ctx->pend.on = true;
     ctx->pend.recv_lo = recv_lo; ctx->pend.flag_lo = flag_lo; ctx->pend.recv_hi = recv_hi; ctx->pend.flag_hi = flag_hi;
     ctx->pend.value = value;

@@ -118,7 +118,8 @@ struct Counters {
     uint32_t n;          // live particles at the start of the tick (= after the previous tick's removal)
     uint32_t n_split;    // strips: the count before the neighbors' records were appended (k_dist_pack) = where the
                          // second, small wall / key pass of the tick starts (see enqueue_search)
-    uint32_t n_wall;     // particles touching a wall this tick
+    uint32_t n_wall[2];  // particles touching a wall, per tick parity (the force kernel of one tick may already fill
+                         // the next tick's list while this tick's is being read, see NextKeys)
     uint32_t n_pairs;    // sum K_i (filled by the count kernel)
     uint32_t overflow;   // capacity problems seen on the device
     uint32_t pair_cursor;  // next free record of the pair buffer (bump allocator, reset every tick)
@@ -127,24 +128,28 @@ struct Counters {
 };
 
 // What the tick's LAST kernel (the force kernel) does for the NEXT tick, spread over its threads, so that a tick does
-// not open with a clearing launch: zero the other cell-count grid and the other pair of wall bitmaps (both are double
-// buffered by tick parity: this tick's are still being read), zero the cell scan's tile descriptors and ticket, carry
-// the live count (the scan total) into cnt->n and reset the wall side list.
+// not open with a clearing launch: zero the cell scan's tile descriptors and ticket and carry the live count (the scan
+// total) into cnt->n.  The cell-count grid needs no clearing: k_place takes every count back to zero.
 struct TickDuty {
-    uint32_t *cells; uint32_t ncells;            // next tick's cell-count grid
-    uint32_t *bits_a, *bits_b; uint32_t nbits;   // next tick's wall bitmaps (words)
     unsigned long long *scan_desc; uint32_t scan_words;
     Counters *cnt;
 };
 __device__ __forceinline__ void end_of_tick(const TickDuty &D, const uint32_t *n_ptr) {
     const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, nth = gridDim.x * blockDim.x;
-    uint4 *c4 = reinterpret_cast<uint4 *>(D.cells);
-    const uint32_t n4 = D.ncells / 4;
-    for (uint32_t i = tid; i < n4; i += nth) c4[i] = make_uint4(0, 0, 0, 0);
-    for (uint32_t i = n4 * 4 + tid; i < D.ncells; i += nth) D.cells[i] = 0;
-    for (uint32_t i = tid; i < D.nbits; i += nth) { D.bits_a[i] = 0; D.bits_b[i] = 0; }
     for (uint32_t i = tid; i < D.scan_words; i += nth) D.scan_desc[i] = 0ull;
-    if (tid == 0) { D.cnt->n = *n_ptr; D.cnt->n_wall = 0; }
+    if (tid == 0) D.cnt->n = *n_ptr;
+}
+
+// What the density kernel (K4) clears for the NEXT tick: the wall bitmaps and the wall side-list counter of the other
+// tick parity.  Not the force kernel: when it computes the next tick's keys (NextKeys) it writes into exactly these.
+struct NextWallClear {
+    uint32_t *bits_a, *bits_b; uint32_t nbits;   // next tick's wall bitmaps (words)
+    uint32_t *n_wall;                            // next tick's wall side-list counter
+};
+__device__ __forceinline__ void clear_next_walls(const NextWallClear &C) {
+    const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, nth = gridDim.x * blockDim.x;
+    for (uint32_t i = tid; i < C.nbits; i += nth) { C.bits_a[i] = 0; C.bits_b[i] = 0; }
+    if (tid == 0) *C.n_wall = 0;
 }
 
 // ---- counter-based pair noise (the production definition; oracle/step_oracle.c restates it) -------------
@@ -236,6 +241,70 @@ __device__ inline uint32_t cell_of(const Grid &g, double x, double y, int &row_o
     cr = cr < 1 ? 1 : (cr > g.nrows - 2 ? g.nrows - 2 : cr);
     cc = cc < 1 ? 1 : (cc > g.ncols - 2 ? g.ncols - 2 : cc);
     return (uint32_t)cr * (uint32_t)g.ncols + (uint32_t)cc;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// K0 + K1 for ONE particle: the work of a tick's pre-pass, run either by k_prepass (sc_sort.cuh) or, for the next
+// tick, by the previous tick's force kernel on the position it has just integrated (force_tail, sc_pair.cuh; see
+// NextKeys).  One routine, so the two paths give the same bits.
+//   kStep = true : remove_particles (crate.py:149-159), calc_virtual_colliders + apply_hard_wall_fix
+//                  (crate.py:213-243, 202-211), then the cell key
+//   kStep = false: cell key only (standalone detect_particle_collisions)
+// Writes cell_key[i] (SC_INVALID_CELL for a removed particle), adds one to the particle's cell count (no value comes
+// back: where a particle goes inside its cell is claimed later, by k_place), and for a particle the wall fix moves:
+// its new position to pos[i], the old one to the wall side list, its slot there and its wall bit.
+// INVARIANT: the particles counted here are exactly the particles k_place places - index below the clamped live count,
+// key valid - because k_place takes each count back down to zero with one decrement per particle it places.  A count
+// left above zero would shift every later cell of the next tick's scan.
+struct KeyOut {
+    uint32_t *cell_key, *cell_count;
+    uint32_t *wall_bits, *wall_slot, *n_wall;
+    double2 *pos, *wall_pre;
+};
+template <bool kStep>
+__device__ __forceinline__ void key_particle(const Grid &g, const DevParams &P, const WallParams &W, const KeyOut &O,
+                                             uint32_t i, double2 p) {
+    if (kStep) {
+        const bool out = (p.x < P.box_lo) | (p.x > P.box_hi) | (p.y < P.box_lo) | (p.y > P.box_hi);
+        if (out) {
+            O.cell_key[i] = SC_INVALID_CELL;
+            return;
+        }
+        // one test for the bulk of the liquid: inside a rectangle that no segment's touch zone reaches
+        const bool clear = p.x > W.safe_contact[0] && p.x < W.safe_contact[1] &&
+                           p.y > W.safe_contact[2] && p.y < W.safe_contact[3];
+        if (!clear) {
+            int V = 0;
+            double sx = 0, sy = 0;
+            for (int q = 0; q < W.S; ++q) {
+                if (p.x < W.seg_box[q][0] || p.x > W.seg_box[q][1] || p.y < W.seg_box[q][2] || p.y > W.seg_box[q][3])
+                    continue;  // cannot be within the touch distance of this segment
+                double cx, cy;
+                const double dist = point_segment(p.x, p.y, W.seg[q][0], W.seg[q][1], W.seg[q][2], W.seg[q][3], cx, cy);
+                if (dist <= P.touch) {
+                    const double vcx = (p.x - cx) * 2, vcy = (p.y - cy) * 2;  // crate.py:234
+                    double rel = P.r / sqrt(vcx * vcx + vcy * vcy);          // crate.py:206
+                    if (rel < 0.5) rel = 0.5;
+                    const double ex = vcx * (rel - 0.5), ey = vcy * (rel - 0.5);
+                    if (V == 0) { sx = ex; sy = ey; } else { sx += ex; sy += ey; }
+                    ++V;
+                }
+            }
+            if (V > 0) {
+                const uint32_t ws = atomicAdd(O.n_wall, 1u);
+                O.wall_pre[ws] = p;  // contacts are re-derived from this position by the force kernel
+                O.wall_slot[i] = ws;
+                atomicOr(&O.wall_bits[i >> 5], 1u << (i & 31));
+                p.x += sx;
+                p.y += sy;
+                O.pos[i] = p;
+            }
+        }
+    }
+    int row;
+    const uint32_t c = cell_of(g, p.x, p.y, row);
+    atomicAdd(&O.cell_count[c], 1u);  // result unused: a fire-and-forget reduction (RED), no round trip
+    O.cell_key[i] = c;
 }
 
 // total order used inside a cell: x ascending (NaN last, like np.lexsort), ties by uid (lexsort is stable and

@@ -261,8 +261,9 @@ k_density(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
           const uint32_t *uid, const double *host_noise,
           const uint32_t *noise_off, const uint32_t *rank_of_uid,
           uint32_t *pair_j, typename Vec2<Real>::type *pair_n,
-          uint32_t *pair_off, uint8_t *pair_cnt, PS<Real> *ps_out) {
+          uint32_t *pair_off, uint8_t *pair_cnt, PS<Real> *ps_out, NextWallClear next) {
     pdl_enter();
+    clear_next_walls(next);
     __shared__ uint32_t s_list[SC_MAX_NEIGHBORS * SC_BLOCK];
     const uint32_t n = cell_start[g.ncells];
     const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
@@ -331,8 +332,17 @@ k_density(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
     ps_out[s] = o;
 }
 
+// NextKeys: K5 is the tick's last kernel and writes the new position of sorted particle s to pos_out[s]; the next tick's
+// pre-pass would read that same array at that same index (the state is kept in the last tick's sorted order).  So K5 can
+// run the next tick's key pass (key_particle) on the position it holds in registers, and the next tick goes straight to
+// the cell scan.  `keys.cell_count == NULL`: not this tick (the host decides, see enqueue_forces).  What the pass writes
+// belongs to the NEXT tick and none of it is read by K5: cell_key, wall_slot_cur and pos_cur are outputs only, and the
+// wall bitmap, side list and its counter are the other tick parity's, which K4 cleared.
+struct NextKeys { Grid g; KeyOut out; };
+
 // Everything of K5 that follows the pair loop, for particle s: wall contact rows of F5, F3-F6 velocity updates, wall
-// bounce, continuous collision, integration.  `visc(vx, vy, ax, ay)` supplies sum_j (v_j - v) (crate.py:319-323).
+// bounce, continuous collision, integration, and the next tick's key pass.  `visc(vx, vy, ax, ay)` supplies
+// sum_j (v_j - v) (crate.py:319-323).
 template <typename Real, bool kMonitor, typename ViscFn>
 __device__ __forceinline__ void force_tail(uint32_t s, int K, Real p_i, Real tx, Real ty, Real qx, Real qy,
                                            const DevParams &P, const WallParams &W, const double2 ps,
@@ -341,8 +351,12 @@ __device__ __forceinline__ void force_tail(uint32_t s, int K, Real p_i, Real tx,
                                            const double2 *wall_pre, double2 *pos_out,
                                            typename Vec2<Real>::type *vel_out,
                                            double *monitor, const uint32_t *n_ptr,
-                                           ViscFn visc) {
+                                           const NextKeys &nk, ViscFn visc) {
     typedef typename Vec2<Real>::type R2;
+    auto store_pos = [&](double2 po) {
+        pos_out[s] = po;
+        if (nk.out.cell_count) key_particle<true>(nk.g, P, W, nk.out, s, po);
+    };
     double mon[6] = {0, 0, 0, 0, 0, 0};
     double mpx = 0, mpy = 0;  // velocity before the current stage
     auto stage = [&](int q, double cx, double cy) {
@@ -425,7 +439,7 @@ __device__ __forceinline__ void force_tail(uint32_t s, int K, Real p_i, Real tx,
         R2 vq;
         vq.x = vx; vq.y = vy;
         vel_out[s] = vq;
-        pos_out[s] = make_double2(ps.x + P.dt * (double)vq.x, ps.y + P.dt * (double)vq.y);   // I, crate.py:361
+        store_pos(make_double2(ps.x + P.dt * (double)vq.x, ps.y + P.dt * (double)vq.y));      // I, crate.py:361
         return;
     }
     double dvx = (double)vx, dvy = (double)vy;
@@ -482,7 +496,7 @@ __device__ __forceinline__ void force_tail(uint32_t s, int K, Real p_i, Real tx,
     double2 po;                                                          // I, crate.py:361
     po.x = ps.x + P.dt * (double)vo.x;
     po.y = ps.y + P.dt * (double)vo.y;
-    pos_out[s] = po;
+    store_pos(po);
 }
 
 // ------------------------------------------------------------------------------------------------------------
@@ -502,7 +516,7 @@ k_force(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallParams W
         const PS<Real> *ps_in, const uint32_t *wall_bits,
         const uint32_t *wall_slot, const double2 *wall_pre,
         double2 *pos_out, typename Vec2<Real>::type *vel_out,
-        double *monitor, TickDuty duty) {
+        double *monitor, TickDuty duty, NextKeys nk) {
     pdl_enter();
     end_of_tick(duty, n_ptr);
     typedef typename Vec2<Real>::type R2;
@@ -558,7 +572,7 @@ k_force(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallParams W
     const R2 v_own = vel[s];
     const bool touching = (wall_bits[s >> 5] >> (s & 31)) & 1u;
     force_tail<Real, kMonitor>(s, K, p_i, tx, ty, qx, qy, P, W, ps_own, v_own, touching, wall_slot, wall_pre, pos_out, vel_out,
-                               monitor, n_ptr, [&](Real vx, Real vy, Real &ax, Real &ay) {
+                               monitor, n_ptr, nk, [&](Real vx, Real vy, Real &ax, Real &ay) {
         if constexpr (sizeof(Real) == 8) {
             for (int q = 0; q < K; ++q) {
                 const R2 vj = vel[PairIO<Real>::load_index(pair_j, pair_n, (size_t)off + q)];

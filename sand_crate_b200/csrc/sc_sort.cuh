@@ -9,40 +9,33 @@
 namespace sc {
 
 // ------------------------------------------------------------------------------------------------------------
-// K0 + K1.  One thread per particle in the order the previous tick left them (that order is the previous
-// tick's sorted order, so neighbouring threads touch neighbouring cells).
-//   kStep = true : remove_particles (crate.py:149-159), calc_virtual_colliders + apply_hard_wall_fix
-//                  (crate.py:213-243, 202-211), then the cell key
-//   kStep = false: cell key only (standalone detect_particle_collisions)
-// particles per thread: the kernel is a chain of two long-latency operations (position load, histogram atomic), so
+// K0 + K1 (key_particle, sc_common.cuh) as a launch of its own.  One thread per particle in the order the previous tick
+// left them (that order is the previous tick's sorted order, so neighbouring threads touch neighbouring cells).  Runs
+// when the previous tick's force kernel did not already do this work (NextKeys): the first tick, a tick after the host
+// changed the state, the walls or the parameters, and every tick of a strip.
+// particles per thread: the kernel is a chain of long-latency operations (position load, then the stores), so
 // independent chains are interleaved (4 measured the same as 2)
 #ifndef SC_PREPASS_ILP
 #define SC_PREPASS_ILP 2
 #endif
 template <bool kStep, bool kUnpack = false>  // kUnpack: the strip variant that appends the neighbors' records itself
 __global__ void __launch_bounds__(SC_BLOCK, 6)  // the wall path may spill; it is rare
-k_prepass(Counters *cnt, Grid g, DevParams P, const __grid_constant__ WallParams W,
-          double2 *pos, uint32_t *cell_key, uint32_t *slot,
-          uint32_t *cell_count, uint32_t *wall_bits, uint32_t *wall_slot,
-          double2 *wall_pre, uint32_t cap, PrepassUnpack U) {
+k_prepass(Counters *cnt, Grid g, DevParams P, const __grid_constant__ WallParams W, KeyOut O, uint32_t cap,
+          PrepassUnpack U) {
     pdl_enter();
     const uint32_t b0 = blockIdx.x * (SC_BLOCK * SC_PREPASS_ILP);
     const uint32_t i0 = b0 + threadIdx.x;
     // the positions are requested BEFORE the live count is known (any index below the capacity is readable): the count
     // is itself a device-resident value, and waiting for it first put one more memory latency at the head of every thread
     double2 p[SC_PREPASS_ILP];
-    uint32_t c[SC_PREPASS_ILP];
 #pragma unroll
     for (int u = 0; u < SC_PREPASS_ILP; ++u) {
         const uint32_t i = i0 + u * SC_BLOCK;
-        if (i < cap) p[u] = pos[i];
+        if (i < cap) p[u] = O.pos[i];
     }
     // every kernel bounds its indices by the count, so the count itself must never exceed the arrays
     uint32_t n = cnt->n < cap ? cnt->n : cap;
-    if (blockIdx.x == 0 && threadIdx.x == 0) {
-        if (cnt->n > cap) cnt->overflow = 1u;
-        cnt->pair_cursor = 0; cnt->n_untiled = 0;  // consumed by this tick's density kernel
-    }
+    if (blockIdx.x == 0 && threadIdx.x == 0 && cnt->n > cap) cnt->overflow = 1u;
     // strips: the neighbors' records are appended HERE (PrepassUnpack).  n_own = the particles already held; a record's
     // place is a pure function of its position in its buffer (lower neighbor's first), so the order is deterministic.
     uint32_t n_own = n, c_lo = 0u;
@@ -76,7 +69,7 @@ k_prepass(Counters *cnt, Grid g, DevParams P, const __grid_constant__ WallParams
                 const WireRec r = k < c_lo ? reinterpret_cast<const WireRec *>(U.lo.hdr + 1)[k]
                                            : reinterpret_cast<const WireRec *>(U.hi.hdr + 1)[k - c_lo];
                 p[u] = make_double2(r.px, r.py);
-                pos[i] = p[u];
+                O.pos[i] = p[u];
                 if (U.vel_is_f64) reinterpret_cast<double2 *>(U.vel)[i] = make_double2(r.vx, r.vy);
                 else reinterpret_cast<float2 *>(U.vel)[i] = make_float2((float)r.vx, (float)r.vy);
                 U.uid[i] = r.kind == SC_WIRE_HALO ? (r.uid | SC_GHOST_BIT) : r.uid;
@@ -86,63 +79,12 @@ k_prepass(Counters *cnt, Grid g, DevParams P, const __grid_constant__ WallParams
 #pragma unroll
     for (int u = 0; u < SC_PREPASS_ILP; ++u) {
         const uint32_t i = i0 + u * SC_BLOCK;
-        c[u] = SC_INVALID_CELL;
-        if (i >= n) continue;
-        if (kStep) {
-            const bool out = (p[u].x < P.box_lo) | (p[u].x > P.box_hi) | (p[u].y < P.box_lo) | (p[u].y > P.box_hi);
-            if (out) {
-                cell_key[i] = SC_INVALID_CELL;
-                continue;
-            }
-            // one test for the bulk of the liquid: inside a rectangle that no segment's touch zone reaches
-            const bool clear = p[u].x > W.safe_contact[0] && p[u].x < W.safe_contact[1] &&
-                               p[u].y > W.safe_contact[2] && p[u].y < W.safe_contact[3];
-            if (!clear) {
-                int V = 0;
-                double sx = 0, sy = 0;
-                for (int q = 0; q < W.S; ++q) {
-                    if (p[u].x < W.seg_box[q][0] || p[u].x > W.seg_box[q][1] || p[u].y < W.seg_box[q][2] ||
-                        p[u].y > W.seg_box[q][3])
-                        continue;  // cannot be within the touch distance of this segment
-                    double cx, cy;
-                    const double dist = point_segment(p[u].x, p[u].y, W.seg[q][0], W.seg[q][1], W.seg[q][2],
-                                                      W.seg[q][3], cx, cy);
-                    if (dist <= P.touch) {
-                        const double vcx = (p[u].x - cx) * 2, vcy = (p[u].y - cy) * 2;  // crate.py:234
-                        double rel = P.r / sqrt(vcx * vcx + vcy * vcy);                  // crate.py:206
-                        if (rel < 0.5) rel = 0.5;
-                        const double ex = vcx * (rel - 0.5), ey = vcy * (rel - 0.5);
-                        if (V == 0) { sx = ex; sy = ey; } else { sx += ex; sy += ey; }
-                        ++V;
-                    }
-                }
-                if (V > 0) {
-                    const uint32_t ws = atomicAdd(&cnt->n_wall, 1u);
-                    wall_pre[ws] = p[u];  // contacts are re-derived from this position by the force kernel
-                    wall_slot[i] = ws;
-                    atomicOr(&wall_bits[i >> 5], 1u << (i & 31));
-                    p[u].x += sx;
-                    p[u].y += sy;
-                    pos[i] = p[u];
-                }
-            }
-        }
-        int row;
-        c[u] = cell_of(g, p[u].x, p[u].y, row);
-    }
-    uint32_t sl[SC_PREPASS_ILP];
-#pragma unroll
-    for (int u = 0; u < SC_PREPASS_ILP; ++u)
-        if (c[u] != SC_INVALID_CELL) sl[u] = atomicAdd(&cell_count[c[u]], 1u);
-#pragma unroll
-    for (int u = 0; u < SC_PREPASS_ILP; ++u) {
-        const uint32_t i = i0 + u * SC_BLOCK;
-        if (c[u] != SC_INVALID_CELL) { cell_key[i] = c[u]; slot[i] = sl[u]; }
+        if (i < n) key_particle<kStep>(g, P, W, O, i, p[u]);
     }
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// exclusive scan of a u32 array, in place, total written to a[n] (three launches: reduce, scan sums, apply).
+// exclusive scan of a u32 array, out of place (in == out is allowed), total written to out[n].
 // 16 items per thread as four 128-bit accesses: a warp request covers 2 KB contiguous.
 #define SC_SCAN_ITEMS 16
 // few, large tiles (256- and 512-thread tiles measured 2-4 us slower on the 1.8M-cell grid; a row-wise scan without
@@ -180,7 +122,7 @@ __device__ __forceinline__ void st_desc(unsigned long long *p, unsigned long lon
 }
 
 __global__ void __launch_bounds__(SC_SCAN_THREADS)
-k_scan_lookback(uint32_t *a, uint32_t n, unsigned long long *desc,
+k_scan_lookback(const uint32_t *in, uint32_t *out, uint32_t n, unsigned long long *desc,
                 uint32_t *ticket) {
     pdl_enter();
     __shared__ uint32_t s_tile, s_prefix;
@@ -189,7 +131,7 @@ k_scan_lookback(uint32_t *a, uint32_t n, unsigned long long *desc,
     const uint32_t tile = s_tile;
     const uint32_t base = tile * SC_SCAN_TILE + threadIdx.x * SC_SCAN_ITEMS;
     uint32_t item[SC_SCAN_ITEMS];
-    scan_load(a, n, base, item);
+    scan_load(in, n, base, item);
     uint32_t v = 0;
 #pragma unroll
     for (int q = 0; q < SC_SCAN_ITEMS; ++q) v += item[q];
@@ -217,41 +159,47 @@ k_scan_lookback(uint32_t *a, uint32_t n, unsigned long long *desc,
         run += t;
     }
     if (base + SC_SCAN_ITEMS <= n) {
-        uint4 *p = reinterpret_cast<uint4 *>(a + base);
+        uint4 *p = reinterpret_cast<uint4 *>(out + base);
 #pragma unroll
         for (int q = 0; q < SC_SCAN_ITEMS / 4; ++q) p[q] = make_uint4(item[4 * q], item[4 * q + 1], item[4 * q + 2], item[4 * q + 3]);
     } else {
 #pragma unroll
         for (int q = 0; q < SC_SCAN_ITEMS; ++q)
-            if (base + q < n) a[base + q] = item[q];
+            if (base + q < n) out[base + q] = item[q];
     }
-    if (tile == gridDim.x - 1 && threadIdx.x == SC_SCAN_THREADS - 1) a[n] = run;  // grand total
+    if (tile == gridDim.x - 1 && threadIdx.x == SC_SCAN_THREADS - 1) out[n] = run;  // grand total
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// K2: counting-sort placement.  The arrival slot inside a cell came from an atomic, so the order inside a cell
-// is arbitrary here; k_rank_gather makes it deterministic.
+// K2: counting-sort placement.  A particle claims its place inside its cell by taking one off the cell's count
+// (key_particle counted it): the returned value minus one is a slot in [0, count), and after the last claim every
+// count is zero again - the grid is ready for the next tick's key pass without a clearing pass.  The order inside a
+// cell is arbitrary here; k_rank_gather makes it deterministic.
 #define SC_PLACE_ILP 4
 __global__ void __launch_bounds__(SC_BLOCK)
-k_place(const Counters *cnt, const uint32_t *cell_key, const uint32_t *slot,
+k_place(const Counters *cnt, const uint32_t *cell_key, uint32_t *cell_count,
         const uint32_t *cell_start, uint32_t *tmpidx, uint32_t cap) {
     pdl_enter();
     const uint32_t i0 = blockIdx.x * (SC_BLOCK * SC_PLACE_ILP) + threadIdx.x;
     uint32_t c[SC_PLACE_ILP], sl[SC_PLACE_ILP], st[SC_PLACE_ILP];
-    // keys and slots are requested before the live count is known (see k_prepass)
+    // keys are requested before the live count is known (see k_prepass)
 #pragma unroll
     for (int u = 0; u < SC_PLACE_ILP; ++u) {
         const uint32_t i = i0 + u * SC_BLOCK;
         c[u] = SC_INVALID_CELL;
-        if (i < cap) { c[u] = cell_key[i]; sl[u] = slot[i]; }
+        if (i < cap) c[u] = cell_key[i];
     }
+    // the same bound key_particle counted under (see the invariant there)
     const uint32_t n = cnt->n < cap ? cnt->n : cap;
 #pragma unroll
     for (int u = 0; u < SC_PLACE_ILP; ++u)
         if (i0 + u * SC_BLOCK >= n) c[u] = SC_INVALID_CELL;
 #pragma unroll
     for (int u = 0; u < SC_PLACE_ILP; ++u)
-        if (c[u] != SC_INVALID_CELL) st[u] = cell_start[c[u]];
+        if (c[u] != SC_INVALID_CELL) {
+            st[u] = cell_start[c[u]];
+            sl[u] = atomicSub(&cell_count[c[u]], 1u) - 1u;
+        }
 #pragma unroll
     for (int u = 0; u < SC_PLACE_ILP; ++u)
         if (c[u] != SC_INVALID_CELL) tmpidx[st[u] + sl[u]] = i0 + u * SC_BLOCK;
@@ -261,7 +209,7 @@ k_place(const Counters *cnt, const uint32_t *cell_key, const uint32_t *slot,
 // Produces exactly np.lexsort((x, floor(y / d))) (collision_detector.py:127) as the concatenation of cells.
 template <typename Real>
 __global__ void __launch_bounds__(SC_BLOCK)
-k_rank_gather(Grid g, const uint32_t *cell_start, const uint32_t *tmpidx,
+k_rank_gather(Counters *cnt, Grid g, const uint32_t *cell_start, const uint32_t *tmpidx,
               const uint32_t *cell_key, const double2 *pos,
               const typename Vec2<Real>::type *vel, const uint32_t *uid,
               const uint32_t *wall_bits, const uint32_t *wall_slot,
@@ -272,6 +220,8 @@ k_rank_gather(Grid g, const uint32_t *cell_start, const uint32_t *tmpidx,
     pdl_enter();
     const uint32_t n = cell_start[g.ncells];
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    // the density kernel's per-tick counters (read by sc_debug_untiled_blocks after the tick, so not reset any later)
+    if (t == 0) { cnt->pair_cursor = 0; cnt->n_untiled = 0; }
     if (t >= n) return;
     const uint32_t i = tmpidx[t];
     const uint32_t c = cell_key[i];
@@ -393,6 +343,16 @@ k_scatter_ps(const uint32_t *n_ptr, const uint32_t *uid,
     const uint32_t r = rank_of_uid[uid[s]];
     if (prs) prs[r] = (double)v.p;
     if (tens) { double2 o; o.x = (double)v.sx; o.y = (double)v.sy; tens[r] = o; }
+}
+// positions in original order.  `wall_bits` (or NULL): the wall bitmap of a next tick whose hard-wall fix the force
+// kernel already applied (NextKeys); a particle it moved is reported at its position before the fix, as the tick left it.
+__global__ void __launch_bounds__(SC_BLOCK)
+k_scatter_pos(const uint32_t *n_ptr, const uint32_t *uid, const uint32_t *rank_of_uid, const double2 *pos,
+              const uint32_t *wall_bits, const uint32_t *wall_slot, const double2 *wall_pre, double2 *dst) {
+    const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= *n_ptr) return;
+    const bool fixed = wall_bits && ((wall_bits[s >> 5] >> (s & 31)) & 1u);
+    dst[rank_of_uid[uid[s]]] = fixed ? wall_pre[wall_slot[s]] : pos[s];
 }
 __global__ void __launch_bounds__(SC_BLOCK)
 k_scatter_uid(const uint32_t *n_ptr, const uint32_t *uid,
@@ -517,25 +477,36 @@ __global__ void __launch_bounds__(SC_BLOCK) k_iota(uint32_t *a, uint32_t base, u
     if (i < n) a[i] = base + i;
 }
 
-// COLD start of a tick (the first tick of a context, or the first after the cell grid was rebuilt): what the previous
-// tick's force kernel would have done (end_of_tick in sc_common.cuh), as a launch of its own.  `carry_count` is kept
-// for the standalone search.
+// COLD start of a tick (the first tick of a context, the first after the cell grid was rebuilt), as a launch of its own:
+// zero the cell-count grid, the tick's wall bitmaps and the scan's descriptors, reset the counters.  `carry` (or NULL):
+// the last scan's total, = the live count when no force kernel carried it.
+// The same launch, with `restore`, takes back what the last force kernel did for a next tick that will not use it
+// (NextKeys, dropped by the host): the positions of the particles it moved in the hard-wall fix are put back from the
+// wall side list (bits_a = that tick's wall bitmap) before the bitmaps are zeroed.
+struct KeyRestore { double2 *pos; const uint32_t *wall_slot; const double2 *wall_pre; };
 __global__ void __launch_bounds__(SC_BLOCK)
-k_begin_tick(Counters *cnt, uint32_t *cell_count, uint32_t ncells, int carry_count,
+k_begin_tick(Counters *cnt, uint32_t *cell_count, uint32_t ncells, const uint32_t *carry,
              uint32_t *bits_a, uint32_t *bits_b, uint32_t nbits_words,
-             unsigned long long *scan_desc, uint32_t scan_words, uint32_t cap) {
+             unsigned long long *scan_desc, uint32_t scan_words, uint32_t cap, KeyRestore restore) {
     pdl_enter();
     const uint32_t tid = blockIdx.x * blockDim.x + threadIdx.x, nth = gridDim.x * blockDim.x;
     if (tid == 0) {
-        if (carry_count) cnt->n = cell_count[ncells];
+        if (carry) cnt->n = *carry;
         if (cnt->n > cap) { cnt->n = cap; cnt->overflow = 1u; }
-        cnt->n_wall = 0; cnt->n_pairs = 0; cnt->pair_cursor = 0; cnt->n_untiled = 0;
+        cnt->n_wall[0] = 0; cnt->n_wall[1] = 0; cnt->n_pairs = 0; cnt->pair_cursor = 0; cnt->n_untiled = 0;
     }
     uint4 *c4 = reinterpret_cast<uint4 *>(cell_count);
     const uint32_t n4 = ncells / 4;
     for (uint32_t i = tid; i < n4; i += nth) c4[i] = make_uint4(0, 0, 0, 0);
     for (uint32_t i = n4 * 4 + tid; i < ncells; i += nth) cell_count[i] = 0;
-    for (uint32_t i = tid; i < nbits_words; i += nth) { bits_a[i] = 0; bits_b[i] = 0; }
+    for (uint32_t i = tid; i < nbits_words; i += nth) {
+        if (restore.pos)  // a set bit is a particle the wall fix moved (only the key pass sets them; K4 zeroed the rest)
+            for (uint32_t m = bits_a[i]; m; m &= m - 1u) {
+                const uint32_t k = i * 32u + (uint32_t)(__ffs(m) - 1);
+                restore.pos[k] = restore.wall_pre[restore.wall_slot[k]];
+            }
+        bits_a[i] = 0; bits_b[i] = 0;
+    }
     for (uint32_t i = tid; i < scan_words; i += nth) scan_desc[i] = 0ull;  // tile descriptors + ticket of the cell scan
 }
 

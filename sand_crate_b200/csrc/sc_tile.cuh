@@ -283,8 +283,9 @@ __global__ void __launch_bounds__(SC_TILE, SC_TILE_RESIDENT / SC_TILE)
 k_density_tile(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
                const BlockDesc *desc, const double2 *pos,
                const SearchRec *rec, const uint32_t *cell_key,
-               uint2 *pair_rec, uint8_t *pair_cnt, PS<float> *ps_out) {
+               uint2 *pair_rec, uint8_t *pair_cnt, PS<float> *ps_out, NextWallClear next) {
     pdl_enter();
+    clear_next_walls(next);
     // staged: [records 20 KB | cell boundaries 4.7 KB | 16-bit lists 10 KB]; pass-through: [32-bit lists 20 KB]
     __shared__ __align__(128) unsigned char s_raw[SC_TILE_SMEM_K4];
     __shared__ __align__(8) unsigned long long s_bar;
@@ -371,7 +372,7 @@ __global__ void __launch_bounds__(SC_TILE, SC_K5_TILE_MINBLOCKS)
 k_force_tile(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallParams W, const BlockDesc *desc,
              const double2 *pos, const float2 *vel, const uint2 *pair_rec,
              const uint8_t *pair_cnt, const PS<float> *ps_in, const uint32_t *wall_bits, const uint32_t *wall_slot,
-             const double2 *wall_pre, double2 *pos_out, float2 *vel_out, double *monitor, TickDuty duty) {
+             const double2 *wall_pre, double2 *pos_out, float2 *vel_out, double *monitor, TickDuty duty, NextKeys nk) {
     pdl_enter();
     end_of_tick(duty, n_ptr);
     __shared__ __align__(128) float4 s_ps[SC_TILE_CAP];
@@ -455,7 +456,7 @@ k_force_tile(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallPar
         for (int k = SC_K5_ROWS; k < K; ++k) pair(my_rec[k * SC_TILE], gp, gv);
     }
     force_tail<float, kMonitor>(s, K, p_i, tx, ty, qx, qy, P, W, ps_own, v_own, touching, wall_slot, wall_pre, pos_out, vel_out,
-                                monitor, n_ptr, [&](float vx, float vy, float &ax, float &ay) {
+                                monitor, n_ptr, nk, [&](float vx, float vy, float &ax, float &ay) {
         ax = sum_vx - (float)K * vx;
         ay = sum_vy - (float)K * vy;
     });
