@@ -174,6 +174,15 @@ int sc_last_pair_count(sc_ctx *ctx, int64_t *n_pairs);
 double sc_debug_rerun(sc_ctx *ctx, int which, int reps);
 /* blocks of the tiled density kernel that ran in pass-through mode in the last tick (windows too large to stage) */
 int64_t sc_debug_untiled_blocks(sc_ctx *ctx);
+/* The pair records the density kernel of the last tick handed to its force kernel, in original index order:
+ * counts[n] = K_i as stored, nbr_row[n x 20] = the neighbors' original indices in list order (-1 padded),
+ * nvec[n x 20 x 2] = the unit vectors as the force kernel decodes them (fp32 in mixed precision, widened).  Valid from
+ * the end of sc_step / sc_step_finish until the next step or sc_debug_rerun rewrites the pair buffers; refused inside a
+ * split step (the buffers still hold the tick before).  Synchronises. */
+int sc_debug_pair_records(sc_ctx *ctx, int32_t *counts, int32_t *nbr_row, double *nvec, int64_t cap);
+/* the cell grid: grid4 = {row_min, col_min, nrows, ncols}; cell of (row, col) = (row - row_min) * ncols + col - col_min,
+ * both clamped to [1, size - 2] */
+int sc_debug_grid(sc_ctx *ctx, int64_t *grid4);
 
 /* ---- multi-GPU strip decomposition (one context per rank) ------------------------------------------------------ */
 /* The reference's search is already a 1-D strip decomposition in y with strip height one diameter

@@ -100,6 +100,8 @@ SIGNATURES = {
     "sc_last_pair_count": (C.c_int, [_ctx, _lp]),
     "sc_debug_rerun": (C.c_double, [_ctx, C.c_int, C.c_int]),
     "sc_debug_untiled_blocks": (C.c_int64, [_ctx]),
+    "sc_debug_pair_records": (C.c_int, [_ctx, _ip, _ip, _dp, C.c_int64]),
+    "sc_debug_grid": (C.c_int, [_ctx, _lp]),
 }
 
 _lib = None
@@ -454,6 +456,21 @@ class Context:
 
     def untiled_blocks(self) -> int:
         return int(self._L.sc_debug_untiled_blocks(self._h))
+
+    def get_pair_records(self, n: int):
+        """(counts, neighbor rows, unit vectors) of the pair records the last tick's density kernel handed to its
+        force kernel, in original index order (sc_debug_pair_records)."""
+        counts = np.empty(n, np.int32)
+        rows = np.empty((n, MAX_NEIGHBORS), np.int32)
+        nvec = np.empty((n, MAX_NEIGHBORS, 2))
+        self._ck(self._L.sc_debug_pair_records(self._h, _ptr(counts, _ip), _ptr(rows, _ip), _ptr(nvec, _dp), n))
+        return counts, rows, nvec
+
+    def grid(self):
+        """(row_min, col_min, nrows, ncols) of the cell grid (sc_debug_grid)."""
+        g = np.zeros(4, np.int64)
+        self._ck(self._L.sc_debug_grid(self._h, _ptr(g, _lp)))
+        return tuple(int(x) for x in g)
 
 
 def source_uniform(seed: int, tick: int, source_index: int, j: int) -> float:

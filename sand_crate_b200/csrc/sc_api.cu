@@ -92,6 +92,7 @@ struct sc_ctx {
     bool carry_count = false; // the device count must be refreshed from the previous tick's scan total
     int pair_mode = 1;  // mixed mode with device noise: 1 = tiled K4 (sc_tile.cuh), 0 = the untiled K4 of sc_pair.cuh
                         // (developer switch: SC_PAIR_MODE, for A/B timing)
+    int pair_path = TAP_PAIRS_F64;  // which pair kernels wrote the last tick's records (TapPairPath, sc_tile.cuh)
     bool monitor_on = false;  // ForceMonitor mode: K5 also sums |dv| per force stage
     double *monitor = nullptr; // 6 sums + particle count of the last tick
     bool dist_on = false;     // strip decomposition: particle arrays hold owned + ghost particles
@@ -935,18 +936,21 @@ static int enqueue_forces(sc_ctx *ctx, const uint32_t *noise_off) {
                 CKR(launch_density<double>(ctx, g, dp, noise_off, n));
             }
             CKR(launch_force<double>(ctx, dp, n_ptr, n, keys));
+            ctx->pair_path = TAP_PAIRS_F64;
         } else if (dp.noise_mode == SC_NOISE_HOST || (ctx->pair_mode == 0)) {
             {
                 ProfScope ps(ctx, SLOT_DENSITY);
                 CKR(launch_density<float>(ctx, g, dp, noise_off, n));
             }
             CKR(launch_force<float>(ctx, dp, n_ptr, n, keys));
+            ctx->pair_path = TAP_PAIRS_UNTILED;
         } else {
             {
                 ProfScope ps(ctx, SLOT_DENSITY);
                 CKR(launch_density_tile(ctx, g, dp, n));
             }
             CKR(launch_force_tile(ctx, dp, n_ptr, n, keys));
+            ctx->pair_path = TAP_PAIRS_TILED;
         }
     }
     // the force kernel carried the count; the density kernel cleared the next tick's wall set, k_place the counts
@@ -1283,6 +1287,43 @@ extern "C" int sc_last_pair_count(sc_ctx *ctx, int64_t *n_pairs) {
     CK(cudaMemcpyAsync(&h, ctx->cnt, sizeof(Counters), cudaMemcpyDeviceToHost, ctx->stream));
     CK(stream_sync(ctx));
     *n_pairs = (int64_t)h.n_pairs;
+    return 0;
+}
+
+// ---- pair-record tap (declared in include/sandcrate.h under "diagnostics"): what the last tick's density kernel handed
+// to its force kernel, per particle in original index order - K, the neighbors' row indices in list order, and the unit
+// vectors as the force kernel decodes them.  It reads the pair buffers, so it must come before anything that rewrites
+// them (the next step, sc_debug_rerun); inside a split step they still hold the tick before.
+extern "C" int sc_debug_pair_records(sc_ctx *ctx, int32_t *counts, int32_t *nbr_row, double *nvec, int64_t cap) {
+    int64_t n = 0;
+    CKR(tap_prologue(ctx, "sc_debug_pair_records", cap, &n));
+    if (ctx->in_step) return fail(ctx, "sc_debug_pair_records: inside a split step (the records are the last tick's)");
+    if (n == 0) return 0;
+    const size_t nr = (size_t)n * SC_MAX_NEIGHBORS;
+    char *out_d = nullptr;  // [vectors nr x 16 | rows nr x 4 | counts n x 4]
+    CK(cudaMalloc((void **)&out_d, nr * 16 + nr * 4 + (size_t)n * 4));
+    double2 *vec_d = reinterpret_cast<double2 *>(out_d);
+    int *row_d = reinterpret_cast<int *>(out_d + nr * 16), *cnt_d = row_d + nr;
+    { ProfScope ps(ctx, SLOT_IO);
+      k_tap_pair_records<<<(unsigned)((n + SC_TILE - 1) / SC_TILE), SC_TILE, 0, ctx->stream>>>(
+          ctx->cell_start + ctx->grid.ncells, ctx->pair_path, ctx->blk_desc, ctx->pair_cnt, ctx->pair_off, ctx->pair_j,
+          ctx->pair_n, sorted_uids(ctx), ctx->rank_of_uid, cnt_d, row_d, vec_d); }
+    if (counts) CK(cudaMemcpyAsync(counts, cnt_d, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
+    if (nbr_row) CK(cudaMemcpyAsync(nbr_row, row_d, sizeof(int32_t) * nr, cudaMemcpyDeviceToHost, ctx->stream));
+    if (nvec) CK(cudaMemcpyAsync(nvec, vec_d, sizeof(double2) * nr, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(stream_sync(ctx));
+    CK(cudaFree(out_d));
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// the cell grid of the last search: origin row / column (the cell of (row, col) is (row - row_min) * ncols + col -
+// col_min, clamped into [1, nrows - 2] x [1, ncols - 2]) and its size
+extern "C" int sc_debug_grid(sc_ctx *ctx, int64_t *grid4) {
+    CKR(enter(ctx, "sc_debug_grid"));
+    if (!grid4) return fail(ctx, "sc_debug_grid: NULL argument");
+    if (!ctx->params_set) return fail(ctx, "sc_debug_grid: sc_set_params has not been called");
+    grid4[0] = ctx->grid.row_min; grid4[1] = ctx->grid.col_min; grid4[2] = ctx->grid.nrows; grid4[3] = ctx->grid.ncols;
     return 0;
 }
 

@@ -462,4 +462,51 @@ k_force_tile(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallPar
     });
 }
 
+// ------------------------------------------------------------------------------------------------------------
+// Pair-record tap (sc_debug_pair_records): the records the last tick's density kernel left for the force kernel, as
+// the force kernel reads them, in original index order.  One thread per sorted particle, blocks of SC_TILE, so that a
+// block here is a block of the tiled kernels and its record region and windows are theirs.  Read-only on the step's
+// buffers.  A record whose index does not map into the live set (which a correct run never writes) is reported as
+// row -2 instead of being followed.
+enum TapPairPath { TAP_PAIRS_F64 = 0, TAP_PAIRS_UNTILED = 1, TAP_PAIRS_TILED = 2 };
+__global__ void __launch_bounds__(SC_TILE)
+k_tap_pair_records(const uint32_t *n_ptr, int path, const BlockDesc *desc, const uint8_t *pair_cnt,
+                   const uint32_t *pair_off, const uint32_t *pair_j, const void *pair_n, const uint32_t *uid,
+                   const uint32_t *rank_of_uid, int *cnt_out, int *row_out, double2 *vec_out) {
+    const uint32_t n = *n_ptr;
+    const uint32_t s = blockIdx.x * SC_TILE + threadIdx.x;
+    if (s >= n) return;
+    const uint32_t r = rank_of_uid[uid[s]];
+    const int K = pair_cnt[s];
+    cnt_out[r] = K;
+    TileWindows w{};
+    if (path == TAP_PAIRS_TILED) w = tile_windows(desc + blockIdx.x);
+    for (int k = 0; k < SC_MAX_NEIGHBORS; ++k) {
+        const size_t o = (size_t)r * SC_MAX_NEIGHBORS + k;
+        if (k >= K) { row_out[o] = -1; vec_out[o] = make_double2(0, 0); continue; }
+        uint32_t j;
+        double2 v;
+        if (path == TAP_PAIRS_F64) {
+            const size_t i = (size_t)pair_off[s] + k;
+            j = pair_j[i];
+            v = reinterpret_cast<const double2 *>(pair_n)[i];
+        } else {
+            const uint2 *rec = reinterpret_cast<const uint2 *>(pair_n);
+            const uint2 e = path == TAP_PAIRS_TILED ? rec[((size_t)blockIdx.x * SC_MAX_NEIGHBORS + k) * SC_TILE + threadIdx.x]
+                                                    : rec[(size_t)pair_off[s] + k];
+            float nx, ny;
+            pair_decode(e, j, nx, ny);
+            v = make_double2((double)nx, (double)ny);
+            if (path == TAP_PAIRS_TILED && w.staged) {  // local index in W0 | W1 | W2 -> sorted index
+                uint32_t m = 0xFFFFFFFFu;
+                for (int q = 0; q < 3; ++q)
+                    if (j >= w.off[q] && j < w.off[q] + w.cnt[q]) m = w.base[q] + (j - w.off[q]);
+                j = m;
+            }
+        }
+        row_out[o] = j < n ? (int)rank_of_uid[uid[j]] : -2;
+        vec_out[o] = v;
+    }
+}
+
 }  // namespace sc

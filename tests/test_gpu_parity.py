@@ -2,7 +2,9 @@
 libsandcrate.so); the oracle is only the checker.
 
 Bars (SURVEY.md section 8(c)):
-  * cell rows, sorted order, neighbor lists (order + 20-trim): bit-exact, both precision modes
+  * cell rows, sorted order, neighbor lists (order + 20-trim): bit-exact, both precision modes.  The lists come from
+    `get_neighbors`, which re-runs the untiled count kernel; the tiled density kernel's own lists and vectors are
+    checked in tests/test_pair_records_gpu.py through `get_pair_records`
   * fp64 parity mode: positions, velocities, pressures, surface normals bit-exact per step
   * mixed mode (fp64 positions, fp32 forces): per step from the same inputs,
       max|dv| <= 1e-5 * max(max|v|, 1)   and   max|dpos| <= 1e-5 * d
