@@ -170,7 +170,8 @@ int64_t sc_sync_count(const sc_ctx *ctx);   /* times an entry point made the hos
 int sc_last_pair_count(sc_ctx *ctx, int64_t *n_pairs);
 
 /* ---- diagnostics (developer aids; no reference counterpart, results are never affected) ---------------------- */
-/* re-run the density (which = 4) or force (which = 5) kernel of the last tick `reps` times; mean milliseconds */
+/* re-run the density (which = 4) or force (which = 5) kernel of the last tick `reps` times; mean milliseconds.
+ * -1 before a step, inside a split step and under SC_NOISE_HOST (the step's noise offsets do not outlive it). */
 double sc_debug_rerun(sc_ctx *ctx, int which, int reps);
 /* blocks of the tiled density kernel that ran in pass-through mode in the last tick (windows too large to stage) */
 int64_t sc_debug_untiled_blocks(sc_ctx *ctx);

@@ -90,9 +90,6 @@ struct sc_ctx {
     bool rows_valid = false;  // pos_cur / uid_cur are still in the order of the last search (cell rows ascending)
     bool lists_valid = false, rank_valid = false;
     bool carry_count = false; // the device count must be refreshed from the previous tick's scan total
-    int pair_mode = 1;  // mixed mode with device noise: 1 = tiled K4 (sc_tile.cuh), 0 = the untiled K4 of sc_pair.cuh
-                        // (developer switch: SC_PAIR_MODE, for A/B timing)
-    int pair_path = TAP_PAIRS_F64;  // which pair kernels wrote the last tick's records (TapPairPath, sc_tile.cuh)
     bool monitor_on = false;  // ForceMonitor mode: K5 also sums |dv| per force stage
     double *monitor = nullptr; // 6 sums + particle count of the last tick
     bool dist_on = false;     // strip decomposition: particle arrays hold owned + ghost particles
@@ -350,7 +347,6 @@ extern "C" int sc_create(int device, int precision, int64_t capacity, void *stre
     sc_ctx *c = new sc_ctx();
     ctx = c;
     c->device = device; c->precision = precision; c->cap = capacity;
-    { const char *e_ = getenv("SC_PAIR_MODE"); if (e_ && e_[0] >= '0' && e_[0] <= '1') c->pair_mode = e_[0] - '0'; }
     if (stream) c->stream = (cudaStream_t)stream;
     else { cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking); c->own_stream = true; }
     // + 16: the tiled kernels bulk-copy windows whose ends are rounded up to 16-byte groups
@@ -367,13 +363,14 @@ extern "C" int sc_create(int device, int precision, int64_t capacity, void *stre
         rc |= dev_alloc(c, &c->blk_desc, (n + SC_TILE - 1) / SC_TILE + 1);
     }
     rc |= dev_alloc(c, (char **)&c->ps, n * 4 * rs);
-    // pair records: the untiled kernels bump-allocate; the tiled kernels give every block of SC_TILE sorted particles its
-    // own slot-major region of SC_TILE x 20 records, so the buffer holds whole blocks
+    // pair records: the fp64 kernels bump-allocate (pair_off); the tiled kernels give every block of SC_TILE sorted
+    // particles its own slot-major region of SC_TILE x 20 records, so the buffer holds whole blocks
     const size_t npair = ((n + SC_TILE - 1) / SC_TILE) * SC_TILE * SC_MAX_NEIGHBORS;
     rc |= dev_alloc(c, &c->pair_j, precision == SC_PRECISION_F64 ? npair : 1);
     rc |= dev_alloc(c, (char **)&c->pair_n, npair * 2 * rs);
     if (!rc) cudaMemsetAsync(c->pair_n, 0, npair * 2 * rs, c->stream);  // K5 bulk-copies slots K4 may not have written
-    rc |= dev_alloc(c, &c->pair_off, n); rc |= dev_alloc(c, &c->pair_cnt, n);
+    rc |= dev_alloc(c, &c->pair_off, precision == SC_PRECISION_F64 ? n : 1);
+    rc |= dev_alloc(c, &c->pair_cnt, n);
     for (int q = 0; q < 2; ++q) { rc |= dev_alloc(c, &c->wbits_cur[q], n / 32 + 1); rc |= dev_alloc(c, &c->wbits_srt[q], n / 32 + 1); }
     c->wall_bits_cur = c->wbits_cur[0]; c->wall_bits_srt = c->wbits_srt[0];
     rc |= dev_alloc(c, &c->wall_slot_cur, n); rc |= dev_alloc(c, &c->wall_slot_srt, n);
@@ -842,20 +839,30 @@ static NextWallClear next_wall_clear(sc_ctx *ctx) {
     return NextWallClear{ctx->wbits_cur[o], ctx->wbits_srt[o], (uint32_t)(ctx->cap / 32 + 1), &ctx->cnt->n_wall[o]};
 }
 
-template <typename Real>
-static int launch_density(sc_ctx *ctx, const Grid &g, const DevParams &dp, const uint32_t *noise_off, int64_t n) {
-    typedef typename Vec2<Real>::type R2;
+static int launch_density(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, int64_t n) {
     auto go = [&](auto kernel) {
-        return launch_pdl(kernel, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream, ctx->cnt, g, dp, ctx->cell_start,
-                          ctx->pos_srt, ctx->rel_srt, ctx->cell_key_srt, ctx->uid_srt, ctx->noise_dev, noise_off,
-                          ctx->rank_of_uid, ctx->pair_j, (R2 *)ctx->pair_n, ctx->pair_off, ctx->pair_cnt,
-                          (PS<Real> *)ctx->ps, next_wall_clear(ctx));
+        return launch_pdl(kernel, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream, ctx->cnt, ctx->grid, dp, ctx->cell_start,
+                          ctx->pos_srt, ctx->rel_srt, ctx->cell_key_srt, ctx->uid_cur, ctx->noise_dev, noise_off,
+                          ctx->rank_of_uid, ctx->pair_j, (double2 *)ctx->pair_n, ctx->pair_off, ctx->pair_cnt,
+                          (PS<double> *)ctx->ps, next_wall_clear(ctx));
     };
-    cudaError_t e;
-    if (dp.noise_mode == SC_NOISE_HOST) e = go(k_density<Real, SC_NOISE_HOST>);
-    else if (dp.noise_mode == SC_NOISE_COUNTER) e = go(k_density<Real, SC_NOISE_COUNTER>);
-    else e = go(k_density<Real, SC_NOISE_NONE>);
-    CK(e);
+    if (dp.noise_mode == SC_NOISE_HOST) CK(go(k_density<SC_NOISE_HOST>));
+    else if (dp.noise_mode == SC_NOISE_COUNTER) CK(go(k_density<SC_NOISE_COUNTER>));
+    else CK(go(k_density<SC_NOISE_NONE>));
+    return 0;
+}
+
+// K4 stages the block's neighborhood in shared memory (sc_tile.cuh)
+static int launch_density_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, int64_t n) {
+    auto go = [&](auto kernel) {
+        return launch_pdl(kernel, dim3((unsigned)((n + SC_TILE - 1) / SC_TILE)), dim3(SC_TILE), ctx->stream, ctx->cnt,
+                          ctx->grid, dp, ctx->cell_start, ctx->blk_desc, ctx->pos_srt, ctx->rec_srt, ctx->cell_key_srt,
+                          (uint2 *)ctx->pair_n, ctx->pair_cnt, (PS<float> *)ctx->ps, next_wall_clear(ctx),
+                          HostNoise{ctx->noise_dev, noise_off, ctx->rank_of_uid});
+    };
+    if (dp.noise_mode == SC_NOISE_HOST) CK(go(k_density_tile<SC_NOISE_HOST>));
+    else if (dp.noise_mode == SC_NOISE_COUNTER) CK(go(k_density_tile<SC_NOISE_COUNTER>));
+    else CK(go(k_density_tile<SC_NOISE_NONE>));
     return 0;
 }
 
@@ -874,28 +881,21 @@ static NextKeys next_keys(sc_ctx *ctx, bool keys) {
     return k;
 }
 
-template <typename Real>
 static int launch_force(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n, bool keys) {
-    typedef typename Vec2<Real>::type R2;
-    if (ctx->monitor_on) CK(cudaMemsetAsync(ctx->monitor, 0, sizeof(double) * 8, ctx->stream));
-    ProfScope ps(ctx, SLOT_FORCE);
-    static int k5_threads = 0;  // SC_K5_THREADS: developer switch for A/B timing of the block size
-    if (!k5_threads) { const char *e = getenv("SC_K5_THREADS"); k5_threads = e ? atoi(e) : SC_K5_THREADS; }
-    const unsigned nt = (unsigned)k5_threads, nb = (unsigned)((n + nt - 1) / nt);
+    const unsigned nb = (unsigned)((n + SC_K5_THREADS - 1) / SC_K5_THREADS);
     auto go = [&](auto kernel) {
-        return launch_pdl(kernel, dim3(nb), dim3(nt), ctx->stream, n_ptr, dp, ctx->walls, ctx->pos_srt,
-                          (const R2 *)ctx->vel_srt, ctx->pair_j, (const R2 *)ctx->pair_n, ctx->pair_off, ctx->pair_cnt,
-                          (const PS<Real> *)ctx->ps, ctx->wall_bits_srt, ctx->wall_slot_srt, ctx->wall_pre,
-                          ctx->pos_cur, (R2 *)ctx->vel_cur, ctx->monitor, tick_duty(ctx), next_keys(ctx, keys));
+        return launch_pdl(kernel, dim3(nb), dim3(SC_K5_THREADS), ctx->stream, n_ptr, dp, ctx->walls, ctx->pos_srt,
+                          (const double2 *)ctx->vel_srt, ctx->pair_j, (const double2 *)ctx->pair_n, ctx->pair_off,
+                          ctx->pair_cnt, (const PS<double> *)ctx->ps, ctx->wall_bits_srt, ctx->wall_slot_srt,
+                          ctx->wall_pre, ctx->pos_cur, (double2 *)ctx->vel_cur, ctx->monitor, tick_duty(ctx),
+                          next_keys(ctx, keys));
     };
-    CK(ctx->monitor_on ? go(k_force<Real, true>) : go(k_force<Real, false>));
+    CK(ctx->monitor_on ? go(k_force<true>) : go(k_force<false>));
     return 0;
 }
 
-// mixed precision with device-side noise: K5 on the same blocks and windows as K4 (sc_tile.cuh)
+// K5 on the same blocks and windows as K4 (sc_tile.cuh)
 static int launch_force_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n, bool keys) {
-    if (ctx->monitor_on) CK(cudaMemsetAsync(ctx->monitor, 0, sizeof(double) * 8, ctx->stream));
-    ProfScope ps(ctx, SLOT_FORCE);
     auto go = [&](auto kernel) {
         return launch_pdl(kernel, dim3((unsigned)((n + SC_TILE - 1) / SC_TILE)), dim3(SC_TILE), ctx->stream, n_ptr, dp,
                           ctx->walls, ctx->blk_desc, ctx->pos_srt, (const float2 *)ctx->vel_srt, (const uint2 *)ctx->pair_n,
@@ -907,59 +907,47 @@ static int launch_force_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *n
     return 0;
 }
 
-// mixed precision with device-side noise: K4 stages the block's neighborhood in shared memory (sc_tile.cuh)
-static int launch_density_tile(sc_ctx *ctx, const Grid &g, const DevParams &dp, int64_t n) {
-    auto go = [&](auto kernel) {
-        return launch_pdl(kernel, dim3((unsigned)((n + SC_TILE - 1) / SC_TILE)), dim3(SC_TILE), ctx->stream, ctx->cnt, g, dp,
-                          ctx->cell_start, ctx->blk_desc, ctx->pos_srt, ctx->rec_srt, ctx->cell_key_srt, (uint2 *)ctx->pair_n,
-                          ctx->pair_cnt, (PS<float> *)ctx->ps, next_wall_clear(ctx));
-    };
-    CK(dp.noise_mode == SC_NOISE_COUNTER ? go(k_density_tile<SC_NOISE_COUNTER>) : go(k_density_tile<SC_NOISE_NONE>));
+// The parameters of the step of tick `tick`: its noise key, and the effective noise mode (a zero noise level is none).
+static DevParams step_params(const sc_ctx *ctx, uint64_t tick) {
+    DevParams dp = ctx->dp;
+    dp.noise_mode = (ctx->noise_mode != SC_NOISE_NONE && ctx->hp.collider_noise_level == 0.0) ? SC_NOISE_NONE
+                                                                                             : ctx->noise_mode;
+    dp.tick_key = tick_key(ctx->seed, tick);
+    return dp;
+}
+
+// The pair kernels of the last search, chosen by the precision alone: k_density / k_force (sc_pair.cuh) in fp64, the
+// tiled kernels (sc_tile.cuh) in mixed precision, in every noise mode.  `k4`, `k5`: which of the two to enqueue.
+// `noise_off`: the CSR offsets of SC_NOISE_HOST.  The sorted set's uids must be in uid_cur.
+static int launch_pair_kernels(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, bool k4, bool k5, bool keys) {
+    const int64_t n = ctx->n_host;
+    const bool f64 = ctx->precision == SC_PRECISION_F64;
+    if (k4) {
+        ProfScope ps(ctx, SLOT_DENSITY);
+        CKR(f64 ? launch_density(ctx, dp, noise_off, n) : launch_density_tile(ctx, dp, noise_off, n));
+    }
+    if (k5) {
+        if (ctx->monitor_on) CK(cudaMemsetAsync(ctx->monitor, 0, sizeof(double) * 8, ctx->stream));
+        ProfScope ps(ctx, SLOT_FORCE);
+        const uint32_t *n_ptr = ctx->cell_start + ctx->grid.ncells;
+        CKR(f64 ? launch_force(ctx, dp, n_ptr, n, keys) : launch_force_tile(ctx, dp, n_ptr, n, keys));
+    }
     return 0;
 }
 
 static int enqueue_forces(sc_ctx *ctx, const uint32_t *noise_off) {
     const int64_t n = ctx->n_host;
-    const Grid &g = ctx->grid;
-    DevParams dp = ctx->dp;
-    dp.noise_mode = (ctx->noise_mode != SC_NOISE_NONE && ctx->hp.collider_noise_level == 0.0) ? SC_NOISE_NONE
-                                                                                             : ctx->noise_mode;
-    dp.tick_key = tick_key(ctx->seed, ctx->tick);
-    const uint32_t *n_ptr = ctx->cell_start + g.ncells;
+    // the new state (pos_cur, vel_cur) is in this tick's sorted order, whose uids are uid_srt
+    uint32_t *t = ctx->uid_cur; ctx->uid_cur = ctx->uid_srt; ctx->uid_srt = t;
     // the force kernel runs the next tick's key pass (NextKeys) unless a call since the last step changed what the keys
     // depend on (drop_keys) or this is a strip, whose exchange changes the particle set between the ticks
     const bool keys = n > 0 && !ctx->keys_dropped && !ctx->dist_on;
-    if (n > 0) {
-        if (ctx->precision == SC_PRECISION_F64) {
-            {
-                ProfScope ps(ctx, SLOT_DENSITY);
-                CKR(launch_density<double>(ctx, g, dp, noise_off, n));
-            }
-            CKR(launch_force<double>(ctx, dp, n_ptr, n, keys));
-            ctx->pair_path = TAP_PAIRS_F64;
-        } else if (dp.noise_mode == SC_NOISE_HOST || (ctx->pair_mode == 0)) {
-            {
-                ProfScope ps(ctx, SLOT_DENSITY);
-                CKR(launch_density<float>(ctx, g, dp, noise_off, n));
-            }
-            CKR(launch_force<float>(ctx, dp, n_ptr, n, keys));
-            ctx->pair_path = TAP_PAIRS_UNTILED;
-        } else {
-            {
-                ProfScope ps(ctx, SLOT_DENSITY);
-                CKR(launch_density_tile(ctx, g, dp, n));
-            }
-            CKR(launch_force_tile(ctx, dp, n_ptr, n, keys));
-            ctx->pair_path = TAP_PAIRS_TILED;
-        }
-    }
+    if (n > 0) CKR(launch_pair_kernels(ctx, step_params(ctx, ctx->tick), noise_off, true, true, keys));
     // the force kernel carried the count; the density kernel cleared the next tick's wall set, k_place the counts
     if (n > 0) { ctx->next_clean = !keys; ctx->next_keyed = keys; ctx->carry_count = false; }
     else ctx->carry_count = true;  // nothing ran: cnt->n is refreshed by the next cold start or by sync_count
     ctx->keys_dropped = false;
     CK(cudaGetLastError());
-    // the new state (pos_cur, vel_cur) is in this tick's sorted order, whose uids are uid_srt
-    uint32_t *t = ctx->uid_cur; ctx->uid_cur = ctx->uid_srt; ctx->uid_srt = t;
     ctx->rows_valid = n > 0;
     ctx->tick += 1;  // crate.py:127
     ctx->n_exact = false;
@@ -1306,8 +1294,8 @@ extern "C" int sc_debug_pair_records(sc_ctx *ctx, int32_t *counts, int32_t *nbr_
     int *row_d = reinterpret_cast<int *>(out_d + nr * 16), *cnt_d = row_d + nr;
     { ProfScope ps(ctx, SLOT_IO);
       k_tap_pair_records<<<(unsigned)((n + SC_TILE - 1) / SC_TILE), SC_TILE, 0, ctx->stream>>>(
-          ctx->cell_start + ctx->grid.ncells, ctx->pair_path, ctx->blk_desc, ctx->pair_cnt, ctx->pair_off, ctx->pair_j,
-          ctx->pair_n, sorted_uids(ctx), ctx->rank_of_uid, cnt_d, row_d, vec_d); }
+          ctx->cell_start + ctx->grid.ncells, ctx->precision == SC_PRECISION_F64, ctx->blk_desc, ctx->pair_cnt,
+          ctx->pair_off, ctx->pair_j, ctx->pair_n, sorted_uids(ctx), ctx->rank_of_uid, cnt_d, row_d, vec_d); }
     if (counts) CK(cudaMemcpyAsync(counts, cnt_d, sizeof(int32_t) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     if (nbr_row) CK(cudaMemcpyAsync(nbr_row, row_d, sizeof(int32_t) * nr, cudaMemcpyDeviceToHost, ctx->stream));
     if (nvec) CK(cudaMemcpyAsync(nvec, vec_d, sizeof(double2) * nr, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1329,24 +1317,21 @@ extern "C" int sc_debug_grid(sc_ctx *ctx, int64_t *grid4) {
 
 // ---- developer aids (declared in include/sandcrate.h under "diagnostics"): re-run one pair kernel of the last tick
 // `reps` times and return the mean milliseconds.  K4 and K5 only read the sorted set, so re-running them is harmless.
+// -1 before a step, inside a split step, and under SC_NOISE_HOST: the step's noise offsets live in count_by_rank, which
+// the next count kernel (sc_get_neighbors, say) overwrites.
 extern "C" double sc_debug_rerun(sc_ctx *ctx, int which, int reps) {
-    if (!ctx || !ctx->srt_valid) return -1.0;
+    if (!ctx || !ctx->srt_valid || ctx->in_step) return -1.0;
+    const DevParams dp = step_params(ctx, ctx->tick - 1);
+    if (dp.noise_mode == SC_NOISE_HOST) return -1.0;
     cudaSetDevice(ctx->device);
     if (drop_keys(ctx)) return -1.0;  // the force kernel re-run below computes no keys, and its own must not be counted twice
-    DevParams dp = ctx->dp;
-    dp.noise_mode = ctx->noise_mode;
-    dp.tick_key = tick_key(ctx->seed, ctx->tick - 1);
-    const int64_t n = ctx->n_host;
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
     float total = 0;
     for (int r = 0; r < reps; ++r) {
-        if (which == 4) cudaMemsetAsync(&ctx->cnt->pair_cursor, 0, 4, ctx->stream);
+        if (which == 4) cudaMemsetAsync(&ctx->cnt->pair_cursor, 0, 4, ctx->stream);  // the fp64 K4 allocates from zero
         cudaEventRecord(e0, ctx->stream);
-        const bool tiled = ctx->pair_mode != 0 && dp.noise_mode != SC_NOISE_HOST;
-        if (which == 4) { if (tiled) launch_density_tile(ctx, ctx->grid, dp, n); else launch_density<float>(ctx, ctx->grid, dp, nullptr, n); }
-        else if (tiled) launch_force_tile(ctx, dp, ctx->cell_start + ctx->grid.ncells, n, false);
-        else launch_force<float>(ctx, dp, ctx->cell_start + ctx->grid.ncells, n, false);
+        launch_pair_kernels(ctx, dp, nullptr, which == 4, which != 4, false);
         cudaEventRecord(e1, ctx->stream);
         cudaEventSynchronize(e1);
         float ms = 0;

@@ -122,7 +122,7 @@ struct Counters {
                          // the next tick's list while this tick's is being read, see NextKeys)
     uint32_t n_pairs;    // sum K_i (filled by the count kernel)
     uint32_t overflow;   // capacity problems seen on the device
-    uint32_t pair_cursor;  // next free record of the pair buffer (bump allocator, reset every tick)
+    uint32_t pair_cursor;  // fp64 K4: next free record of the pair buffer (bump allocator, reset every tick)
     uint32_t n_tmp;        // scratch count (strip decomposition pack / readback)
     uint32_t n_untiled;    // blocks of the tiled K4 that ran in pass-through mode this tick (windows too large to stage)
 };

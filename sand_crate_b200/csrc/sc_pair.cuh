@@ -1,4 +1,5 @@
-// sc_pair.cuh - the two fused pair kernels (density, force+integrate), templated on the arithmetic type.
+// sc_pair.cuh - the two fused pair kernels of fp64 mode (density, force+integrate), and what they share with the
+// mixed-precision kernels of sc_tile.cuh and the count kernel: the neighbor walk, the acceptance test, the force tail.
 //
 //   k_density  (K4)  collision_detector.py:52-121 pair discovery fused with crate.py:161-175 (populate_colliders),
 //                    261-275 (pressure) and 337-342 (surface normals); emits one record per directed pair
@@ -101,12 +102,11 @@ __device__ __forceinline__ int collect_neighbors(uint32_t s, uint32_t c, const G
 
 // crate.py:167-174 for one directed pair (i <- j): unit vector from the (noised) neighbor to i and the weight
 // w = 1 - clip(dist / d, 0, 1) (crate.py:270).
-template <typename Real> struct PairGeom { Real nx, ny, w; };
+struct PairGeom { double nx, ny, w; };
 
 template <int kNoise>
-__device__ __forceinline__ PairGeom<double> pair_geom_f64(const DevParams &P, double2 pi, double2 pj, uint32_t uid_i,
-                                                          uint32_t uid_j, const double *host_noise,
-                                                          uint32_t noise_index) {
+__device__ __forceinline__ PairGeom pair_geom_f64(const DevParams &P, double2 pi, double2 pj, uint32_t uid_i,
+                                                  uint32_t uid_j, const double *host_noise, uint32_t noise_index) {
     double qx = pj.x, qy = pj.y;
     if constexpr (kNoise != SC_NOISE_NONE) {
         double ux, uy;
@@ -123,7 +123,7 @@ __device__ __forceinline__ PairGeom<double> pair_geom_f64(const DevParams &P, do
     }
     const double rx = pi.x - qx, ry = pi.y - qy;
     const double dist = sqrt(rx * rx + ry * ry);
-    PairGeom<double> g;
+    PairGeom g;
     g.nx = rx / dist;
     g.ny = ry / dist;
     double cl = dist / P.d;
@@ -132,99 +132,6 @@ __device__ __forceinline__ PairGeom<double> pair_geom_f64(const DevParams &P, do
     g.w = 1 - cl;
     return g;
 }
-
-// fp32 flavour: (rx, ry) = p_i - p_j formed from the cell-relative coordinates (absolute fp32 coordinates would lose
-// 1e-4-level precision in the weights at d ~ 1e-4, SURVEY.md section 7.2 item 7)
-template <int kNoise>
-__device__ __forceinline__ PairGeom<float> pair_geom_f32(const DevParams &P, float rx, float ry, uint32_t uid_i,
-                                                         uint32_t uid_j, const double *host_noise,
-                                                         uint32_t noise_index) {
-    if constexpr (kNoise != SC_NOISE_NONE) {
-        float ux, uy;
-        if constexpr (kNoise == SC_NOISE_HOST) {
-            ux = (float)host_noise[2 * (size_t)noise_index];
-            uy = (float)host_noise[2 * (size_t)noise_index + 1];
-        } else {
-            float fx, fy;
-            pair_noise_f32_1to2(pair_noise_bits(P.tick_key, uid_i, uid_j), fx, fy);
-            ux = fx - 1.0f;
-            uy = fy - 1.0f;
-        }
-        const float amp = (float)(P.d * P.level);
-        rx = fmaf(0.5f - ux, amp, rx);
-        ry = fmaf(0.5f - uy, amp, ry);
-    }
-    const float d2 = fmaf(rx, rx, ry * ry);
-    const float inv = rsqrtf(d2);
-    const float dist = d2 * inv;
-    PairGeom<float> g;
-    g.nx = rx * inv;
-    g.ny = ry * inv;
-    float cl = dist * (float)(1.0 / P.d);
-    cl = fminf(fmaxf(cl, 0.0f), 1.0f);
-    g.w = 1.0f - cl;
-    return g;
-}
-
-__device__ __forceinline__ float sqrt_ftz(float x) {
-    float r;
-    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
-    return r;
-}
-
-// ------------------------------------------------------------------------------------------------------------
-// The record K4 hands to K5 for each directed pair (i <- j) in mixed mode: ONE 8-byte word.
-//   .x  the SMALLER-magnitude component m of the unit vector n_ij, as a full fp32
-//   .y  bits 0..27  the neighbor's index L in the block's frame (staged block: position in W0 | W1 | W2; pass-through
-//                   block: sorted index) - K4 and K5 cut the sorted set into the same blocks and windows, so K5 reads
-//                   its neighbor's (p, s, v) from shared memory at L with no translation
-//       bit 28      which component m is (0: n.x, 1: n.y)
-//       bit 29      sign of the other component, whose magnitude K5 restores as sqrt(1 - m^2) (>= 0.707: well conditioned)
-// The vector K5 sees is good to ~1e-7 (fp32 grade).  Round 1 packed it as two signed 16-bit fractions (1.5e-5 per
-// component): that was 250x coarser than the arithmetic around it and showed in the per-tick velocity INCREMENT.
-__device__ __forceinline__ uint2 pair_encode(uint32_t L, float nx, float ny) {
-    const bool y_small = fabsf(ny) < fabsf(nx);
-    const float m = y_small ? ny : nx, big = y_small ? nx : ny;
-    return make_uint2(__float_as_uint(m), L | (y_small ? 0x10000000u : 0u) | ((__float_as_uint(big) >> 2) & 0x20000000u));
-}
-__device__ __forceinline__ void pair_decode(uint2 r, uint32_t &L, float &nx, float &ny) {
-    const float m = __uint_as_float(r.x);
-    float big = sqrt_ftz(fmaf(-m, m, 1.0f));
-    big = __uint_as_float(__float_as_uint(big) | ((r.y << 2) & 0x80000000u));
-    const bool y_small = (r.y & 0x10000000u) != 0u;
-    nx = y_small ? big : m;
-    ny = y_small ? m : big;
-    L = r.y & SC_IDX_MASK;
-}
-
-// fp64 mode keeps two exact arrays (u32 index, double2 vector); mixed mode uses the 8-byte record above, whose index
-// field holds the SORTED index in the untiled kernels of this file.
-template <typename Real> struct PairIO;
-template <> struct PairIO<double> {
-    static __device__ __forceinline__ void store(uint32_t *pj, void *pn, size_t i, uint32_t j, double nx, double ny) {
-        pj[i] = j;
-        reinterpret_cast<double2 *>(pn)[i] = make_double2(nx, ny);
-    }
-    static __device__ __forceinline__ uint32_t load_index(const uint32_t *pj, const void *, size_t i) { return pj[i]; }
-    static __device__ __forceinline__ void load(const uint32_t *pj, const void *pn, size_t i, uint32_t &j, double &nx,
-                                                double &ny) {
-        j = pj[i];
-        const double2 v = reinterpret_cast<const double2 *>(pn)[i];
-        nx = v.x; ny = v.y;
-    }
-};
-template <> struct PairIO<float> {
-    static __device__ __forceinline__ void store(uint32_t *, void *pn, size_t i, uint32_t j, float nx, float ny) {
-        reinterpret_cast<uint2 *>(pn)[i] = pair_encode(j, nx, ny);
-    }
-    static __device__ __forceinline__ uint32_t load_index(const uint32_t *, const void *pn, size_t i) {
-        return reinterpret_cast<const uint2 *>(pn)[i].y & SC_IDX_MASK;
-    }
-    static __device__ __forceinline__ void load(const uint32_t *, const void *pn, size_t i, uint32_t &j, float &nx,
-                                                float &ny) {
-        pair_decode(reinterpret_cast<const uint2 *>(pn)[i], j, nx, ny);
-    }
-};
 
 // crate.py:272 np.sum over a 1-D array: NumPy pairwise_sum (sequential below 8; 8 lanes + tail up to 20)
 __device__ inline double np_sum_1d(const double *a, int n) {
@@ -254,14 +161,14 @@ __device__ inline double np_sum_1d(const double *a, int n) {
 // is consumed by K5, so the pair geometry - noise hash, reciprocal square root - is evaluated once per tick instead
 // of twice.  HBM is the idle resource on this path (the kernels are issue / L1 bound), so 12 bytes per pair are a
 // good trade.
-template <typename Real, int kNoise>  // kNoise: SC_NOISE_* resolved at compile time (no branch in the pair loop)
+template <int kNoise>  // kNoise: SC_NOISE_* resolved at compile time (no branch in the pair loop)
 __global__ void __launch_bounds__(SC_BLOCK)
 k_density(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
           const double2 *pos, const float2 *rel, const uint32_t *cell_key,
           const uint32_t *uid, const double *host_noise,
           const uint32_t *noise_off, const uint32_t *rank_of_uid,
-          uint32_t *pair_j, typename Vec2<Real>::type *pair_n,
-          uint32_t *pair_off, uint8_t *pair_cnt, PS<Real> *ps_out, NextWallClear next) {
+          uint32_t *pair_j, double2 *pair_n,
+          uint32_t *pair_off, uint8_t *pair_cnt, PS<double> *ps_out, NextWallClear next) {
     pdl_enter();
     clear_next_walls(next);
     __shared__ uint32_t s_list[SC_MAX_NEIGHBORS * SC_BLOCK];
@@ -293,41 +200,25 @@ k_density(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
     const uint32_t uid_s = uid[s];
     uint32_t nbase = 0u;
     if constexpr (kNoise == SC_NOISE_HOST) nbase = noise_off[rank_of_uid[uid_s]];
-    Real ax = 0, ay = 0;
-    Real psum = 0;
-    double wl[sizeof(Real) == 8 ? SC_MAX_NEIGHBORS : 1];  // fp64 only: np.sum's pairwise order needs the list
-    double2 ps64 = make_double2(0, 0);
-    float2 rs = make_float2(0, 0);
-    float df = 0;
-    if constexpr (sizeof(Real) == 8) ps64 = pos[s]; else { rs = rel[s]; df = (float)g.d; }
+    double ax = 0, ay = 0;
+    double wl[SC_MAX_NEIGHBORS];  // np.sum's pairwise order needs the list
+    const double2 ps64 = pos[s];
     for (int k = 0; k < K; ++k) {
-        const uint32_t e = lst.get(k);
-        const uint32_t j = e & SC_IDX_MASK;
-        PairGeom<Real> pg;
-        if constexpr (sizeof(Real) == 8) {
-            pg = pair_geom_f64<kNoise>(P, ps64, pos[j], uid_s, uid[j], host_noise, nbase + (uint32_t)k);
-        } else {
-            const uint32_t cx = (e >> 28) & 3u, cy = e >> 30;  // (dc + 1), (dr + 1)
-            const float ox = cx == 0u ? -df : (cx == 2u ? df : 0.0f), oy = cy == 0u ? -df : (cy == 2u ? df : 0.0f);
-            const float2 rj = rel[j];
-            const float rx = (rs.x - rj.x) - ox;
-            const float ry = (rs.y - rj.y) - oy;
-            pg = pair_geom_f32<kNoise>(P, rx, ry, uid_s, uid[j], host_noise, nbase + (uint32_t)k);
-        }
-        PairIO<Real>::store(pair_j, pair_n, (size_t)off + k, j, pg.nx, pg.ny);
-        if constexpr (sizeof(Real) == 8) wl[k] = (double)pg.w; else psum += pg.w;
-        const Real c = (1 - pg.w) * pg.w;
-        const Real tx = c * pg.nx, ty = c * pg.ny;
+        const uint32_t j = lst.get(k) & SC_IDX_MASK;
+        const PairGeom pg = pair_geom_f64<kNoise>(P, ps64, pos[j], uid_s, uid[j], host_noise, nbase + (uint32_t)k);
+        pair_j[(size_t)off + k] = j;
+        pair_n[(size_t)off + k] = make_double2(pg.nx, pg.ny);
+        wl[k] = pg.w;
+        const double c = (1 - pg.w) * pg.w;
+        const double tx = c * pg.nx, ty = c * pg.ny;
         if (k == 0) { ax = tx; ay = ty; } else { ax += tx; ay += ty; }
     }
-    Real p = 0;
+    double p = 0;
     if (K > 0) {
-        Real pr;
-        if constexpr (sizeof(Real) == 8) pr = (Real)np_sum_1d(wl, K) - (Real)P.ignored;
-        else pr = psum - (Real)P.ignored;
-        p = (pr > 0 || pr != pr) ? pr : (Real)0;  // np.maximum(0, pr), crate.py:273
+        const double pr = np_sum_1d(wl, K) - P.ignored;
+        p = (pr > 0 || pr != pr) ? pr : 0.0;  // np.maximum(0, pr), crate.py:273
     }
-    PS<Real> o;
+    PS<double> o;
     o.p = p; o.sx = ax; o.sy = ay; o.pad_ = 0;
     ps_out[s] = o;
 }
@@ -507,81 +398,72 @@ __device__ __forceinline__ void force_tail(uint32_t s, int K, Real p_i, Real tx,
 #ifndef SC_K5_MINBLOCKS
 #define SC_K5_MINBLOCKS 1
 #endif
-template <typename Real, bool kMonitor>
+template <bool kMonitor>
 __global__ void __launch_bounds__(SC_BLOCK, SC_K5_MINBLOCKS)
 k_force(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallParams W,
-        const double2 *pos, const typename Vec2<Real>::type *vel,
-        const uint32_t *pair_j, const typename Vec2<Real>::type *pair_n,
+        const double2 *pos, const double2 *vel,
+        const uint32_t *pair_j, const double2 *pair_n,
         const uint32_t *pair_off, const uint8_t *pair_cnt,
-        const PS<Real> *ps_in, const uint32_t *wall_bits,
+        const PS<double> *ps_in, const uint32_t *wall_bits,
         const uint32_t *wall_slot, const double2 *wall_pre,
-        double2 *pos_out, typename Vec2<Real>::type *vel_out,
+        double2 *pos_out, double2 *vel_out,
         double *monitor, TickDuty duty, NextKeys nk) {
     pdl_enter();
     end_of_tick(duty, n_ptr);
-    typedef typename Vec2<Real>::type R2;
     const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= *n_ptr) return;
-    const PS<Real> me = ps_in[s];
-    const Real p_i = me.p;
+    const PS<double> me = ps_in[s];
+    const double p_i = me.p;
     const uint32_t off = pair_off[s];
     const int K = pair_cnt[s];
-    const Real smooth = (Real)P.smooth, two_target = (Real)(2 * P.target);
-    Real tx = 0, ty = 0;  // F3 sum
-    Real qx = 0, qy = 0;  // F5 sum
-    Real sum_vx = 0, sum_vy = 0;  // fp32 mode: sum of neighbor velocities
+    const double smooth = P.smooth, two_target = 2 * P.target;
+    double tx = 0, ty = 0;  // F3 sum
+    double qx = 0, qy = 0;  // F5 sum
     // batches of SC_K5_BATCH pairs: index loads, then the dependent gathers, then the arithmetic in list order - the loop is
     // latency bound (two dependent L2 round trips per pair), so the loads of a batch are issued back to back
     for (int k0 = 0; k0 < K; k0 += SC_K5_BATCH) {
         uint32_t jj[SC_K5_BATCH];
-        R2 nn[SC_K5_BATCH];
-        PS<Real> pp[SC_K5_BATCH];
-        R2 vv[SC_K5_BATCH];
-#pragma unroll
-        for (int u = 0; u < SC_K5_BATCH; ++u)
-            if (k0 + u < K) PairIO<Real>::load(pair_j, pair_n, (size_t)off + k0 + u, jj[u], nn[u].x, nn[u].y);
+        double2 nn[SC_K5_BATCH];
+        PS<double> pp[SC_K5_BATCH];
 #pragma unroll
         for (int u = 0; u < SC_K5_BATCH; ++u)
             if (k0 + u < K) {
-                pp[u] = ps_in[jj[u]];
-                if constexpr (sizeof(Real) == 4) vv[u] = vel[jj[u]];
+                jj[u] = pair_j[(size_t)off + k0 + u];
+                nn[u] = pair_n[(size_t)off + k0 + u];
             }
 #pragma unroll
         for (int u = 0; u < SC_K5_BATCH; ++u)
+            if (k0 + u < K) pp[u] = ps_in[jj[u]];
+#pragma unroll
+        for (int u = 0; u < SC_K5_BATCH; ++u)
             if (k0 + u < K) {
-                const R2 nv = nn[u];
-                const PS<Real> nb = pp[u];
+                const double2 nv = nn[u];
+                const PS<double> nb = pp[u];
                 // F3 pass 2, crate.py:347-353
-                const Real ddx = me.sx - nb.sx, ddy = me.sy - nb.sy;
-                const Real align = (ddx * nv.x + ddy * nv.y) * smooth;
-                const Real fix = nb.p + p_i - two_target;
-                const Real cc = align + fix;
-                const Real ex = cc * nv.x, ey = cc * nv.y;
+                const double ddx = me.sx - nb.sx, ddy = me.sy - nb.sy;
+                const double align = (ddx * nv.x + ddy * nv.y) * smooth;
+                const double fix = nb.p + p_i - two_target;
+                const double cc = align + fix;
+                const double ex = cc * nv.x, ey = cc * nv.y;
                 // F5, crate.py:301-306
-                const Real ps_ = p_i + nb.p;
-                const Real fx = nv.x * ps_, fy = nv.y * ps_;
+                const double ps_ = p_i + nb.p;
+                const double fx = nv.x * ps_, fy = nv.y * ps_;
                 if (k0 + u == 0) { tx = ex; ty = ey; qx = fx; qy = fy; }
                 else { tx += ex; ty += ey; qx += fx; qy += fy; }
-                if constexpr (sizeof(Real) == 4) { sum_vx += vv[u].x; sum_vy += vv[u].y; }
             }
     }
 
     // own position / velocity are only needed from here on: loading them late keeps the pair loop's register
     // footprint (and with it the occupancy that hides the gather latency of this untiled kernel) small
     const double2 ps_own = pos[s];
-    const R2 v_own = vel[s];
+    const double2 v_own = vel[s];
     const bool touching = (wall_bits[s >> 5] >> (s & 31)) & 1u;
-    force_tail<Real, kMonitor>(s, K, p_i, tx, ty, qx, qy, P, W, ps_own, v_own, touching, wall_slot, wall_pre, pos_out, vel_out,
-                               monitor, n_ptr, nk, [&](Real vx, Real vy, Real &ax, Real &ay) {
-        if constexpr (sizeof(Real) == 8) {
-            for (int q = 0; q < K; ++q) {
-                const R2 vj = vel[PairIO<Real>::load_index(pair_j, pair_n, (size_t)off + q)];
-                const Real ex = vj.x - vx, ey = vj.y - vy;
-                if (q == 0) { ax = ex; ay = ey; } else { ax += ex; ay += ey; }
-            }
-        } else {
-            ax = sum_vx - (Real)K * vx;
-            ay = sum_vy - (Real)K * vy;
+    force_tail<double, kMonitor>(s, K, p_i, tx, ty, qx, qy, P, W, ps_own, v_own, touching, wall_slot, wall_pre, pos_out,
+                                 vel_out, monitor, n_ptr, nk, [&](double vx, double vy, double &ax, double &ay) {
+        for (int q = 0; q < K; ++q) {
+            const double2 vj = vel[pair_j[(size_t)off + q]];
+            const double ex = vj.x - vx, ey = vj.y - vy;
+            if (q == 0) { ax = ex; ay = ey; } else { ax += ex; ay += ey; }
         }
     });
 }

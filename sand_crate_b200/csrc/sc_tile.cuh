@@ -1,5 +1,4 @@
-// sc_tile.cuh - the production (mixed precision, device noise) density kernel: K4 with the neighborhood of a block
-// staged in shared memory.
+// sc_tile.cuh - the mixed-precision pair kernels: K4 and K5 with the neighborhood of a block staged in shared memory.
 //
 // A block owns SC_TILE consecutive particles of the sorted set.  Because the sort is cell-major (row, col, x), every
 // neighbor of those particles lies in one of three CONTIGUOUS windows of the sorted set - the block's own stretch of
@@ -21,11 +20,10 @@
 // arithmetic is identical in both modes, so a particle's result does not depend on which mode its block ran in
 // (the strip decomposition relies on that: a ghost and its owner must compute the same bits).
 //
-// What the kernel computes is what k_density in sc_pair.cuh computes (same reference lines, same list order, same
-// 20-trim, same fp32-screen / fp64-replay acceptance); only the data movement differs.  Measured on B200 (dam-break
-// 1M): 69 -> 59 us.  The same staging for K5 (neighbor pressure / normal / velocity from shared memory instead of
-// gathers) was built and measured SLOWER than the gathering kernel (60 vs 46 us: K5 does too little work per staged
-// byte to pay for the extra barrier and the 3x staging traffic), so K5 stays untiled and reads sorted indices.
+// The neighbor search is the one of k_density in sc_pair.cuh (same reference lines, same list order, same 20-trim, same
+// fp32-screen / fp64-replay acceptance); only the data movement differs, and the pair geometry is fp32.  Measured on
+// B200 (dam-break 1M) against an fp32 K4 that gathered from global memory: 69 -> 59 us.  K5 (k_force_tile) reads the
+// neighbors' pressure, normal and velocity from the same staged windows.
 #pragma once
 #include "sc_pair.cuh"
 
@@ -174,6 +172,41 @@ __device__ __forceinline__ float rsqrt_ftz(float x) {
     asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
+__device__ __forceinline__ float sqrt_ftz(float x) {
+    float r;
+    asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+    return r;
+}
+
+// ------------------------------------------------------------------------------------------------------------
+// The record K4 hands to K5 for each directed pair (i <- j): ONE 8-byte word.
+//   .x  the SMALLER-magnitude component m of the unit vector n_ij, as a full fp32
+//   .y  bits 0..27  the neighbor's index L in the block's frame (staged block: position in W0 | W1 | W2; pass-through
+//                   block: sorted index) - K4 and K5 cut the sorted set into the same blocks and windows, so K5 reads
+//                   its neighbor's (p, s, v) from shared memory at L with no translation
+//       bit 28      which component m is (0: n.x, 1: n.y)
+//       bit 29      sign of the other component, whose magnitude K5 restores as sqrt(1 - m^2) (>= 0.707: well conditioned)
+// The vector K5 sees is good to ~1e-7 (fp32 grade).  Round 1 packed it as two signed 16-bit fractions (1.5e-5 per
+// component): that was 250x coarser than the arithmetic around it and showed in the per-tick velocity INCREMENT.
+__device__ __forceinline__ uint2 pair_encode(uint32_t L, float nx, float ny) {
+    const bool y_small = fabsf(ny) < fabsf(nx);
+    const float m = y_small ? ny : nx, big = y_small ? nx : ny;
+    return make_uint2(__float_as_uint(m), L | (y_small ? 0x10000000u : 0u) | ((__float_as_uint(big) >> 2) & 0x20000000u));
+}
+__device__ __forceinline__ void pair_decode(uint2 r, uint32_t &L, float &nx, float &ny) {
+    const float m = __uint_as_float(r.x);
+    float big = sqrt_ftz(fmaf(-m, m, 1.0f));
+    big = __uint_as_float(__float_as_uint(big) | ((r.y << 2) & 0x80000000u));
+    const bool y_small = (r.y & 0x10000000u) != 0u;
+    nx = y_small ? big : m;
+    ny = y_small ? m : big;
+    L = r.y & SC_IDX_MASK;
+}
+
+// SC_NOISE_HOST: the reference's noise stream.  Pair k of the particle with uid u takes the uniforms
+// u[2 (off[rank_of_uid[u]] + k) + {0, 1}]: off holds CSR offsets in original index order (sc_step_finish) and is only
+// valid until the next count kernel overwrites it.
+struct HostNoise { const double *u; const uint32_t *off, *rank_of_uid; };
 // ------------------------------------------------------------------------------------------------------------
 // K4 body for one particle.  s = sorted index; b[] = the six boundaries of its four candidate ranges as LOCAL
 // indices (m0, m3 | n0, n3 | p0, p3 of collect_neighbors, shifted into the staged windows).  List order = reference
@@ -182,7 +215,7 @@ template <int kNoise, class Acc, class List>
 __device__ __forceinline__ void density_particle(const Acc &A, List lst, const TileWindows &w, bool live, uint32_t s,
                                                  const uint32_t (&b)[6], const Grid &g, const DevParams &P,
                                                  const double2 *pos, uint2 *pair_rec,
-                                                 uint8_t *pair_cnt, PS<float> *ps_out) {
+                                                 uint8_t *pair_cnt, PS<float> *ps_out, const HostNoise &hn) {
     const float df = P.f_d;
     const uint32_t d0 = w.off[0] - w.base[0], d1 = w.off[1] - w.base[1], d2 = w.off[2] - w.base[2];
     int K = 0;
@@ -236,6 +269,8 @@ __device__ __forceinline__ void density_particle(const Acc &A, List lst, const T
     const uint32_t uid_s = __float_as_uint(me.w);
     const float inv_d = P.f_inv_d;
     const float amp = P.f_amp;
+    uint32_t nbase = 0u;
+    if constexpr (kNoise == SC_NOISE_HOST) nbase = hn.off[hn.rank_of_uid[uid_s]];
     float ax = 0, ay = 0, psum = 0;
     uint2 *out = pair_rec + (size_t)blockIdx.x * (SC_MAX_NEIGHBORS * SC_TILE) + threadIdx.x;
     for (int k = 0; k < K; ++k) {
@@ -250,6 +285,11 @@ __device__ __forceinline__ void density_particle(const Acc &A, List lst, const T
             pair_noise_f32_1to2(pair_noise_bits(P.tick_key, uid_s, __float_as_uint(r.w)), fx, fy);
             rx = fmaf(1.5f - fx, amp, rx);  // 0.5 - u, exact
             ry = fmaf(1.5f - fy, amp, ry);
+        } else if constexpr (kNoise == SC_NOISE_HOST) {
+            const size_t q = 2 * (size_t)(nbase + (uint32_t)k);
+            const float ux = (float)hn.u[q], uy = (float)hn.u[q + 1];
+            rx = fmaf(0.5f - ux, amp, rx);
+            ry = fmaf(0.5f - uy, amp, ry);
         }
         const float q = fmaf(rx, rx, ry * ry);
         const float inv = rsqrt_ftz(q);
@@ -283,7 +323,8 @@ __global__ void __launch_bounds__(SC_TILE, SC_TILE_RESIDENT / SC_TILE)
 k_density_tile(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
                const BlockDesc *desc, const double2 *pos,
                const SearchRec *rec, const uint32_t *cell_key,
-               uint2 *pair_rec, uint8_t *pair_cnt, PS<float> *ps_out, NextWallClear next) {
+               uint2 *pair_rec, uint8_t *pair_cnt, PS<float> *ps_out, NextWallClear next,
+               HostNoise hn) {  // last: the other parameters keep their offsets in every instantiation
     pdl_enter();
     clear_next_walls(next);
     // staged: [records 20 KB | cell boundaries 4.7 KB | 16-bit lists 10 KB]; pass-through: [32-bit lists 20 KB]
@@ -341,7 +382,7 @@ k_density_tile(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
             b[4] = r2[0] + d2; b[5] = r2[3] + d2;
         }
         density_particle<kNoise>(SmemAcc<SearchRec>{smem_addr_pinned(s_rec)}, TileList<uint16_t, 13>{s_list + threadIdx.x}, w, live,
-                                 s, b, g, P, pos, pair_rec, pair_cnt, ps_out);
+                                 s, b, g, P, pos, pair_rec, pair_cnt, ps_out, hn);
     } else {
         if (threadIdx.x == 0) atomicAdd(&cnt->n_untiled, 1u);  // rare; lets a test prove this path ran
         if (live) {
@@ -352,15 +393,15 @@ k_density_tile(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
         }
         density_particle<kNoise>(GmemAcc<SearchRec>{rec},
                                  TileList<uint32_t, 28>{reinterpret_cast<uint32_t *>(s_raw) + threadIdx.x}, w,
-                                 live, s, b, g, P, pos, pair_rec, pair_cnt, ps_out);
+                                 live, s, b, g, P, pos, pair_rec, pair_cnt, ps_out, hn);
     }
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// K5 (mixed mode, device noise): the same blocks and windows as K4.  The neighbors' pressure / surface normal
+// K5 (mixed mode): the same blocks and windows as K4.  The neighbors' pressure / surface normal
 // (16 bytes) and velocity (8 bytes) are bulk-copied into shared memory while the threads fetch their own record
 // offsets; the pair loop then reads ld.shared.v4 / .v2 at the local index the pair record carries, instead of two
-// dependent global gathers per pair (which made the untiled kernel latency bound at 38 % occupancy).
+// dependent global gathers per pair (which made a gathering K5 latency bound at 38 % occupancy).
 // Round 1 built this with a load/store staging loop and measured it SLOWER than gathering (60 vs 46 us): the loop's
 // instructions, its registers in flight and its barrier cost more than the gathers saved.  The bulk copy has none of
 // the three.
@@ -468,9 +509,9 @@ k_force_tile(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallPar
 // block here is a block of the tiled kernels and its record region and windows are theirs.  Read-only on the step's
 // buffers.  A record whose index does not map into the live set (which a correct run never writes) is reported as
 // row -2 instead of being followed.
-enum TapPairPath { TAP_PAIRS_F64 = 0, TAP_PAIRS_UNTILED = 1, TAP_PAIRS_TILED = 2 };
+// `f64`: the fp64 kernels' records (index + vector arrays behind pair_off), else the tiled kernels' (sc_tile.cuh).
 __global__ void __launch_bounds__(SC_TILE)
-k_tap_pair_records(const uint32_t *n_ptr, int path, const BlockDesc *desc, const uint8_t *pair_cnt,
+k_tap_pair_records(const uint32_t *n_ptr, bool f64, const BlockDesc *desc, const uint8_t *pair_cnt,
                    const uint32_t *pair_off, const uint32_t *pair_j, const void *pair_n, const uint32_t *uid,
                    const uint32_t *rank_of_uid, int *cnt_out, int *row_out, double2 *vec_out) {
     const uint32_t n = *n_ptr;
@@ -480,24 +521,22 @@ k_tap_pair_records(const uint32_t *n_ptr, int path, const BlockDesc *desc, const
     const int K = pair_cnt[s];
     cnt_out[r] = K;
     TileWindows w{};
-    if (path == TAP_PAIRS_TILED) w = tile_windows(desc + blockIdx.x);
+    if (!f64) w = tile_windows(desc + blockIdx.x);
     for (int k = 0; k < SC_MAX_NEIGHBORS; ++k) {
         const size_t o = (size_t)r * SC_MAX_NEIGHBORS + k;
         if (k >= K) { row_out[o] = -1; vec_out[o] = make_double2(0, 0); continue; }
         uint32_t j;
         double2 v;
-        if (path == TAP_PAIRS_F64) {
+        if (f64) {
             const size_t i = (size_t)pair_off[s] + k;
             j = pair_j[i];
             v = reinterpret_cast<const double2 *>(pair_n)[i];
         } else {
             const uint2 *rec = reinterpret_cast<const uint2 *>(pair_n);
-            const uint2 e = path == TAP_PAIRS_TILED ? rec[((size_t)blockIdx.x * SC_MAX_NEIGHBORS + k) * SC_TILE + threadIdx.x]
-                                                    : rec[(size_t)pair_off[s] + k];
             float nx, ny;
-            pair_decode(e, j, nx, ny);
+            pair_decode(rec[((size_t)blockIdx.x * SC_MAX_NEIGHBORS + k) * SC_TILE + threadIdx.x], j, nx, ny);
             v = make_double2((double)nx, (double)ny);
-            if (path == TAP_PAIRS_TILED && w.staged) {  // local index in W0 | W1 | W2 -> sorted index
+            if (w.staged) {  // local index in W0 | W1 | W2 -> sorted index
                 uint32_t m = 0xFFFFFFFFu;
                 for (int q = 0; q < 3; ++q)
                     if (j >= w.off[q] && j < w.off[q] + w.cnt[q]) m = w.base[q] + (j - w.off[q]);

@@ -3,8 +3,8 @@
 `Context.get_pair_records` (sc_debug_pair_records) returns what the last tick's density kernel handed to its force
 kernel: K_i, the neighbors in list order and the unit vectors as the force kernel decodes them.  `get_neighbors` re-runs
 the untiled count kernel instead, so only this tap shows the tiled kernel's own lists.  Every case takes ONE step from
-identical inputs and compares with `oracle.step(..., want_all=True)`, in three modes: fp64, mixed precision with
-counter noise (the tiled kernels), and mixed precision without noise (`k_density_tile<SC_NOISE_NONE>`).
+identical inputs and compares with `oracle.step(..., want_all=True)`: in fp64, and through the tiled mixed-precision
+kernels with counter noise, without noise, and with the reference's noise stream from the host (a split step).
 
 The scenes aim at the places a tiled kernel can be wrong while a random scene still passes: pairs inside the fp32
 screen's band around d (the fp64 replay, per range and column offset), cell borders, the 20-trim in each of the four
@@ -59,7 +59,9 @@ MODES = {
     "mixed_counter": (_lib.PRECISION_MIXED, _lib.NOISE_COUNTER, None),
     "mixed_none": (_lib.PRECISION_MIXED, _lib.NOISE_NONE, None),
     "mixed_level0": (_lib.PRECISION_MIXED, _lib.NOISE_COUNTER, 0.0),   # counter mode with a zero noise level
+    "mixed_host": (_lib.PRECISION_MIXED, _lib.NOISE_HOST, None),       # uniforms from the host, split step
 }
+ORACLE_NOISE = {_lib.NOISE_NONE: 0, _lib.NOISE_COUNTER: 1, _lib.NOISE_HOST: 2}
 NO_WALLS = (np.zeros((0, 4)), np.zeros(0, np.int32), np.zeros((0, 5)))
 BOX_WALLS = (np.array(UNIT_BOX["fixed"]["segments"], np.float64).reshape(-1, 4), np.array([4], np.int32),
              np.zeros((1, 5)))
@@ -309,10 +311,16 @@ def run_step(pos, vel, mode, d, walls=NO_WALLS, seed=17, tick=5):
     ctx.set_noise(noise, seed)
     ctx.set_state(pos, vel)
     ctx.set_tick(tick)
-    ctx.step()
+    host = None
+    if noise == _lib.NOISE_HOST:
+        _, n_pairs = ctx.step_begin()
+        host = np.random.RandomState(seed).rand(n_pairs, 2)
+        ctx.step_finish(host)
+    else:
+        ctx.step()
     tkey = O.tick_key(seed, tick)
-    ref = O.step(cv, pos, vel, *walls, noise_mode=0 if noise == _lib.NOISE_NONE else 1, tkey=tkey, want_all=True)
-    return ctx, ref, cv, vel, tkey
+    ref = O.step(cv, pos, vel, *walls, noise_mode=ORACLE_NOISE[noise], noise=host, tkey=tkey, want_all=True)
+    return ctx, ref, cv, vel, tkey, host
 
 
 def ref_vectors(ref, cv, noise_on, tkey=None, host_noise=None):
@@ -392,8 +400,8 @@ def predicted_blocks(ctx, ref, d):
 
 def run_case(pos, mode, d, walls=NO_WALLS, vel=None, seed=17):
     vel = np.zeros_like(pos) if vel is None else vel
-    ctx, ref, cv, vin, tkey = run_step(pos, vel, mode, d, walls, seed)
-    check_records(ctx, ref, cv, mode, tkey)
+    ctx, ref, cv, vin, tkey, host = run_step(pos, vel, mode, d, walls, seed)
+    check_records(ctx, ref, cv, mode, tkey, host)
     return ctx, ref, cv, vin
 
 
@@ -468,7 +476,7 @@ def test_band_lattice_staged(mode):
 
 
 @gpu
-@pytest.mark.parametrize("mode", ["mixed_counter", "mixed_none", "f64"])
+@pytest.mark.parametrize("mode", ["mixed_counter", "mixed_none", "mixed_host", "f64"])
 def test_band_lattice_pass_through(mode):
     d = 2.0 ** -10
     pos = scene_band_pass_through(d)
@@ -499,7 +507,7 @@ def test_cell_borders(mode):
 
 
 @gpu
-@pytest.mark.parametrize("mode", ["f64", "mixed_counter", "mixed_none"])
+@pytest.mark.parametrize("mode", ["f64", "mixed_counter", "mixed_none", "mixed_host"])
 def test_trim_in_every_range(mode):
     d = 1e-3
     pos = scene_trim_clumps(d, duplicates=MODES[mode][1] != _lib.NOISE_NONE)
@@ -529,7 +537,7 @@ def test_block_shapes_small_n(n):
 
 
 @gpu
-@pytest.mark.parametrize("mode", ["mixed_counter", "mixed_none", "mixed_level0", "f64"])
+@pytest.mark.parametrize("mode", ["mixed_counter", "mixed_none", "mixed_level0", "mixed_host", "f64"])
 def test_block_kinds_predicted_exactly(mode):
     """One scene with every block kind: staged, staged windows with cell slices from global memory (a block wrapping a
     row end), pass-through; records beyond the staged slots (K > SC_K5_ROWS) and K == 0."""
@@ -548,8 +556,8 @@ def test_block_kinds_predicted_exactly(mode):
 
 @gpu
 @pytest.mark.parametrize("name", step_goldens()[::3])
-def test_golden_steps_untiled_mixed_kernels(name):
-    """Host noise: the untiled mixed-precision kernels, whose records hold sorted indices."""
+def test_golden_steps_tiled_host_noise(name):
+    """Host noise through the tiled kernels on the recorded scenes (walls, moving bodies)."""
     g = golden(name)
     ctx = _lib.Context(max(len(g["pos_in"]), 1), _lib.PRECISION_MIXED)
     ctx.set_params(**params_from_coeffs(g["coeffs"]))
@@ -576,6 +584,28 @@ def test_tap_refuses_before_a_step():
     ctx.set_params(**params_from_coeffs(coeffs_for(1e-3)))
     with pytest.raises(_lib.SandCrateError, match="no search state"):
         ctx.get_pair_records(4)
+
+
+@gpu
+@pytest.mark.parametrize("mode", ["f64", "mixed_counter", "mixed_level0", "mixed_host"])
+def test_debug_rerun_repeats_the_step_kernels(mode):
+    """sc_debug_rerun re-runs the kernels the step ran, with its effective noise mode: state and records are unchanged.
+    Under host noise it refuses (-1): the noise offsets need not outlive the step."""
+    d = 1e-3
+    pos = scene_blob(3000, d)
+    ctx, ref, cv, vin, tkey, host = run_step(pos, np.zeros_like(pos), mode, d, BOX_WALLS)
+    if mode != "mixed_host":
+        ctx.step()                     # this step's force kernel also keys the next tick: the rerun must drop that
+    n = len(pos)
+    before = ctx.get_state() + ctx.get_pair_records(n)
+    rerun = lambda which: ctx._L.sc_debug_rerun(ctx._h, which, 1)
+    if mode == "mixed_host":
+        assert rerun(4) == -1.0 and rerun(5) == -1.0
+    else:
+        assert rerun(4) > 0 and rerun(5) > 0
+    after = ctx.get_state() + ctx.get_pair_records(n)
+    for a, b in zip(before, after):
+        assert np.array_equal(a, b)
 
 
 # ---- the monitor variant against the bulk fast path --------------------------------------------------------------
