@@ -184,6 +184,12 @@ int sc_debug_pair_records(sc_ctx *ctx, int32_t *counts, int32_t *nbr_row, double
 /* the cell grid: grid4 = {row_min, col_min, nrows, ncols}; cell of (row, col) = (row - row_min) * ncols + col - col_min,
  * both clamped to [1, size - 2] */
 int sc_debug_grid(sc_ctx *ctx, int64_t *grid4);
+/* The conservative wall culls of the current walls (never change a result, only skip work), each box / rectangle as
+ * (xmin, xmax, ymin, ymax): rects[12] = safe_contact, safe_ccd, safe_ccd_f32 (widened to double); seg_box[S x 4] =
+ * each segment's box grown by the touch distance; pad_box[2S x 4] = each padded segment's box.  Buffers may be NULL;
+ * the boxes need room for SC_MAX_SEGMENTS rows.  counts[2] = {S, the wall contacts per particle the cell grid has room
+ * for}.  Refused before sc_set_walls. */
+int sc_debug_walls(sc_ctx *ctx, double *rects, double *seg_box, double *pad_box, int32_t *counts);
 
 /* ---- multi-GPU strip decomposition (one context per rank) ------------------------------------------------------ */
 /* The reference's search is already a 1-D strip decomposition in y with strip height one diameter

@@ -102,6 +102,7 @@ SIGNATURES = {
     "sc_debug_untiled_blocks": (C.c_int64, [_ctx]),
     "sc_debug_pair_records": (C.c_int, [_ctx, _ip, _ip, _dp, C.c_int64]),
     "sc_debug_grid": (C.c_int, [_ctx, _lp]),
+    "sc_debug_walls": (C.c_int, [_ctx, _dp, _dp, _dp, _ip]),
 }
 
 _lib = None
@@ -471,6 +472,19 @@ class Context:
         g = np.zeros(4, np.int64)
         self._ck(self._L.sc_debug_grid(self._h, _ptr(g, _lp)))
         return tuple(int(x) for x in g)
+
+    def debug_walls(self):
+        """The wall culls of the current walls (sc_debug_walls): a dict of safe_contact, safe_ccd, safe_ccd_f32 (4 each),
+        seg_box (S x 4), pad_box (2S x 4), each as (xmin, xmax, ymin, ymax), and `contacts`, the wall contacts per
+        particle the cell grid has room for."""
+        rects = np.empty(12)
+        seg_box, pad_box = np.empty((MAX_SEGMENTS, 4)), np.empty((2 * MAX_SEGMENTS, 4))
+        counts = np.zeros(2, np.int32)
+        self._ck(self._L.sc_debug_walls(self._h, _ptr(rects, _dp), _ptr(seg_box, _dp), _ptr(pad_box, _dp),
+                                        _ptr(counts, _ip)))
+        S = int(counts[0])
+        return {"safe_contact": rects[0:4], "safe_ccd": rects[4:8], "safe_ccd_f32": rects[8:12],
+                "seg_box": seg_box[:S].copy(), "pad_box": pad_box[:2 * S].copy(), "contacts": int(counts[1])}
 
 
 def source_uniform(seed: int, tick: int, source_index: int, j: int) -> float:

@@ -46,6 +46,7 @@ struct sc_ctx {
     DevParams dp{};
     Grid grid{};
     WallParams walls{};
+    int grid_contacts = 1;  // wall contacts per particle the cell grid has room for (world_rows); only ever grows
     int noise_mode = SC_NOISE_NONE;
     uint64_t seed = 0, tick = 0;
     // particle state: *_cur = current state (order left by the previous tick), *_srt = this tick's sorted gather
@@ -252,17 +253,30 @@ static int setup_grid(sc_ctx *ctx, double d, int row_min, int row_max, int col_m
 }
 
 static void refresh_wall_boxes(sc_ctx *ctx);
+static int contact_bound(const WallParams &w);
 static int sync_count(sc_ctx *ctx);
+static void refresh_count(sc_ctx *ctx);
 
 #define SC_DIST_ROW_SLACK 96
 #define SC_K5_THREADS 128  // K5 block size: 128 measured 2 us faster than 256 (blocks drain sooner, the gather-latency-bound kernel keeps more warps resident)
 
+// Rows (= columns) of the world box's cell grid.  Live particles satisfy -r <= coord <= 1 + r (crate.py:152) before
+// apply_hard_wall_fix, which adds one push of r - dist <= r per wall contact: with V contacts a particle moves by up to
+// V r.  The grid has room for grid_contacts contacts, so every position the search sees lies in an interior cell (a
+// clamped one would merge rows the reference keeps apart).  With one contact this is the grid of a contact-free scene.
+static void world_rows(const sc_ctx *ctx, long long &lo, long long &hi) {
+    const double d = ctx->dp.d, r = ctx->dp.r, m = r + ctx->grid_contacts * r;
+    lo = (long long)std::floor(-m / d) - 1;
+    hi = (long long)std::floor((1 + m) / d) + 1;
+}
+
 // Cell grid of the world box; in strip mode only the rows this rank can ever hold (its strip, the halo, and the
 // one-row shift the wall fix can add), so clearing and scanning the grid scales with the strip, not the scene.
 static int world_grid(sc_ctx *ctx) {
-    // live particles satisfy -r <= coord <= 1 + r (crate.py:152) and apply_hard_wall_fix moves by < r
-    const double d = ctx->dp.d, r = ctx->dp.r;
-    const int lo = (int)std::floor((-2 * r) / d) - 1, hi = (int)std::floor((1 + 2 * r) / d) + 1;
+    long long wlo, whi;
+    world_rows(ctx, wlo, whi);
+    if (wlo < -(1LL << 30) || whi > (1LL << 30)) return fail(ctx, "cell grid too large for the wall-fix margin");
+    const int lo = (int)wlo, hi = (int)whi;
     int rlo = lo, rhi = hi;
     if (ctx->dist_on) {
         // halo + wall-fix shift + slack for cuts that slide while the partition is re-balanced (sc_dist_set_rows)
@@ -270,7 +284,7 @@ static int world_grid(sc_ctx *ctx) {
         if (ctx->dist.has_lo && ctx->dist.row_lo - margin > rlo) rlo = (int)(ctx->dist.row_lo - margin);
         if (ctx->dist.has_hi && ctx->dist.row_hi + margin < rhi) rhi = (int)(ctx->dist.row_hi + margin);
     }
-    CKR(setup_grid(ctx, d, rlo, rhi, lo, hi));
+    CKR(setup_grid(ctx, ctx->dp.d, rlo, rhi, lo, hi));
     ctx->srt_valid = false; ctx->rows_valid = false;
     return 0;
 }
@@ -413,12 +427,12 @@ extern "C" int sc_set_params(sc_ctx *ctx, const sc_params *p) {
     ctx->hp = *p;
     refresh_dev_params(ctx);
     if (regrid) {
-        // live particles satisfy -r <= coord <= 1 + r (crate.py:152) and apply_hard_wall_fix moves by < r
-        CKR(world_grid(ctx));
         if (ctx->walls_set) {
             sc_pad_segments(&ctx->walls.seg[0][0], ctx->walls.S, ctx->dp.r, &ctx->walls.pad[0][0]);
             refresh_wall_boxes(ctx);
+            ctx->grid_contacts = std::max(ctx->grid_contacts, contact_bound(ctx->walls));
         }
+        CKR(world_grid(ctx));  // room for the wall fix's shift (world_rows)
     }
     ctx->params_set = true;
     return 0;
@@ -486,6 +500,23 @@ static void refresh_wall_boxes(sc_ctx *ctx) {
     }
 }
 
+// The most wall contacts one particle can have: the largest number of touch boxes (seg_box) that share a point.  A
+// contact needs the particle inside its segment's box (the cull of key_particle), so no particle has more.  The deepest
+// point of a set of closed boxes is the lower-left corner of their intersection, (xmin of one box, ymin of another):
+// trying those S^2 points is exact.  At least 1, so a grid is never smaller than a one-contact grid.
+static int contact_bound(const WallParams &w) {
+    int best = 1;
+    for (int i = 0; i < w.S; ++i)
+        for (int j = 0; j < w.S; ++j) {
+            const double x = w.seg_box[i][0], y = w.seg_box[j][2];
+            int n = 0;
+            for (int k = 0; k < w.S; ++k)
+                n += x >= w.seg_box[k][0] && x <= w.seg_box[k][1] && y >= w.seg_box[k][2] && y <= w.seg_box[k][3];
+            best = std::max(best, n);
+        }
+    return best;
+}
+
 extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const int32_t *body_len,
                             const double *body_kin, int nbodies) {
     CKR(enter(ctx, "sc_set_walls"));
@@ -517,6 +548,17 @@ extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const in
     sc_pad_segments(&w.seg[0][0], S, ctx->dp.r, &w.pad[0][0]);
     refresh_wall_boxes(ctx);
     ctx->walls_set = true;
+    // walls that can give a particle more contacts than the grid has room for: a larger grid (never a smaller one, so
+    // a moving body does not re-grid back and forth).  refresh_count carries the live count out of the old cell
+    // array on the stream: no host wait.
+    const int v = contact_bound(w);
+    if (v > ctx->grid_contacts) {
+        if (ctx->in_step) return fail(ctx, "sc_set_walls: walls that need a larger cell grid inside a split step");
+        CKR(drop_keys(ctx));
+        refresh_count(ctx);
+        ctx->grid_contacts = v;
+        CKR(world_grid(ctx));
+    }
     return 0;
 }
 
@@ -1315,6 +1357,21 @@ extern "C" int sc_debug_grid(sc_ctx *ctx, int64_t *grid4) {
     return 0;
 }
 
+// the conservative wall culls refresh_wall_boxes derived from the last sc_set_walls / radius (WallParams)
+extern "C" int sc_debug_walls(sc_ctx *ctx, double *rects, double *seg_box, double *pad_box, int32_t *counts) {
+    CKR(enter(ctx, "sc_debug_walls"));
+    if (!ctx->walls_set) return fail(ctx, "sc_debug_walls: sc_set_walls has not been called");
+    const WallParams &w = ctx->walls;
+    if (rects)
+        for (int q = 0; q < 4; ++q) {
+            rects[q] = w.safe_contact[q]; rects[4 + q] = w.safe_ccd[q]; rects[8 + q] = (double)w.safe_ccd_f32[q];
+        }
+    if (seg_box && w.S) std::memcpy(seg_box, &w.seg_box[0][0], sizeof(double) * 4 * (size_t)w.S);
+    if (pad_box && w.S) std::memcpy(pad_box, &w.pad_box[0][0], sizeof(double) * 8 * (size_t)w.S);
+    if (counts) { counts[0] = w.S; counts[1] = ctx->grid_contacts; }
+    return 0;
+}
+
 // ---- developer aids (declared in include/sandcrate.h under "diagnostics"): re-run one pair kernel of the last tick
 // `reps` times and return the mean milliseconds.  K4 and K5 only read the sorted set, so re-running them is harmless.
 // -1 before a step, inside a split step, and under SC_NOISE_HOST: the step's noise offsets live in count_by_rank, which
@@ -1451,8 +1508,8 @@ extern "C" int sc_dist_set_rows(sc_ctx *ctx, int64_t row_lo, int64_t row_hi) {
     const bool lo_ok = !ctx->dist.has_lo || row_lo - need >= g_lo, hi_ok = !ctx->dist.has_hi || row_hi + need <= g_hi;
     if (!lo_ok || !hi_ok) {
         // the world grid is a superset check: rows of the world box are always inside (world_grid clamps to them)
-        const double d = ctx->dp.d, r = ctx->dp.r;
-        const long long w_lo = (long long)std::floor((-2 * r) / d) - 1, w_hi = (long long)std::floor((1 + 2 * r) / d) + 1;
+        long long w_lo, w_hi;
+        world_rows(ctx, w_lo, w_hi);
         if ((ctx->dist.has_lo && row_lo - need < g_lo && g_lo > w_lo) ||
             (ctx->dist.has_hi && row_hi + need > g_hi && g_hi < w_hi)) {
             CKR(sync_count(ctx));
