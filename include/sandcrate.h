@@ -202,17 +202,20 @@ int sc_debug_walls(sc_ctx *ctx, double *rects, double *seg_box, double *pad_box,
  * (they stay here as ghosts for this tick) and copies owned particles within `halo_rows` of a cut into HALO records;
  * send_*_dev: device buffers of sc_dist_wire_bytes(capacity) bytes (16-byte header with the record count, then 40-byte
  * records), NULL where there is no neighbor.  The unpack appends received migrants as owned particles and received
- * halos as ghosts.  A ghost is simulated like any particle and discarded by the next pack.  With halo_rows >= 4 every
- * owned particle sees the neighbors, pressures and normals of the global computation in the same order:
- * SC_PRECISION_F64 results are bit-identical to a single-GPU run.
+ * halos as ghosts.  A ghost is simulated like any particle and discarded by the next pack.  With the halo the walls
+ * need (sc_dist_halo_rows: 2 + 2 ceil(V r / d) rows for walls that give a particle up to V contacts, 4 for V <= 2)
+ * every owned particle sees the neighbors, pressures and normals of the global computation in the same order:
+ * results are bit-identical to a single-GPU run.  sc_dist_configure, and sc_set_walls on a strip context, refuse
+ * walls that need more halo rows than configured (nothing is launched, the message names the halo needed).
  * The unpack only records the receive buffers: the next step's first kernel appends their records.  Until then the
  * particle state is incomplete, so the next call on the context must be sc_step, sc_step_n or sc_step_begin; only
  * sc_set_tick, sc_synchronize, sc_destroy, sc_last_error, sc_profile_*, sc_launch_count and sc_sync_count may come
  * before it.  Every other call that takes the context returns an error.
  * Restrictions of the strip mode: noise must be SC_NOISE_COUNTER or SC_NOISE_NONE (the reference's global RNG
- * stream cannot be split across ranks); uids must be < 2^31 (bit 31 marks a ghost copy); the host mirror
- * (sand_crate_b200/strips.py) additionally requires closed scenes (no particle sources) and fixed walls; on a context
- * with a neighbor, sc_get_state / sc_get_uids / the parity taps return an error - read back with sc_dist_get_owned. */
+ * stream cannot be split across ranks); uids must be < 2^31 (bit 31 marks a ghost copy); particle sources go through
+ * sc_dist_emit_particles (sc_emit_particles is refused); on a context with a neighbor, sc_get_state / sc_get_uids /
+ * the parity taps return an error - read back with sc_dist_get_owned.  Moving bodies need nothing special: every
+ * rank passes the same walls to sc_set_walls. */
 int64_t sc_dist_wire_bytes(int64_t wire_capacity);
 int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_lo, int64_t row_hi, int halo_rows,
                       int64_t wire_capacity);
@@ -249,6 +252,23 @@ int sc_dist_set_rows(sc_ctx *ctx, int64_t row_lo, int64_t row_hi);
 int sc_dist_set_reach(sc_ctx *ctx, int64_t far_lo, int64_t far_hi);
 /* like sc_set_state but with caller-chosen uids (global particle ids of a partitioned scene) */
 int sc_set_state_uids(sc_ctx *ctx, const double *pos, const double *vel, const uint32_t *uid, int64_t n);
+/* The halo rows a strip needs under walls `segments` (S x 4, as sc_set_walls) for particles of radius
+ * `particle_radius` (see above); -1 for bad arguments.  Host arithmetic, no context. */
+int sc_dist_halo_rows(const double *segments, int S, double particle_radius);
+/* Particle sources on a strip.  sc_dist_owned_count enqueues a kernel that writes this rank's live particles that are
+ * not ghosts to the caller's device word `count_dev` (no host wait); summed over the ranks (e.g. an all-reduce on the
+ * context's stream) it is the scene's particle_count that sc_emit_particles clamps against.  Take it before
+ * sc_dist_pack: last tick's ghosts are excluded and a particle about to migrate is counted once.
+ * sc_dist_emit_particles is sc_emit_particles for a strip: every rank passes the same records, the same
+ * `max_particles` and the same scene-wide `first_uid` (the uid of the tick's first drawn particle; identities advance by
+ * the drawn counts, so the caller tracks it without device data).  The device clamps each source exactly like
+ * sc_emit_particles with particle_count read from `scene_count_dev` (NULL: the caller has proven that the clamp cannot
+ * bind, every drawn particle is emitted), generates the same stream elements and identities, and appends only the
+ * particles whose row floor(y / d) this rank owns, in (source, particle) order.  The next sc_dist_pack sends the ones
+ * within a halo of a cut to the neighbor.  A rank whose capacity is exceeded raises the overflow flag. */
+int sc_dist_owned_count(sc_ctx *ctx, uint32_t *count_dev);
+int sc_dist_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsources, int64_t max_particles,
+                           uint32_t first_uid, const uint32_t *scene_count_dev);
 
 #ifdef __cplusplus
 }

@@ -90,6 +90,9 @@ SIGNATURES = {
     "sc_dist_set_rows": (C.c_int, [_ctx, C.c_int64, C.c_int64]),
     "sc_dist_set_reach": (C.c_int, [_ctx, C.c_int64, C.c_int64]),
     "sc_set_state_uids": (C.c_int, [_ctx, _dp, _dp, _up, C.c_int64]),
+    "sc_dist_halo_rows": (C.c_int, [_dp, C.c_int, C.c_double]),
+    "sc_dist_owned_count": (C.c_int, [_ctx, C.c_void_p]),
+    "sc_dist_emit_particles": (C.c_int, [_ctx, C.POINTER(ScSource), C.c_int, C.c_int64, C.c_uint32, C.c_void_p]),
     "sc_set_monitor": (C.c_int, [_ctx, C.c_int]),
     "sc_get_monitor": (C.c_int, [_ctx, _dp, _lp]),
     "sc_profile_enable": (C.c_int, [_ctx, C.c_int]),
@@ -393,6 +396,17 @@ class Context:
     def dist_set_reach(self, far_lo: int, far_hi: int):
         self._ck(self._L.sc_dist_set_reach(self._h, int(far_lo), int(far_hi)))
 
+    def dist_owned_count(self, count_dev):
+        """Enqueue: this rank's live non-ghost particle count -> the 4-byte device word `count_dev` (no host wait)."""
+        self._ck(self._L.sc_dist_owned_count(self._h, self._devptr(count_dev)))
+
+    def dist_emit_particles(self, records, max_particles: int, first_uid: int, scene_count_dev=None):
+        """Device-side sources on a strip: `records` as for emit_particles, the same on every rank; `scene_count_dev`:
+        a device word holding the scene's particle count, or None where the clamp cannot bind."""
+        arr = (ScSource * len(records))(*[ScSource(*r) for r in records])
+        self._ck(self._L.sc_dist_emit_particles(self._h, arr, len(records), int(max_particles), C.c_uint32(first_uid),
+                                                self._devptr(scene_count_dev)))
+
     def dist_get_owned(self, want_vel=True, want_uid=True, reuse=False):
         """(pos, vel, uid) of the owned particles.  reuse=True: views of page-locked buffers, valid until the next
         reuse=True call; parts not asked for come back as None."""
@@ -496,6 +510,15 @@ def source_uniform(seed: int, tick: int, source_index: int, j: int) -> float:
 
 def wire_bytes(wire_capacity: int) -> int:
     return int(load().sc_dist_wire_bytes(int(wire_capacity)))
+
+
+def dist_halo_rows(segments, particle_radius: float) -> int:
+    """The halo rows a strip needs under these walls (sc_dist_halo_rows; host arithmetic, no GPU needed)."""
+    seg = _f64(segments, 4)
+    h = int(load().sc_dist_halo_rows(_ptr(seg, _dp), seg.shape[0], float(particle_radius)))
+    if h < 0:
+        raise SandCrateError("sc_dist_halo_rows: bad arguments")
+    return h
 
 
 def pad_segments(segments, pad):

@@ -25,8 +25,8 @@ import yaml
 
 from . import _lib
 from .load_config import WorldConfig
-from .particle_source import build_particle_sources
-from .rigid_body import FixedRigidBody, MotoredRigidBody, build_rigid_bodies
+from .particle_source import build_particle_sources, counter_records
+from .rigid_body import advance_bodies, apply_gravity_to_free_bodies, build_rigid_bodies, wall_arrays
 
 _PRECISIONS = {"f64": _lib.PRECISION_F64, "mixed": _lib.PRECISION_MIXED}
 _NOISES = {"reference": _lib.NOISE_HOST, "counter": _lib.NOISE_COUNTER, "none": _lib.NOISE_NONE}
@@ -238,13 +238,7 @@ class Crate:
         """Production mode: the emission counts come from the counter stream (host arithmetic only), the particles
         are generated, clamped to max_particles and appended by the device - no synchronisation (the reference-stream
         path above has to know the live count, which costs a device round trip per tick while sources are active)."""
-        records = []
-        for index, source in enumerate(self.particle_sources):
-            if source.active_ticks <= self.tick:
-                continue
-            count = source.counter_count(_lib.source_uniform(self._noise_seed, self.tick, index, 0), self.dt)
-            if count:
-                records.append(source.emit_record(index, count))
+        records = counter_records(self.particle_sources, self._noise_seed, self.tick, self.dt)
         if records:
             self._ensure_capacity(int(self.max_particles))   # a no-op after the first call: capacity = max_particles
             self._push_params()
@@ -254,14 +248,10 @@ class Crate:
             self._cache = {}
 
     def apply_bodies_velocity(self) -> None:  # crate.py:363-365
-        for body in self.rigid_bodies:
-            body.apply_velocity(self.dt)
+        advance_bodies(self.rigid_bodies, self.dt)
 
     def apply_gravity_to_free_bodies(self) -> None:  # crate.py:311-314 (the particle part runs on the device)
-        for body in self.rigid_bodies:
-            if isinstance(body, (FixedRigidBody, MotoredRigidBody)):
-                continue
-            body.center_velocity = body.center_velocity + self.dt * np.asarray(self.gravity, dtype=np.float64)
+        apply_gravity_to_free_bodies(self.rigid_bodies, self.dt, self.gravity)
 
     def _push_params(self) -> None:
         g = np.asarray(self.gravity, dtype=np.float64)
@@ -273,9 +263,7 @@ class Crate:
                              gravity_x=g[0], gravity_y=g[1])
 
     def _push_walls(self) -> None:
-        body_len = [len(b) for b in self.rigid_bodies]
-        body_kin = [b.kinematics() for b in self.rigid_bodies]
-        self._ctx.set_walls(self.segments, body_len, np.array(body_kin, dtype=np.float64).reshape(-1, 5))
+        self._ctx.set_walls(*wall_arrays(self.rigid_bodies))
 
     # ---- overlay text (crate.py:131-136, 367-371) ------------------------------------------------------------
     @property

@@ -94,6 +94,7 @@ struct sc_ctx {
     bool monitor_on = false;  // ForceMonitor mode: K5 also sums |dv| per force stage
     double *monitor = nullptr; // 6 sums + particle count of the last tick
     bool dist_on = false;     // strip decomposition: particle arrays hold owned + ghost particles
+    bool dist_tail = false;   // strips: sc_dist_emit_particles appended rows behind the last search's sorted order
     DistCfg dist{};
     // [0], [1]: send headers standing in for a missing lower / upper neighbor's; [2].count: the "blocks done"
     // counter of the direct pack kernel (k_dist_pack<..., true>)
@@ -253,7 +254,7 @@ static int setup_grid(sc_ctx *ctx, double d, int row_min, int row_max, int col_m
 }
 
 static void refresh_wall_boxes(sc_ctx *ctx);
-static int contact_bound(const WallParams &w);
+static int contact_bound(const double (*seg_box)[4], int S);
 static int sync_count(sc_ctx *ctx);
 static void refresh_count(sc_ctx *ctx);
 
@@ -270,8 +271,14 @@ static void world_rows(const sc_ctx *ctx, long long &lo, long long &hi) {
     hi = (long long)std::floor((1 + m) / d) + 1;
 }
 
+// Strips (DESIGN.md section 6).  The wall fix moves a particle with V contacts by at most V r, so by at most
+// ceil(V r / d) = ceil(V / 2) rows (d = 2 r); counted on both sides of a cut that is 2 ceil(V / 2) rows, 2 for V <= 2.
+static int wall_fix_rows(int contacts) { return 2 * ((contacts + 1) / 2); }
+// The halo a strip needs: 1 row of neighbors + 1 row for the neighbors' pressures and normals + the wall-fix rows.
+static int halo_needed(int contacts) { return 2 + wall_fix_rows(contacts); }
+
 // Cell grid of the world box; in strip mode only the rows this rank can ever hold (its strip, the halo, and the
-// one-row shift the wall fix can add), so clearing and scanning the grid scales with the strip, not the scene.
+// rows the wall fix can shift a position by), so clearing and scanning the grid scales with the strip, not the scene.
 static int world_grid(sc_ctx *ctx) {
     long long wlo, whi;
     world_rows(ctx, wlo, whi);
@@ -280,7 +287,7 @@ static int world_grid(sc_ctx *ctx) {
     int rlo = lo, rhi = hi;
     if (ctx->dist_on) {
         // halo + wall-fix shift + slack for cuts that slide while the partition is re-balanced (sc_dist_set_rows)
-        const long long margin = ctx->dist.halo + 2 + SC_DIST_ROW_SLACK;
+        const long long margin = ctx->dist.halo + wall_fix_rows(ctx->grid_contacts) + SC_DIST_ROW_SLACK;
         if (ctx->dist.has_lo && ctx->dist.row_lo - margin > rlo) rlo = (int)(ctx->dist.row_lo - margin);
         if (ctx->dist.has_hi && ctx->dist.row_hi + margin < rhi) rhi = (int)(ctx->dist.row_hi + margin);
     }
@@ -430,7 +437,7 @@ extern "C" int sc_set_params(sc_ctx *ctx, const sc_params *p) {
         if (ctx->walls_set) {
             sc_pad_segments(&ctx->walls.seg[0][0], ctx->walls.S, ctx->dp.r, &ctx->walls.pad[0][0]);
             refresh_wall_boxes(ctx);
-            ctx->grid_contacts = std::max(ctx->grid_contacts, contact_bound(ctx->walls));
+            ctx->grid_contacts = std::max(ctx->grid_contacts, contact_bound(ctx->walls.seg_box, ctx->walls.S));
         }
         CKR(world_grid(ctx));  // room for the wall fix's shift (world_rows)
     }
@@ -453,16 +460,19 @@ extern "C" int sc_pad_segments(const double *segments, int S, double pad, double
     return 0;
 }
 
-// bounding boxes for the conservative culls of WallParams (grown so that rounding can never cull a true hit)
+// bounding box of segment (a, b) grown by m (and so that rounding can never cull a true hit)
+static void grow_box(double *box, double ax, double ay, double bx, double by, double m) {
+    const double xmin = std::fmin(ax, bx), xmax = std::fmax(ax, bx), ymin = std::fmin(ay, by), ymax = std::fmax(ay, by);
+    const double scale = std::fmax(1.0, std::fmax(std::fmax(std::fabs(xmin), std::fabs(xmax)),
+                                                  std::fmax(std::fabs(ymin), std::fabs(ymax))));
+    const double e = m * (1.0 + 1e-6) + 1e-12 * scale;
+    box[0] = xmin - e; box[1] = xmax + e; box[2] = ymin - e; box[3] = ymax + e;
+}
+
+// bounding boxes for the conservative culls of WallParams
 static void refresh_wall_boxes(sc_ctx *ctx) {
     WallParams &w = ctx->walls;
-    auto grow = [](double *box, double ax, double ay, double bx, double by, double m) {
-        const double xmin = std::fmin(ax, bx), xmax = std::fmax(ax, bx), ymin = std::fmin(ay, by), ymax = std::fmax(ay, by);
-        const double scale = std::fmax(1.0, std::fmax(std::fmax(std::fabs(xmin), std::fabs(xmax)),
-                                                      std::fmax(std::fabs(ymin), std::fabs(ymax))));
-        const double e = m * (1.0 + 1e-6) + 1e-12 * scale;
-        box[0] = xmin - e; box[1] = xmax + e; box[2] = ymin - e; box[3] = ymax + e;
-    };
+    auto grow = grow_box;
     for (int k = 0; k < w.S; ++k) grow(w.seg_box[k], w.seg[k][0], w.seg[k][1], w.seg[k][2], w.seg[k][3], ctx->dp.touch);
     for (int k = 0; k < 2 * w.S; ++k) grow(w.pad_box[k], w.pad[k][0], w.pad[k][1], w.pad[k][2], w.pad[k][3], 0.0);
     // Largest-area-greedy rectangle inside the world box that meets none of the boxes.  Only ever used as
@@ -504,17 +514,31 @@ static void refresh_wall_boxes(sc_ctx *ctx) {
 // contact needs the particle inside its segment's box (the cull of key_particle), so no particle has more.  The deepest
 // point of a set of closed boxes is the lower-left corner of their intersection, (xmin of one box, ymin of another):
 // trying those S^2 points is exact.  At least 1, so a grid is never smaller than a one-contact grid.
-static int contact_bound(const WallParams &w) {
+static int contact_bound(const double (*seg_box)[4], int S) {
     int best = 1;
-    for (int i = 0; i < w.S; ++i)
-        for (int j = 0; j < w.S; ++j) {
-            const double x = w.seg_box[i][0], y = w.seg_box[j][2];
+    for (int i = 0; i < S; ++i)
+        for (int j = 0; j < S; ++j) {
+            const double x = seg_box[i][0], y = seg_box[j][2];
             int n = 0;
-            for (int k = 0; k < w.S; ++k)
-                n += x >= w.seg_box[k][0] && x <= w.seg_box[k][1] && y >= w.seg_box[k][2] && y <= w.seg_box[k][3];
+            for (int k = 0; k < S; ++k)
+                n += x >= seg_box[k][0] && x <= seg_box[k][1] && y >= seg_box[k][2] && y <= seg_box[k][3];
             best = std::max(best, n);
         }
     return best;
+}
+
+// contact_bound of segments S x 4 whose touch distance is `touch` (host arithmetic, no context)
+static int segment_contact_bound(const double *segments, int S, double touch) {
+    double box[SC_MAX_SEGMENTS][4];
+    for (int k = 0; k < S; ++k)
+        grow_box(box[k], segments[4 * k], segments[4 * k + 1], segments[4 * k + 2], segments[4 * k + 3], touch);
+    return contact_bound(box, S);
+}
+
+static std::string halo_message(const char *who, int contacts, int halo) {
+    return std::string(who) + ": the walls give a particle up to " + std::to_string(contacts) +
+           " wall contacts, so a strip needs halo_rows >= " + std::to_string(halo_needed(contacts)) + " (configured: " +
+           std::to_string(halo) + ")";
 }
 
 extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const int32_t *body_len,
@@ -523,6 +547,10 @@ extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const in
     if (S < 0 || S > SC_MAX_SEGMENTS) return fail(ctx, "sc_set_walls: more than SC_MAX_SEGMENTS segments");
     if (nbodies < 0 || nbodies > SC_MAX_BODIES) return fail(ctx, "sc_set_walls: more than SC_MAX_BODIES bodies");
     if (!ctx->params_set) return fail(ctx, "sc_set_walls: call sc_set_params first (padding needs the radius)");
+    if (ctx->dist_on) {  // a strip's halo must cover the new walls' wall-fix reach: refuse before anything changes
+        const int v = segment_contact_bound(segments, S, ctx->dp.touch);
+        if (halo_needed(v) > ctx->dist.halo) return fail(ctx, halo_message("sc_set_walls", v, ctx->dist.halo));
+    }
     WallParams &w = ctx->walls;
     {   // the same walls again (a Crate pushes them every tick) leave the next tick's keys valid; moving ones do not
         bool same = ctx->walls_set && S == w.S && nbodies == w.nbodies &&
@@ -551,7 +579,7 @@ extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const in
     // walls that can give a particle more contacts than the grid has room for: a larger grid (never a smaller one, so
     // a moving body does not re-grid back and forth).  refresh_count carries the live count out of the old cell
     // array on the stream: no host wait.
-    const int v = contact_bound(w);
+    const int v = contact_bound(w.seg_box, w.S);
     if (v > ctx->grid_contacts) {
         if (ctx->in_step) return fail(ctx, "sc_set_walls: walls that need a larger cell grid inside a split step");
         CKR(drop_keys(ctx));
@@ -991,6 +1019,7 @@ static int enqueue_forces(sc_ctx *ctx, const uint32_t *noise_off) {
     ctx->keys_dropped = false;
     CK(cudaGetLastError());
     ctx->rows_valid = n > 0;
+    ctx->dist_tail = false;
     ctx->tick += 1;  // crate.py:127
     ctx->n_exact = false;
     return 0;
@@ -1471,6 +1500,10 @@ extern "C" int64_t sc_dist_wire_bytes(int64_t wire_capacity) {
 extern "C" int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_lo, int64_t row_hi, int halo_rows,
                                  int64_t wire_capacity) {
     CKR(enter(ctx, "sc_dist_configure"));
+    if (ctx->walls_set) {  // refused before anything is launched
+        const int v = contact_bound(ctx->walls.seg_box, ctx->walls.S);
+        if (halo_rows < halo_needed(v)) return fail(ctx, halo_message("sc_dist_configure", v, halo_rows));
+    }
     CKR(drop_keys(ctx));
     if (nranks < 1 || rank < 0 || rank >= nranks) return fail(ctx, "sc_dist_configure: bad rank");
     if (halo_rows < 1) return fail(ctx, "sc_dist_configure: halo_rows must be >= 1");
@@ -1503,7 +1536,7 @@ extern "C" int sc_dist_set_rows(sc_ctx *ctx, int64_t row_lo, int64_t row_hi) {
     ctx->dist.row_lo = row_lo; ctx->dist.row_hi = row_hi;
     if (!ctx->dist.reach_set) { ctx->dist.far_lo = row_lo - ctx->dist.halo; ctx->dist.far_hi = row_hi + ctx->dist.halo; }
     // the restricted cell grid must still cover the strip, its halo and the wall-fix shift
-    const long long need = ctx->dist.halo + 2;
+    const long long need = ctx->dist.halo + wall_fix_rows(ctx->grid_contacts);
     const long long g_lo = (long long)ctx->grid.row_min + 1, g_hi = (long long)ctx->grid.row_min + ctx->grid.nrows - 2;
     const bool lo_ok = !ctx->dist.has_lo || row_lo - need >= g_lo, hi_ok = !ctx->dist.has_hi || row_hi + need <= g_hi;
     if (!lo_ok || !hi_ok) {
@@ -1579,10 +1612,12 @@ static int enqueue_pack(sc_ctx *ctx, const char *who, void *send_lo_dev, void *s
     const Grid &g = ctx->grid;
     // Boundary zones in sorted-index space (see k_dist_pack).  Rows that can hold a ghost, a migrant or a halo particle:
     // within halo of a cut, plus the rows a particle can cross in a tick (< 2) and a sliding cut can move (<= halo - 2),
-    // on either side.  Valid only while the arrays are still in the order of the last search.
+    // on either side.  Valid only while the arrays are still in the order of the last search.  Particles a source
+    // appended since (dist_tail) sit behind the sorted ones, where only the upper range [B, n) reaches: a rank without an
+    // upper neighbor (B = n) covers everything instead.
     PackRange R{nullptr, 0u, 0u};
     int64_t launch_n = n;
-    if (ctx->rows_valid) {
+    if (ctx->rows_valid && (ctx->dist.has_hi || !ctx->dist_tail)) {
         const long long zone = 2LL * ctx->dist.halo + 4;
         long long ra = ctx->dist.row_lo + zone - g.row_min, rb = ctx->dist.row_hi - zone - g.row_min;
         ra = ra < 0 ? 0 : (ra > g.nrows ? g.nrows : ra);
@@ -1592,7 +1627,9 @@ static int enqueue_pack(sc_ctx *ctx, const char *who, void *send_lo_dev, void *s
         if (ra < rb) {
             R.cell_start = ctx->cell_start;
             R.cell_a = (uint32_t)(ra * g.ncols); R.cell_b = (uint32_t)(rb * g.ncols);
-            const int64_t zone_cap = 4LL * ctx->dist.cap;   // wire capacity is 4 (halo + 2) rows' worth: ample for two zones
+            // grid size only (the blocks stride over the whole work list): the default wire capacity is 4 (halo + 2)
+            // rows' worth, so this covers the two zones of 2 halo + 4 rows at any halo depth
+            const int64_t zone_cap = 4LL * ctx->dist.cap;
             launch_n = std::min<int64_t>(n, zone_cap);
         }
     }
@@ -1702,5 +1739,69 @@ extern "C" int sc_dist_status(sc_ctx *ctx, const void *send_lo_dev, const void *
     if (n_local) *n_local = h.n;
     ctx->n_host = ctx->cap;  // back to the conservative launch bound (sync_count narrowed it)
     ctx->n_exact = false;
+    return 0;
+}
+
+extern "C" int sc_dist_halo_rows(const double *segments, int S, double particle_radius) {
+    if (S < 0 || S > SC_MAX_SEGMENTS || (S && !segments) || !(particle_radius > 0)) return -1;
+    return halo_needed(segment_contact_bound(segments, S, particle_radius * 1.2));  // touch: refresh_dev_params
+}
+
+extern "C" int sc_dist_owned_count(sc_ctx *ctx, uint32_t *count_dev) {
+    CKR(dist_ready(ctx, "sc_dist_owned_count"));
+    if (!count_dev) return fail(ctx, "sc_dist_owned_count: NULL argument");
+    refresh_count(ctx);
+    CK(cudaMemsetAsync(count_dev, 0, sizeof(uint32_t), ctx->stream));
+    if (ctx->n_host > 0) {
+        ProfScope ps(ctx, SLOT_IO);
+        const unsigned nb = std::min<unsigned>(blocks_for(ctx->n_host), 4 * 148);  // grid-stride over the live count
+        k_dist_owned_count<<<nb, SC_BLOCK, 0, ctx->stream>>>(&ctx->cnt->n, ctx->uid_cur, count_dev);
+    }
+    CK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int sc_dist_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsources, int64_t max_particles,
+                                      uint32_t first_uid, const uint32_t *scene_count_dev) {
+    CKR(dist_ready(ctx, "sc_dist_emit_particles"));
+    if (nsources > 0 && !sources) return fail(ctx, "sc_dist_emit_particles: NULL argument");
+    if (nsources < 0 || nsources > SC_MAX_SOURCES)
+        return fail(ctx, "sc_dist_emit_particles: more than SC_MAX_SOURCES sources");
+    EmitParams E{};
+    E.nsrc = 0;
+    E.max_particles = (uint32_t)std::min<int64_t>(std::max<int64_t>(max_particles, 0), 0xFFFFFFFFLL);  // scene-wide
+    uint64_t total = 0;
+    const uint64_t tkey = tick_key(ctx->seed, ctx->tick);
+    for (int q = 0; q < nsources; ++q) {
+        if (sources[q].count <= 0) continue;
+        EmitSource &S = E.src[E.nsrc++];
+        S.px = sources[q].position_x; S.py = sources[q].position_y; S.radius = sources[q].radius;
+        S.vx = sources[q].velocity_x; S.vy = sources[q].velocity_y; S.vnoise = sources[q].velocity_noise;
+        S.key = source_key(tkey, sources[q].index);
+        S.n = (uint32_t)sources[q].count;
+        S.uid_base = first_uid + (uint32_t)total;   // as sc_emit_particles: identities advance by the DRAWN count
+        total += S.n;
+    }
+    if (!E.nsrc) return 0;
+    if ((uint64_t)first_uid + total >= (uint64_t)SC_GHOST_BIT)
+        return fail(ctx, "particle identities exhausted (2^31 particles created in this scene)");
+    CKR(drop_keys(ctx));  // the new particles have no keys
+    refresh_count(ctx);
+    {
+        ProfScope ps(ctx, SLOT_IO);
+        if (ctx->precision == SC_PRECISION_F64)
+            CK(launch_pdl(k_dist_emit<double>, dim3(1), dim3(SC_BLOCK), ctx->stream, ctx->cnt, E, scene_count_dev, ctx->grid,
+                          ctx->dist.row_lo, ctx->dist.row_hi, ctx->pos_cur, (double2 *)ctx->vel_cur, ctx->uid_cur,
+                          (uint32_t)ctx->cap));
+        else
+            CK(launch_pdl(k_dist_emit<float>, dim3(1), dim3(SC_BLOCK), ctx->stream, ctx->cnt, E, scene_count_dev, ctx->grid,
+                          ctx->dist.row_lo, ctx->dist.row_hi, ctx->pos_cur, (float2 *)ctx->vel_cur, ctx->uid_cur,
+                          (uint32_t)ctx->cap));
+    }
+    ctx->next_uid = std::max<uint32_t>(ctx->next_uid, first_uid + (uint32_t)total);
+    ctx->n_host = std::min<int64_t>(ctx->n_host + (int64_t)total, ctx->cap);  // an upper bound
+    ctx->n_exact = false;
+    ctx->srt_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
+    ctx->dist_tail = true;  // behind the sorted rows: the next pack must reach them (enqueue_pack)
     return 0;
 }

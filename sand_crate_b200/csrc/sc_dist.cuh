@@ -226,6 +226,76 @@ k_dist_row_hist(const uint32_t *n_ptr, Grid g, const double2 *pos,
     if (threadIdx.x < SC_HIST_WIN && s_h[threadIdx.x]) atomicAdd(&hist[base + threadIdx.x], (unsigned long long)s_h[threadIdx.x]);
 }
 
+// live particles that are not ghosts, added to *out (zeroed by the caller): this rank's share of the scene's count
+__global__ void __launch_bounds__(SC_BLOCK)
+k_dist_owned_count(const uint32_t *n_ptr, const uint32_t *uid, uint32_t *out) {
+    const uint32_t n = *n_ptr;
+    uint32_t c = 0u;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        c += (uid[i] & SC_GHOST_BIT) ? 0u : 1u;
+    c = __reduce_add_sync(0xffffffffu, c);
+    if ((threadIdx.x & 31) == 0 && c) atomicAdd(out, c);
+}
+
+// Particle sources on a strip (sc_dist_emit_particles).  k_emit's clamp with P = the SCENE's count (*scene_n, summed
+// over the ranks by the caller; NULL = the clamp cannot bind) - the same count, the same stream elements and identities
+// on every rank - but a rank appends only the particles whose row floor(y / d) it owns, in (source, k) order: a
+// block-wide ordered compaction per SC_BLOCK candidates.  The pack of the same tick hands the ones near a cut on as
+// halos (enqueue_pack: the appended tail is part of its work list).
+template <typename Real>
+__global__ void __launch_bounds__(SC_BLOCK)
+k_dist_emit(Counters *cnt, const __grid_constant__ EmitParams E, const uint32_t *scene_n, Grid g, long long row_lo,
+            long long row_hi, double2 *pos, typename Vec2<Real>::type *vel, uint32_t *uid, uint32_t cap) {
+    pdl_enter();
+    __shared__ uint32_t s_cnt[SC_MAX_SOURCES], s_at;
+    if (threadIdx.x == 0) {
+        uint32_t P = scene_n ? *scene_n : 0u;
+        for (int q = 0; q < E.nsrc; ++q) {
+            uint32_t a = E.src[q].n;
+            if (scene_n) {
+                const uint32_t room = E.max_particles > P ? E.max_particles - P : 0u;
+                a = a < room ? a : room;
+            }
+            s_cnt[q] = a;
+            P += a;
+        }
+        s_at = cnt->n;
+    }
+    __syncthreads();
+    uint32_t at = s_at;
+    for (int q = 0; q < E.nsrc; ++q) {
+        const EmitSource &S = E.src[q];
+        for (uint32_t k0 = 0; k0 < s_cnt[q]; k0 += blockDim.x) {   // uniform trip count: the scan needs every thread
+            const uint32_t k = k0 + threadIdx.x;
+            bool mine = false;
+            double2 p = make_double2(0, 0);
+            typename Vec2<Real>::type v;
+            if (k < s_cnt[q]) {
+                const double ux = source_uniform(S.key, 1ull + 4ull * k), uy = source_uniform(S.key, 2ull + 4ull * k);
+                const double wx = source_uniform(S.key, 3ull + 4ull * k), wy = source_uniform(S.key, 4ull + 4ull * k);
+                p = make_double2((ux - 0.5) * S.radius + S.px, (uy - 0.5) * S.radius + S.py);   // as k_emit
+                v.x = (Real)(S.vx + (wx - 0.5) * S.vnoise);
+                v.y = (Real)(S.vy + (wy - 0.5) * S.vnoise);
+                const double fr = floor_div(p.y, g);   // the pack's row rule
+                const long long row = (fr >= -9.0e18 && fr <= 9.0e18) ? (long long)fr : 0;
+                mine = row >= row_lo && row < row_hi;
+            }
+            uint32_t total;
+            const uint32_t i = at + block_exclusive_scan(mine ? 1u : 0u, total);
+            if (mine && i < cap) {
+                pos[i] = p;
+                vel[i] = v;
+                uid[i] = S.uid_base + k;
+            }
+            at += total;
+        }
+    }
+    if (threadIdx.x == 0) {
+        if (at > cap) { at = cap; cnt->overflow = 1u; }
+        cnt->n = at;
+    }
+}
+
 __global__ void k_wire_reset(WireHeader *a, WireHeader *b) {
     a->count = 0; a->overflow = 0; a->too_far = 0; a->pad_ = 0;
     b->count = 0; b->overflow = 0; b->too_far = 0; b->pad_ = 0;

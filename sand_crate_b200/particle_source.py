@@ -71,5 +71,20 @@ class ParticleSource:
                 float(self.velocity[1]), float(self.noise), int(count), int(index))
 
 
+def counter_records(sources, seed: int, tick: int, dt: float) -> list[tuple]:
+    """The `sc_source` records of the sources that emit at `tick` in the counter mode: each count drawn from element 0
+    of the source's counter stream (host arithmetic, no device data), so every caller - one context or every rank of a
+    strip-decomposed scene - draws the same ones."""
+    from . import _lib
+    records = []
+    for index, source in enumerate(sources):
+        if source.active_ticks <= tick:
+            continue
+        count = source.counter_count(_lib.source_uniform(seed, tick, index, 0), dt)
+        if count:
+            records.append(source.emit_record(index, count))
+    return records
+
+
 def build_particle_sources(particle_source_configs) -> list[ParticleSource]:
     return [ParticleSource(**cfg) for cfg in (particle_source_configs or [])]

@@ -102,6 +102,26 @@ class MotoredRigidBody(RigidBody):
         super().apply_velocity(dt)
 
 
+def advance_bodies(bodies, dt: float) -> None:
+    """apply_bodies_velocity (crate.py:363-365): every body's motion law for one tick."""
+    for body in bodies:
+        body.apply_velocity(dt)
+
+
+def apply_gravity_to_free_bodies(bodies, dt: float, gravity) -> None:
+    """The rigid-body part of crate.py:311-314 (the particle part runs on the device)."""
+    for body in bodies:
+        if isinstance(body, (FixedRigidBody, MotoredRigidBody)):
+            continue
+        body.center_velocity = body.center_velocity + dt * np.asarray(gravity, dtype=np.float64)
+
+
+def wall_arrays(bodies):
+    """The `sc_set_walls` arguments of `bodies`: segments S x 2 x 2, segments per body, kinematics nbodies x 5."""
+    seg = np.vstack([b.segments for b in bodies]) if bodies else np.zeros((0, 2, 2))
+    return seg, [len(b) for b in bodies], np.array([b.kinematics() for b in bodies], dtype=np.float64).reshape(-1, 5)
+
+
 BODY_TYPE_TO_CLASS = {"motored": MotoredRigidBody, "fixed": FixedRigidBody, "free": RigidBody}
 
 

@@ -86,6 +86,33 @@ def dam_break_wide(n: int, seed: int = 42, **overrides):
     return dam_break(n, seed, width=0.5, height=0.98, **overrides)
 
 
+# wave_machine.yaml's paddle: a thin rectangle against the right wall, rocking about its top corner (placed in the unit box)
+WAVE_PADDLE = {"motored": {"name": "moving_wall", "segments": [
+    [[0.0, 0.0], [0.0, -1.0]], [[0.0, 0.0], [-1.0, 0.0]], [[-1.0, 0.0], [-1.0, -1.0]], [[0.0, -1.0], [-1.0, -1.0]]],
+    "angular_velocity_func": "lambda t: np.cos(t * 8) * 1.5", "scale": [0.02, 0.9], "rotation": -12,
+    "position": [1.0, 1.3]}}
+
+
+def wave_tank(n: int, seed: int = 42, depth: float = 0.4, flow_fraction: float = 1.0, **overrides):
+    """An OPEN scene at size (strip decomposition with sources and moving bodies): wave_machine.yaml's paddle in the unit
+    box, a liquid bed of n particles filling the bottom `depth` of the box (lattice as dam_break), and one source pouring
+    from the upper left.  Scaling as the other scenes: d from the lattice, dt with d, and so the paddle's motion law
+    (physical time) moves it by the same number of rows per tick at any n.  The source runs for 0.5 s of physical time
+    at `flow_fraction * n` particles per second (Binomial(flow, dt) per tick); max_particles = n + 0.25 * flow, so the
+    clamp binds halfway through - override it to move that point."""
+    d, lat = _dam_break_geometry(n, 0.98, depth)
+    pts = _lattice(*lat, seed)
+    world = _world(n, d, **overrides)
+    flow = float(flow_fraction * n)
+    dt = world.coefficients["dt"]
+    world.rigid_bodies = [UNIT_BOX, WAVE_PADDLE]
+    world.particle_sources = [{"radius": 0.05, "position": [0.1, 0.1], "velocity": [2.0, 0.0], "flow": flow,
+                               "noise": 0.05, "active_ticks": int(round(0.5 / dt))}]
+    if "max_particles" not in overrides:
+        world.coefficients["max_particles"] = int(n + 0.25 * flow)
+    return world, pts, np.zeros_like(pts)
+
+
 SCENES = {"dam_break": dam_break, "box_fill": box_fill, "dam_break_wide": dam_break_wide}
 
 

@@ -23,7 +23,8 @@ import numpy as np
 
 from . import _lib
 
-HALO_ROWS = 4  # see DESIGN.md section 6: 1 row of neighbors + 1 row for their pressures/normals + 2 for wall-fix shifts
+HALO_ROWS = 4  # DESIGN.md section 6: 1 row of neighbors + 1 for their pressures / normals + 2 for wall-fix shifts; the
+               # least a strip takes, and what walls with at most 2 contacts per particle need (_lib.dist_halo_rows)
 INT64_MIN, INT64_MAX = -(2 ** 62), 2 ** 62
 
 
@@ -105,6 +106,19 @@ def partition_histogram(hist: np.ndarray, row0: int, nranks: int, halo_rows: int
     return cuts
 
 
+def even_cuts(row0: int, nrows: int, nranks: int) -> list[int]:
+    """Cuts that split the rows [row0, row0 + nrows) evenly: the partition of a scene that starts (nearly) empty, before a
+    re-cut balances it."""
+    return [INT64_MIN] + [row0 + (k * nrows) // nranks for k in range(1, nranks)] + [INT64_MAX]
+
+
+def emission_may_clamp(bound: int, drawn: int, max_particles: int) -> bool:
+    """Can the max_particles clamp of this tick's emission bind?  `bound` is an upper bound on the scene's particle count
+    (the initial count plus every particle drawn so far: removal only lowers the true count), `drawn` this tick's drawn
+    total.  If bound + drawn <= max_particles, every source emits all it drew, whatever the true count is."""
+    return bound + drawn > max_particles
+
+
 def world_rows(particle_radius: float) -> tuple[int, int]:
     """(first row, number of rows) covering every position a live particle can have (crate.py:152: -r <= y <= 1 + r,
     plus the wall fix's shift of < r)."""
@@ -131,33 +145,46 @@ def next_rebalance_interval(every: int, shift: int, first: int, floor: int = 1) 
 class StripDomain:
     """One rank's share of a strip-decomposed scene.
 
-    `world` is a WorldConfig (closed scenes: no particle sources).  The initial scene comes either as `pos` / `vel`
-    (the WHOLE scene, every rank generates it from the same seed and keeps its rows) or as `chunks` (a callable returning
-    an iterator of (first row index, positions): `scenes.scene_chunks`; velocities zero) - the form the 16M / 64M scenes
-    use, so that no rank ever holds the whole scene.  uids are the global row indices of the scene.
+    `world` is a WorldConfig: the whole scene model runs - particle sources, fixed, motored and free bodies, removal.
+    The initial scene comes either as `pos` / `vel` (the WHOLE scene, every rank generates it from the same seed and
+    keeps its rows; omitted: the scene starts empty) or as `chunks` (a callable returning an iterator of (first row
+    index, positions): `scenes.scene_chunks`; velocities zero) - the form the 16M / 64M scenes use, so that no rank ever
+    holds the whole scene.  uids are the global row indices of the scene; emitted particles take the next ones, as in
+    `Crate`.  Every rank evaluates the same body motion laws and draws the same emission counts, so the per-tick scene
+    work is host arithmetic shared with `Crate` (rigid_body.py, particle_source.py).
 
-    Restrictions of the strip mode (they hold for the synthetic multi-GPU configs): closed scenes, fixed walls,
-    counter or no noise."""
+    `halo_rows` defaults to what the tick-0 walls need (`_lib.dist_halo_rows`, at least HALO_ROWS); a later tick whose
+    walls need more raises.  Restrictions of the strip mode: counter or no noise, no live coefficient edits."""
 
     def __init__(self, world, pos=None, vel=None, *, rank: int, world_size: int, precision: str = "mixed",
                  noise: str = "counter", noise_seed: int = 0, device: int = 0, stream: int | None = None,
-                 halo_rows: int = HALO_ROWS, slack: float = 1.3, wire_capacity: int | None = None,
+                 halo_rows: int | None = None, slack: float = 1.3, wire_capacity: int | None = None,
                  context_factory=None, tensor_device=None, comm=None, transport: str = "nccl",
                  rebalance_every: int = 0, cuts: list | None = None, chunks=None, check_every: int = 256,
                  adaptive_rebalance: bool = True):
         import torch
+        from .particle_source import build_particle_sources
+        from .rigid_body import build_rigid_bodies, wall_arrays
 
-        if world.particle_sources:
-            raise ValueError("strip decomposition supports closed scenes only (no particle sources)")
         if noise == "reference":
             raise ValueError("the reference-RNG noise mode is single-GPU only")
         self.rank, self.world_size = rank, world_size
         self.world = world
-        self.halo_rows = halo_rows
         c = world.coefficients
         self.diameter = 2 * c["particle_radius"]
+        self.dt = c["dt"]
+        self.gravity = np.asarray(c["gravity"], dtype=np.float64)
+        self.noise_seed = int(noise_seed)
+        self.bodies = build_rigid_bodies(world.rigid_bodies)
+        self.sources = build_particle_sources(world.particle_sources)
+        self.max_particles = int(c.get("max_particles", 0) or 0)
+        if halo_rows is None:
+            halo_rows = max(HALO_ROWS, _lib.dist_halo_rows(wall_arrays(self.bodies)[0], c["particle_radius"]))
+        self.halo_rows = halo_rows
         self._row0, self._nrows = world_rows(c["particle_radius"])
         if chunks is None:
+            if pos is None:
+                pos, vel = np.zeros((0, 2)), np.zeros((0, 2))
             whole_pos, whole_vel = np.asarray(pos, dtype=np.float64), np.asarray(vel, dtype=np.float64)
             chunks = lambda: iter([(0, whole_pos)])  # noqa: E731
         else:
@@ -169,7 +196,12 @@ class StripDomain:
             r = np.clip(rows_of(p, self.diameter) - self._row0, 0, self._nrows - 1)
             hist += np.bincount(r, minlength=self._nrows)
             n_total += len(p)
-        self.cuts = list(cuts) if cuts is not None else partition_histogram(hist, self._row0, world_size, halo_rows)
+        if cuts is None and n_total:
+            try:
+                cuts = partition_histogram(hist, self._row0, world_size, halo_rows)
+            except ValueError:   # too few occupied rows for the strips: re-cuts balance the scene later
+                cuts = None
+        self.cuts = list(cuts) if cuts is not None else even_cuts(self._row0, self._nrows, world_size)
         assert len(self.cuts) == world_size + 1
         self.row_lo, self.row_hi = self.cuts[rank], self.cuts[rank + 1]
         # pass 2: this rank's rows
@@ -185,9 +217,12 @@ class StripDomain:
         del keep_uid, keep_pos, keep_vel
         self.n_total = n_total
         per_row = max(int(hist.max()), 1)
+        if self.sources:   # rows the sources fill later: a row of liquid at rest holds about 1.8 / d particles
+            per_row = max(per_row, int(np.ceil(2 / self.diameter)))
         self.wire_capacity = int(wire_capacity or max(4 * (halo_rows + 2) * per_row, 1024))
         # room for this rank's share after re-balancing as well as for an unbalanced start
-        capacity = int(max(len(mine), -(-n_total // world_size)) * slack) + 2 * self.wire_capacity + 1024
+        share = -(-max(n_total, self.max_particles) // world_size)
+        capacity = int(max(len(mine), share) * slack) + 2 * self.wire_capacity + 1024
         self.wire_capacity = min(self.wire_capacity, capacity)
         self._torch_stream = None
         if context_factory is None:
@@ -211,18 +246,20 @@ class StripDomain:
                             collider_noise_level=c["collider_noise_level"], viscosity=c["viscosity"],
                             surface_smoothing=c["surface_smoothing"], target_pressure=c["target_pressure"],
                             gravity_x=c["gravity"][0], gravity_y=c["gravity"][1])
-        from .rigid_body import build_rigid_bodies
-        bodies = build_rigid_bodies(world.rigid_bodies)
-        if any(b.kind != "fixed" for b in bodies):
-            raise ValueError("strip decomposition supports fixed walls only")
-        seg = np.vstack([b.segments for b in bodies]) if bodies else np.zeros((0, 2, 2))
-        self.ctx.set_walls(seg, [len(b) for b in bodies], np.array([b.kinematics() for b in bodies]).reshape(-1, 5))
+        self.ctx.set_walls(*wall_arrays(self.bodies))
         self.ctx.set_noise({"counter": _lib.NOISE_COUNTER, "none": _lib.NOISE_NONE}[noise], noise_seed)
         self.ctx.set_state_uids(pos_mine, vel_mine, mine)
         del pos_mine, vel_mine, mine
         self.ctx.dist_configure(rank, world_size, self.row_lo, self.row_hi, halo_rows, self.wire_capacity)
         self._push_reach()
         self.tick = 0
+        # sources: the next scene-wide uid, and an upper bound on the scene's particle count (the initial count plus
+        # every particle drawn: removal only lowers the true count).  While the bound shows that the max_particles
+        # clamp cannot bind, emission needs no device count and no collective (emission_may_clamp).
+        self.next_uid = n_total
+        self.count_bound = n_total
+        self.scene_counts = 0          # ticks whose emission took the scene count from the device (and a collective)
+        self._count_word = None
         # re-balancing: every `rebalance_every` ticks the per-row histogram is summed over the ranks (the scheme's
         # only collective) and the cuts then SLIDE towards the new equal-count positions by at most halo - 2 rows per
         # tick, so the rows a cut hands over travel as ordinary migrants (DESIGN.md section 6)
@@ -383,13 +420,75 @@ class StripDomain:
             self.ctx.dist_set_rows(self.row_lo, self.row_hi)
             self._push_reach()
 
-    def physics_tick(self) -> None:
+    # ---- the phases of one tick (physics_tick runs them in this order; so does the one-GPU lockstep test driver) ----
+    def advance_scene(self) -> None:
+        """Set the tick, move the bodies and push the walls (every rank evaluates the same motion laws).  Walls that
+        need a deeper halo than this strip has make the library raise."""
+        from .rigid_body import advance_bodies, wall_arrays
         self.ctx.set_tick(self.tick)
+        if any(b.kind != "fixed" for b in self.bodies):
+            advance_bodies(self.bodies, self.dt)
+            self.ctx.set_walls(*wall_arrays(self.bodies))
+
+    def draw_emission(self) -> tuple[list, bool]:
+        """This tick's source records (counter stream, host arithmetic) and whether the max_particles clamp may bind,
+        in which case emit() needs the scene's device count."""
+        from .particle_source import counter_records
+        records = counter_records(self.sources, self.noise_seed, self.tick, self.dt)
+        drawn = sum(r[6] for r in records)
+        return records, bool(records) and emission_may_clamp(self.count_bound, drawn, self.max_particles)
+
+    def count_owned(self):
+        """Enqueue this rank's non-ghost particle count into a device word (an int32 tensor on the context's
+        stream) and return the word; summed over the ranks it is the scene's count."""
+        import torch
+        if self._count_word is None:
+            dev = self._tensor_device if self._tensor_device is not None else torch.device("cuda", self.ctx.device)
+            with self._on_stream():
+                self._count_word = torch.zeros(1, dtype=torch.int32, device=dev)
+        self.ctx.dist_owned_count(self._count_word)
+        return self._count_word
+
+    def emit(self, records: list, scene_count=None) -> None:
+        """Append this rank's rows of the tick's emission; `scene_count`: the device word holding the scene's count,
+        or None when draw_emission found that the clamp cannot bind."""
+        if not records:
+            return
+        self.ctx.dist_emit_particles(records, self.max_particles, self.next_uid, scene_count)
+        drawn = sum(r[6] for r in records)
+        self.next_uid += drawn
+        self.count_bound += drawn
+        self.scene_counts += scene_count is not None
+
+    def recut(self) -> None:
+        """Re-cut (collective) on its ticks, then slide the cuts towards their targets."""
         if self.world_size > 1:
             if self.rebalance_every and self.tick and self.tick >= self._next_rebalance:
                 self.rebalance()
             if self.cuts != self.target_cuts:
                 self._slide_cuts()
+
+    def finish_tick(self) -> None:
+        """After the step: free bodies fall (the rigid-body part of the reference's gravity), tick += 1."""
+        from .rigid_body import apply_gravity_to_free_bodies
+        apply_gravity_to_free_bodies(self.bodies, self.dt, self.gravity)
+        self.tick += 1
+        if self.check_every and self.world_size > 1 and self.tick % self.check_every == 0:
+            self._check_flags()
+
+    def physics_tick(self) -> None:
+        self.advance_scene()
+        records, may_clamp = self.draw_emission()
+        count = None
+        if may_clamp:
+            count = self.count_owned()
+            if self.world_size > 1:
+                import torch.distributed as dist
+                with self._on_stream():   # the same process group as the re-cut, ordered on the launch stream
+                    dist.all_reduce(count)
+        self.emit(records, count)
+        self.recut()
+        if self.world_size > 1:
             if self._symm is not None:
                 self._exchange_p2p()
             else:
@@ -397,9 +496,7 @@ class StripDomain:
                 self.exchange()
                 self.ctx.dist_unpack(self.recv_lo, self.recv_hi)
         self.ctx.step()
-        self.tick += 1
-        if self.check_every and self.world_size > 1 and self.tick % self.check_every == 0:
-            self._check_flags()
+        self.finish_tick()
 
     def _check_flags(self) -> None:
         """Raise if the device has flagged a capacity overflow or a particle that outran the halo (results after such
