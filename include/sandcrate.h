@@ -270,6 +270,54 @@ int sc_dist_owned_count(sc_ctx *ctx, uint32_t *count_dev);
 int sc_dist_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsources, int64_t max_particles,
                            uint32_t first_uid, const uint32_t *scene_count_dev);
 
+/* ---- ensembles: M members of one scene in one context (DESIGN.md section 12) ------------------------------------ */
+/* An ensemble steps M variants of one scene - a coefficient sweep or seed replicas - with one launch sequence per tick
+ * whatever M is.  The members share dt, particle_radius and the walls (sc_set_walls, once for all); each has its own
+ * other coefficients, noise seed, particles and identities, and each is bit-identical to a single-scene context run with
+ * its coefficients and seed.  Member m's cells are m * (cells of the scene's grid) + its own cell, so the cell grid is
+ * the scene's stacked M times and M times its cells must fit the 32-bit cell key; member m's uids are
+ * (m << uid_bits) | local uid, local uids in order of creation as on a single-scene context.
+ * sc_ens_configure makes a fresh context (no parameters, no state yet) an ensemble.  M * 2^uid_bits <= 2^31; the
+ * readback map takes 4 * M * 2^uid_bits bytes of device memory.  Refused with SC_NOISE_HOST, on a strip context and with
+ * the ForceMonitor on; those calls are refused on an ensemble later as well.
+ * On an ensemble context:
+ *   works, all members at once: sc_set_walls, sc_set_tick, sc_step, sc_step_n, sc_synchronize, sc_particle_count (the
+ *     total), sc_get_state / sc_get_uids (all members, member-major = ascending global uid; the uids are global),
+ *     sc_last_pair_count (the directed pairs of all members), measurement, sc_debug_untiled_blocks, sc_debug_grid (the
+ *     stacked grid), sc_debug_walls, sc_detect_particle_collisions / sc_points_to_segments_distance (they do not touch
+ *     the context's state);
+ *   sc_set_noise: the mode only (SC_NOISE_COUNTER or SC_NOISE_NONE); the seeds come with sc_ens_set_params;
+ *   refused: sc_set_params, sc_set_state, sc_set_state_uids, sc_append_particles, sc_emit_particles (use the sc_ens_
+ *     forms), sc_step_begin / sc_step_finish, the parity taps, sc_debug_pair_records, sc_debug_rerun (returns -1),
+ *     sc_set_monitor and sc_get_monitor (the monitor cannot be switched on, so there is nothing to read), sc_set_state_uids,
+ *     sc_dist_* (sc_dist_configure refuses; the other sc_dist_ calls need it). */
+int sc_ens_configure(sc_ctx *ctx, int members, int uid_bits);
+/* p[M], seeds[M]: each member's coefficients and noise seed.  dt and particle_radius must be the same in every member
+ * (the error names the field and the member).  Changing any member's bytes drops the next tick's precomputed keys, as
+ * sc_set_params does; pushing unchanged bytes costs no launch. */
+int sc_ens_set_params(sc_ctx *ctx, const sc_params *p, const uint64_t *seeds);
+/* The whole state: pos, vel = n x 2 with n = sum(counts), member 0's rows first.  uid[n]: the rows' global uids (each
+ * one of its member's), or NULL for local uids 0 .. counts[m] - 1; next_local[M]: the local uid each member's next
+ * particle gets, or NULL for one past its largest.  (With both, a state read back with sc_ens_get_state and sc_get_uids
+ * continues exactly in a context of another capacity.) */
+int sc_ens_set_state(sc_ctx *ctx, const double *pos, const double *vel, const int64_t *counts, const uint32_t *uid,
+                     const uint32_t *next_local);
+/* sc_emit_particles for every member: sources[nsources] as for sc_emit_particles (their `count` is ignored),
+ * counts[M x nsources] = the counts member m drew from its own counter stream (its seed), max_particles[M].  Each member
+ * is clamped against its own live count, and its identities advance by its drawn count.  The draws travel as kernel
+ * parameters: one launch while M * (nsources + 1) <= 7936, one more per further 7936 words.  No host wait, no host
+ * buffer copied.  Refused before anything is launched when a member's identities would pass 2^uid_bits, and when the
+ * members' counts could outgrow the capacity: each member's count is bounded by what the last state set and what every
+ * emission's clamp allowed since (max(bound, min(bound + drawn, max_particles))), and the sum must fit. */
+int sc_ens_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsources, const int32_t *counts,
+                          const int64_t *max_particles);
+/* Per-member live counts: to the caller's device words counts_dev[M] (uint32, may be NULL; enqueued, no host wait) and,
+ * when counts[M] is not NULL, to the host (synchronises). */
+int sc_ens_member_counts(sc_ctx *ctx, int64_t *counts, uint32_t *counts_dev);
+/* sc_get_state of all members, member-major, with offsets[M + 1]: member m's rows are offsets[m] .. offsets[m + 1] - 1.
+ * Synchronises. */
+int sc_ens_get_state(sc_ctx *ctx, double *pos, double *vel, double *pressure, int64_t cap, int64_t *offsets);
+
 #ifdef __cplusplus
 }
 #endif

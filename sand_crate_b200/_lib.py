@@ -106,6 +106,12 @@ SIGNATURES = {
     "sc_debug_pair_records": (C.c_int, [_ctx, _ip, _ip, _dp, C.c_int64]),
     "sc_debug_grid": (C.c_int, [_ctx, _lp]),
     "sc_debug_walls": (C.c_int, [_ctx, _dp, _dp, _dp, _ip]),
+    "sc_ens_configure": (C.c_int, [_ctx, C.c_int, C.c_int]),
+    "sc_ens_set_params": (C.c_int, [_ctx, C.POINTER(ScParams), C.POINTER(C.c_uint64)]),
+    "sc_ens_set_state": (C.c_int, [_ctx, _dp, _dp, _lp, _up, _up]),
+    "sc_ens_emit_particles": (C.c_int, [_ctx, C.POINTER(ScSource), C.c_int, _ip, _lp]),
+    "sc_ens_member_counts": (C.c_int, [_ctx, _lp, C.c_void_p]),
+    "sc_ens_get_state": (C.c_int, [_ctx, _dp, _dp, _dp, C.c_int64, _lp]),
 }
 
 _lib = None
@@ -499,6 +505,53 @@ class Context:
         S = int(counts[0])
         return {"safe_contact": rects[0:4], "safe_ccd": rects[4:8], "safe_ccd_f32": rects[8:12],
                 "seg_box": seg_box[:S].copy(), "pad_box": pad_box[:2 * S].copy(), "contacts": int(counts[1])}
+
+
+    # ---- ensembles (include/sandcrate.h "ensembles") ----
+    def ens_configure(self, members: int, uid_bits: int):
+        self._ck(self._L.sc_ens_configure(self._h, int(members), int(uid_bits)))
+        self.members = int(members)
+
+    def ens_set_params(self, params, seeds):
+        """params: one keyword dict of PARAM_FIELDS per member; seeds: one noise seed per member."""
+        arr = (ScParams * len(params))(*[ScParams(*[float(p[n]) for n in PARAM_FIELDS]) for p in params])
+        sd = np.ascontiguousarray(seeds, dtype=np.uint64)
+        self._ck(self._L.sc_ens_set_params(self._h, arr, sd.ctypes.data_as(C.POINTER(C.c_uint64))))
+
+    def ens_set_state(self, pos, vel, counts, uid=None, next_local=None):
+        """Member-major rows, counts[m] of member m; uid (global) and next_local (per member) default to a fresh
+        numbering (sc_ens_set_state)."""
+        pos, vel = _f64(pos, 2), _f64(vel, 2)
+        counts = np.ascontiguousarray(counts, dtype=np.int64)
+        assert pos.shape == vel.shape and counts.sum() == pos.shape[0]
+        uid = None if uid is None else np.ascontiguousarray(uid, dtype=np.uint32)
+        nxt = None if next_local is None else np.ascontiguousarray(next_local, dtype=np.uint32)
+        self._ck(self._L.sc_ens_set_state(self._h, _ptr(pos, _dp), _ptr(vel, _dp), _ptr(counts, _lp), _ptr(uid, _up),
+                                          _ptr(nxt, _up)))
+
+    def ens_emit_particles(self, records, counts, max_particles):
+        """records: `ParticleSource.emit_record` tuples (their count is ignored); counts: members x len(records) drawn
+        counts; max_particles: one per member."""
+        arr = (ScSource * len(records))(*[ScSource(*r) for r in records])
+        cnt = np.ascontiguousarray(counts, dtype=np.int32).reshape(-1)
+        mx = np.ascontiguousarray(max_particles, dtype=np.int64)
+        self._ck(self._L.sc_ens_emit_particles(self._h, arr, len(records), _ptr(cnt, _ip), _ptr(mx, _lp)))
+
+    def ens_member_counts(self, counts_dev=None, want_host=True):
+        """Per-member live counts (synchronises) and/or, enqueued without a host wait, into the uint32 device words
+        `counts_dev`."""
+        counts = np.zeros(self.members, np.int64) if want_host else None
+        self._ck(self._L.sc_ens_member_counts(self._h, _ptr(counts, _lp), self._devptr(counts_dev)))
+        return counts
+
+    def ens_get_state(self, want_pressure=True):
+        """(pos, vel, pressure, offsets) of all members, member-major; member m's rows are offsets[m]:offsets[m + 1]."""
+        n = self.particle_count()
+        pos, vel = np.empty((n, 2)), np.empty((n, 2))
+        prs = np.empty(n) if want_pressure else None
+        off = np.zeros(self.members + 1, np.int64)
+        self._ck(self._L.sc_ens_get_state(self._h, _ptr(pos, _dp), _ptr(vel, _dp), _ptr(prs, _dp), n, _ptr(off, _lp)))
+        return pos, vel, prs, off
 
 
 def source_uniform(seed: int, tick: int, source_index: int, j: int) -> float:

@@ -108,6 +108,21 @@ struct sc_ctx {
     // arrays and the device count lack the records: enter() refuses every call that would read or change them.
     struct { bool on = false; const void *recv_lo = nullptr, *flag_lo = nullptr, *recv_hi = nullptr, *flag_hi = nullptr;
              uint32_t value = 0; } pend;
+    // ensemble (sc_ens_configure, DESIGN.md section 12): `members` stacked copies of the scene's cell grid, uids
+    // (m << uid_bits) | local uid, per-member parameters and seeds in device tables
+    bool ens = false;
+    uint32_t members = 1, uid_bits = 0;
+    DevParams *ens_params = nullptr;
+    unsigned long long *ens_seed = nullptr;
+    uint32_t *ens_count = nullptr;   // per-member live counts, current unless ens_stale
+    uint32_t *ens_next_dev = nullptr;  // next local uid per member, advanced by k_emit_members
+    bool ens_stale = false;          // a step ran since ens_count was written: the counts are in its cell scan
+    std::vector<sc_params> ens_hp;   // host copies of the tables
+    std::vector<unsigned long long> ens_seeds;
+    std::vector<uint32_t> ens_next;  // host copy of ens_next_dev (identities advance by the drawn count)
+    // per-member upper bound of the live count: what the state set, raised by every emission to what its clamp allows.
+    // Removal only lowers a count, so the sum bounds the particles the arrays must hold (sc_ens_emit_particles).
+    std::vector<uint64_t> ens_bound;
     int64_t launches = 0;
     int64_t syncs = 0;        // host waits on the stream (cudaStreamSynchronize) issued by this context's entry points
     bool profiling = false;
@@ -146,6 +161,12 @@ static int enter(sc_ctx *ctx, const char *who, bool consumes_unpack = false) {
         return fail(ctx, std::string(who) + ": a strip unpack is pending (the next call must be a step)");
     cudaError_t e = cudaSetDevice(ctx->device);
     if (e != cudaSuccess) return fail(ctx, std::string("cudaSetDevice: ") + cudaGetErrorString(e));
+    return 0;
+}
+
+// the single-scene entry points an ensemble refuses (include/sandcrate.h, "ensembles")
+static int no_ensemble(sc_ctx *ctx, const char *who) {
+    if (ctx->ens) return fail(ctx, std::string(who) + ": not available on an ensemble context");
     return 0;
 }
 
@@ -228,9 +249,15 @@ static int setup_grid(sc_ctx *ctx, double d, int row_min, int row_max, int col_m
     const int64_t nrows = (int64_t)row_max - row_min + 3, ncols = (int64_t)col_max - col_min + 3;
     if (nrows <= 0 || ncols <= 0 || nrows * ncols > (int64_t)1 << 31)
         return fail(ctx, "cell grid too large: " + std::to_string(nrows) + " x " + std::to_string(ncols));
-    g.nrows = (int)nrows;
+    // an ensemble stacks one grid per member: M nrows rows; the 32-bit cell key (SC_INVALID_CELL reserved) and the
+    // scan's tail of 8 must hold them all
+    const int64_t M = ctx->members;
+    if (M * nrows * ncols + 8 >= (int64_t)SC_INVALID_CELL)
+        return fail(ctx, "too many cells: " + std::to_string(M) + " members x " + std::to_string(nrows * ncols) +
+                             " cells do not fit the 32-bit cell key");
+    g.nrows = (int)(M * nrows);
     g.ncols = (int)ncols;
-    g.ncells = (uint32_t)(nrows * ncols);
+    g.ncells = (uint32_t)(M * nrows * ncols);
     const size_t need = (size_t)g.ncells + 8;  // + the live count at [ncells]; bulk copies read whole 16-byte groups
     if (need > ctx->cell_cap) {
         if (ctx->cell_count) CK(cudaFree(ctx->cell_count));
@@ -279,7 +306,9 @@ static int halo_needed(int contacts) { return 2 + wall_fix_rows(contacts); }
 
 // Cell grid of the world box; in strip mode only the rows this rank can ever hold (its strip, the halo, and the
 // rows the wall fix can shift a position by), so clearing and scanning the grid scales with the strip, not the scene.
+static int ens_fold_counts(sc_ctx *ctx);
 static int world_grid(sc_ctx *ctx) {
+    CKR(ens_fold_counts(ctx));  // the members' counts may still sit in the old grid's scan
     long long wlo, whi;
     world_rows(ctx, wlo, whi);
     if (wlo < -(1LL << 30) || whi > (1LL << 30)) return fail(ctx, "cell grid too large for the wall-fix margin");
@@ -296,9 +325,8 @@ static int world_grid(sc_ctx *ctx) {
     return 0;
 }
 
-static int refresh_dev_params(sc_ctx *ctx) {
-    const sc_params &h = ctx->hp;
-    DevParams &p = ctx->dp;
+static DevParams dev_params_of(const sc_params &h) {
+    DevParams p{};
     p.dt = h.dt; p.r = h.particle_radius; p.d = h.particle_radius * 2;  // crate.py:65-67
     p.touch = h.particle_radius * 1.2;                                   // crate.py:229
     p.decay = h.wall_collision_decay; p.amp = h.pressure_amplifier; p.ignored = h.ignored_pressure;
@@ -311,6 +339,12 @@ static int refresh_dev_params(sc_ctx *ctx) {
     p.f_dt = (float)p.dt; p.f_dt_gx = (float)(p.dt * p.gx); p.f_dt_gy = (float)(p.dt * p.gy);
     p.f_dt_amp = (float)(p.dt * p.amp); p.f_dt_visc = (float)(p.dt * p.visc);
     p.f_smooth = (float)p.smooth; p.f_two_target = (float)(2 * p.target); p.f_ignored = (float)p.ignored;
+    return p;
+}
+static int refresh_dev_params(sc_ctx *ctx) {
+    const int nm = ctx->dp.noise_mode; const uint64_t tk = ctx->dp.tick_key;  // (set per step by step_params)
+    ctx->dp = dev_params_of(ctx->hp);
+    ctx->dp.noise_mode = nm; ctx->dp.tick_key = tk;
     return 0;
 }
 
@@ -414,7 +448,8 @@ extern "C" void sc_destroy(sc_ctx *c) {
     void *ptrs[] = {c->pos_cur, c->pos_srt, c->vel_cur, c->vel_srt, c->uid_cur, c->uid_srt, c->cell_key,
                     c->cell_key_srt, c->tmpidx, c->cell_count, c->cell_start, c->bsum, c->bsum2, c->rel_srt, c->rec_srt, c->blk_desc, c->ps, c->pair_j, c->pair_n, c->pair_off, c->pair_cnt,
                     c->wbits_cur[0], c->wbits_cur[1], c->wbits_srt[0], c->wbits_srt[1], c->wall_slot_cur, c->wall_slot_srt, c->wall_pre_buf[0], c->wall_pre_buf[1], c->cnt,
-                    c->rank_of_uid, c->count_by_rank, c->list_sorted, c->noise_dev, c->stage2, c->stage1, c->wire_dummy, c->monitor};
+                    c->rank_of_uid, c->count_by_rank, c->list_sorted, c->noise_dev, c->stage2, c->stage1, c->wire_dummy, c->monitor,
+                    c->ens_params, c->ens_seed, c->ens_count, c->ens_next_dev};
     for (void *p : ptrs) if (p) cudaFree(p);
     for (auto &p : c->pending) { cudaEventDestroy(p.e0); cudaEventDestroy(p.e1); }
     for (auto e : c->pool) cudaEventDestroy(e);
@@ -422,8 +457,7 @@ extern "C" void sc_destroy(sc_ctx *c) {
     delete c;
 }
 
-extern "C" int sc_set_params(sc_ctx *ctx, const sc_params *p) {
-    CKR(enter(ctx, "sc_set_params"));
+static int set_params(sc_ctx *ctx, const sc_params *p) {
     if (!p) return fail(ctx, "sc_set_params: NULL argument");
     if (!(p->particle_radius > 0) || !(p->dt == p->dt)) return fail(ctx, "sc_set_params: particle_radius must be > 0");
     const bool regrid = !ctx->params_set || p->particle_radius != ctx->hp.particle_radius;
@@ -443,6 +477,11 @@ extern "C" int sc_set_params(sc_ctx *ctx, const sc_params *p) {
     }
     ctx->params_set = true;
     return 0;
+}
+extern "C" int sc_set_params(sc_ctx *ctx, const sc_params *p) {
+    CKR(enter(ctx, "sc_set_params"));
+    CKR(no_ensemble(ctx, "sc_set_params"));
+    return set_params(ctx, p);
 }
 
 extern "C" int sc_pad_segments(const double *segments, int S, double pad, double *padded) {
@@ -590,10 +629,15 @@ extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const in
     return 0;
 }
 
+static int ens_upload(sc_ctx *ctx);
 extern "C" int sc_set_noise(sc_ctx *ctx, int mode, uint64_t seed) {
     CKR(enter(ctx, "sc_set_noise"));
     if (mode < SC_NOISE_NONE || mode > SC_NOISE_HOST) return fail(ctx, "sc_set_noise: bad mode");
+    if (ctx->ens && mode == SC_NOISE_HOST)
+        return fail(ctx, "sc_set_noise: an ensemble cannot take the reference's noise stream (SC_NOISE_HOST): that "
+                         "stream is one per process");
     ctx->noise_mode = mode; ctx->seed = seed;
+    if (ctx->ens && ctx->params_set) CKR(ens_upload(ctx));  // the members' effective modes follow the mode
     return 0;
 }
 extern "C" int sc_set_tick(sc_ctx *ctx, uint64_t tick) {
@@ -650,8 +694,7 @@ static int upload_particles(sc_ctx *ctx, const double *pos, const double *vel, i
     return 0;
 }
 
-extern "C" int sc_set_state(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
-    CKR(enter(ctx, "sc_set_state"));
+static int set_state(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
     CKR(drop_keys(ctx));
     if (n < 0 || n > ctx->cap) return fail(ctx, "sc_set_state: n exceeds capacity");
     if (ctx->in_step) return fail(ctx, "sc_set_state: inside a split step");
@@ -663,9 +706,15 @@ extern "C" int sc_set_state(sc_ctx *ctx, const double *pos, const double *vel, i
     ctx->n_host = 0; ctx->n_exact = true;
     return upload_particles(ctx, pos, vel, 0, n);
 }
+extern "C" int sc_set_state(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
+    CKR(enter(ctx, "sc_set_state"));
+    CKR(no_ensemble(ctx, "sc_set_state"));
+    return set_state(ctx, pos, vel, n);
+}
 
 extern "C" int sc_set_state_uids(sc_ctx *ctx, const double *pos, const double *vel, const uint32_t *uid, int64_t n) {
     CKR(enter(ctx, "sc_set_state_uids"));
+    CKR(no_ensemble(ctx, "sc_set_state_uids"));
     if (!uid) return fail(ctx, "sc_set_state_uids: uid is NULL");
     uint32_t top = 0;
     for (int64_t i = 0; i < n; ++i) {
@@ -681,6 +730,7 @@ extern "C" int sc_set_state_uids(sc_ctx *ctx, const double *pos, const double *v
 
 extern "C" int sc_append_particles(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
     CKR(enter(ctx, "sc_append_particles"));
+    CKR(no_ensemble(ctx, "sc_append_particles"));
     CKR(drop_keys(ctx));
     if (ctx->in_step) return fail(ctx, "sc_append_particles: inside a split step");
     if (n < 0) return fail(ctx, "sc_append_particles: n < 0");
@@ -698,6 +748,7 @@ extern "C" uint64_t sc_source_stream(uint64_t seed, uint64_t tick, uint32_t sour
 
 extern "C" int sc_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsources, int64_t max_particles) {
     CKR(enter(ctx, "sc_emit_particles"));
+    CKR(no_ensemble(ctx, "sc_emit_particles"));
     if (nsources > 0 && !sources) return fail(ctx, "sc_emit_particles: NULL argument");
     if (ctx->in_step) return fail(ctx, "sc_emit_particles: inside a split step");
     if (nsources < 0 || nsources > SC_MAX_SOURCES) return fail(ctx, "sc_emit_particles: more than SC_MAX_SOURCES sources");
@@ -809,6 +860,22 @@ static int require_ready(sc_ctx *ctx, const char *who, bool consumes_unpack = fa
     return 0;
 }
 
+// The ensemble descriptor of a launch (Members, sc_common.cuh): `uid` = the uids of the arrays the kernel indexes,
+// `tick` = the tick whose noise and sources it draws.  Zero on a single-scene context (the kernels then ignore it).
+static Members members_arg(const sc_ctx *ctx, const uint32_t *uid, uint64_t tick) {
+    Members E{};
+    if (!ctx->ens) return E;
+    E.params = ctx->ens_params; E.seed = ctx->ens_seed; E.uid = uid; E.tick = tick;
+    E.uid_bits = ctx->uid_bits; E.ncells = ctx->grid.ncells / ctx->members; E.nrows = ctx->grid.nrows / (int)ctx->members;
+    return E;
+}
+// the grid of one member (= the grid on a single-scene context): what the key pass clamps a position into
+static Grid scene_grid(const sc_ctx *ctx) {
+    Grid g = ctx->grid;
+    g.nrows /= (int)ctx->members; g.ncells /= ctx->members;
+    return g;
+}
+
 // where the key pass of a tick of parity `q` writes (key_particle, sc_common.cuh)
 static KeyOut key_out(sc_ctx *ctx, int q) {
     return KeyOut{ctx->cell_key, ctx->cell_count, ctx->wbits_cur[q], ctx->wall_slot_cur, &ctx->cnt->n_wall[q],
@@ -848,9 +915,11 @@ template <bool kStep> static int enqueue_search(sc_ctx *ctx) {
         ProfScope ps(ctx, SLOT_PREPASS);
         auto go = [&](auto kernel) {
             return launch_pdl(kernel, dim3(blocks_for((n + SC_PREPASS_ILP - 1) / SC_PREPASS_ILP)), dim3(SC_BLOCK),
-                              ctx->stream, ctx->cnt, g, ctx->dp, ctx->walls, key_out(ctx, ctx->par), (uint32_t)ctx->cap, U);
+                              ctx->stream, ctx->cnt, scene_grid(ctx), ctx->dp, ctx->walls, key_out(ctx, ctx->par),
+                              (uint32_t)ctx->cap, U, members_arg(ctx, ctx->uid_cur, ctx->tick));
         };
-        CK(U.on ? go(k_prepass<kStep, true>) : go(k_prepass<kStep, false>));
+        if (ctx->ens) CK(go(k_prepass<kStep, false, true>));
+        else CK(U.on ? go(k_prepass<kStep, true>) : go(k_prepass<kStep, false>));
     }
     CKR(exclusive_scan(ctx, ctx->cell_count, ctx->cell_start, g.ncells, SLOT_SCAN, true));
     if (n > 0) {
@@ -861,16 +930,21 @@ template <bool kStep> static int enqueue_search(sc_ctx *ctx) {
                           (const uint32_t *)ctx->cell_start, ctx->tmpidx, (uint32_t)ctx->cap));
         }
         ProfScope ps(ctx, SLOT_RANK_GATHER);
-        if (ctx->precision == SC_PRECISION_F64)
-            CK(launch_pdl(k_rank_gather<double>, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream,
+        const Members E = members_arg(ctx, nullptr, ctx->tick);
+        auto go64 = [&](auto kernel) {
+            return launch_pdl(kernel, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream,
                 ctx->cnt, g, ctx->cell_start, ctx->tmpidx, ctx->cell_key, ctx->pos_cur, (const double2 *)ctx->vel_cur,
                 ctx->uid_cur, ctx->wall_bits_cur, ctx->wall_slot_cur, ctx->pos_srt, ctx->rel_srt, (double2 *)ctx->vel_srt,
-                ctx->uid_srt, ctx->cell_key_srt, ctx->wall_bits_srt, ctx->wall_slot_srt, (float4 *)nullptr, (BlockDesc *)nullptr));
-        else
-            CK(launch_pdl(k_rank_gather<float>, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream,
+                ctx->uid_srt, ctx->cell_key_srt, ctx->wall_bits_srt, ctx->wall_slot_srt, (float4 *)nullptr, (BlockDesc *)nullptr, E);
+        };
+        auto go32 = [&](auto kernel) {
+            return launch_pdl(kernel, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream,
                 ctx->cnt, g, ctx->cell_start, ctx->tmpidx, ctx->cell_key, ctx->pos_cur, (const float2 *)ctx->vel_cur,
                 ctx->uid_cur, ctx->wall_bits_cur, ctx->wall_slot_cur, ctx->pos_srt, ctx->rel_srt, (float2 *)ctx->vel_srt,
-                ctx->uid_srt, ctx->cell_key_srt, ctx->wall_bits_srt, ctx->wall_slot_srt, ctx->rec_srt, ctx->blk_desc));
+                ctx->uid_srt, ctx->cell_key_srt, ctx->wall_bits_srt, ctx->wall_slot_srt, ctx->rec_srt, ctx->blk_desc, E);
+        };
+        if (ctx->precision == SC_PRECISION_F64) CK(ctx->ens ? go64(k_rank_gather<double, true>) : go64(k_rank_gather<double>));
+        else CK(ctx->ens ? go32(k_rank_gather<float, true>) : go32(k_rank_gather<float>));
     }
     CK(cudaGetLastError());
     ctx->srt_valid = true;
@@ -909,28 +983,31 @@ static NextWallClear next_wall_clear(sc_ctx *ctx) {
     return NextWallClear{ctx->wbits_cur[o], ctx->wbits_srt[o], (uint32_t)(ctx->cap / 32 + 1), &ctx->cnt->n_wall[o]};
 }
 
-static int launch_density(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, int64_t n) {
+static int launch_density(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, int64_t n, const Members &E) {
     auto go = [&](auto kernel) {
         return launch_pdl(kernel, dim3(blocks_for(n)), dim3(SC_BLOCK), ctx->stream, ctx->cnt, ctx->grid, dp, ctx->cell_start,
                           ctx->pos_srt, ctx->rel_srt, ctx->cell_key_srt, ctx->uid_cur, ctx->noise_dev, noise_off,
                           ctx->rank_of_uid, ctx->pair_j, (double2 *)ctx->pair_n, ctx->pair_off, ctx->pair_cnt,
-                          (PS<double> *)ctx->ps, next_wall_clear(ctx));
+                          (PS<double> *)ctx->ps, next_wall_clear(ctx), E);
     };
-    if (dp.noise_mode == SC_NOISE_HOST) CK(go(k_density<SC_NOISE_HOST>));
+    if (ctx->ens) CK(dp.noise_mode == SC_NOISE_COUNTER ? go(k_density<SC_NOISE_COUNTER, true>) : go(k_density<SC_NOISE_NONE, true>));
+    else if (dp.noise_mode == SC_NOISE_HOST) CK(go(k_density<SC_NOISE_HOST>));
     else if (dp.noise_mode == SC_NOISE_COUNTER) CK(go(k_density<SC_NOISE_COUNTER>));
     else CK(go(k_density<SC_NOISE_NONE>));
     return 0;
 }
 
 // K4 stages the block's neighborhood in shared memory (sc_tile.cuh)
-static int launch_density_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, int64_t n) {
+static int launch_density_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, int64_t n, const Members &E) {
     auto go = [&](auto kernel) {
         return launch_pdl(kernel, dim3((unsigned)((n + SC_TILE - 1) / SC_TILE)), dim3(SC_TILE), ctx->stream, ctx->cnt,
                           ctx->grid, dp, ctx->cell_start, ctx->blk_desc, ctx->pos_srt, ctx->rec_srt, ctx->cell_key_srt,
                           (uint2 *)ctx->pair_n, ctx->pair_cnt, (PS<float> *)ctx->ps, next_wall_clear(ctx),
-                          HostNoise{ctx->noise_dev, noise_off, ctx->rank_of_uid});
+                          HostNoise{ctx->noise_dev, noise_off, ctx->rank_of_uid}, E);
     };
-    if (dp.noise_mode == SC_NOISE_HOST) CK(go(k_density_tile<SC_NOISE_HOST>));
+    if (ctx->ens)
+        CK(dp.noise_mode == SC_NOISE_COUNTER ? go(k_density_tile<SC_NOISE_COUNTER, true>) : go(k_density_tile<SC_NOISE_NONE, true>));
+    else if (dp.noise_mode == SC_NOISE_HOST) CK(go(k_density_tile<SC_NOISE_HOST>));
     else if (dp.noise_mode == SC_NOISE_COUNTER) CK(go(k_density_tile<SC_NOISE_COUNTER>));
     else CK(go(k_density_tile<SC_NOISE_NONE>));
     return 0;
@@ -946,34 +1023,37 @@ static TickDuty tick_duty(sc_ctx *ctx) {
 }
 static NextKeys next_keys(sc_ctx *ctx, bool keys) {
     NextKeys k{};
-    k.g = ctx->grid;
+    k.g = scene_grid(ctx);
     if (keys) k.out = key_out(ctx, ctx->par ^ 1);
     return k;
 }
 
-static int launch_force(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n, bool keys) {
+static int launch_force(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n, bool keys, const Members &E) {
     const unsigned nb = (unsigned)((n + SC_K5_THREADS - 1) / SC_K5_THREADS);
     auto go = [&](auto kernel) {
         return launch_pdl(kernel, dim3(nb), dim3(SC_K5_THREADS), ctx->stream, n_ptr, dp, ctx->walls, ctx->pos_srt,
                           (const double2 *)ctx->vel_srt, ctx->pair_j, (const double2 *)ctx->pair_n, ctx->pair_off,
                           ctx->pair_cnt, (const PS<double> *)ctx->ps, ctx->wall_bits_srt, ctx->wall_slot_srt,
                           ctx->wall_pre, ctx->pos_cur, (double2 *)ctx->vel_cur, ctx->monitor, tick_duty(ctx),
-                          next_keys(ctx, keys));
+                          next_keys(ctx, keys), E);
     };
-    CK(ctx->monitor_on ? go(k_force<true>) : go(k_force<false>));
+    if (ctx->ens) CK(go(k_force<false, true>));  // (no ForceMonitor on an ensemble: sc_set_monitor refuses)
+    else CK(ctx->monitor_on ? go(k_force<true>) : go(k_force<false>));
     return 0;
 }
 
 // K5 on the same blocks and windows as K4 (sc_tile.cuh)
-static int launch_force_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n, bool keys) {
+static int launch_force_tile(sc_ctx *ctx, const DevParams &dp, const uint32_t *n_ptr, int64_t n, bool keys,
+                             const Members &E) {
     auto go = [&](auto kernel) {
         return launch_pdl(kernel, dim3((unsigned)((n + SC_TILE - 1) / SC_TILE)), dim3(SC_TILE), ctx->stream, n_ptr, dp,
                           ctx->walls, ctx->blk_desc, ctx->pos_srt, (const float2 *)ctx->vel_srt, (const uint2 *)ctx->pair_n,
                           ctx->pair_cnt, (const PS<float> *)ctx->ps, ctx->wall_bits_srt, ctx->wall_slot_srt,
                           ctx->wall_pre, ctx->pos_cur, (float2 *)ctx->vel_cur, ctx->monitor, tick_duty(ctx),
-                          next_keys(ctx, keys));
+                          next_keys(ctx, keys), E);
     };
-    CK(ctx->monitor_on ? go(k_force_tile<true>) : go(k_force_tile<false>));
+    if (ctx->ens) CK(go(k_force_tile<false, true>));
+    else CK(ctx->monitor_on ? go(k_force_tile<true>) : go(k_force_tile<false>));
     return 0;
 }
 
@@ -982,6 +1062,7 @@ static DevParams step_params(const sc_ctx *ctx, uint64_t tick) {
     DevParams dp = ctx->dp;
     dp.noise_mode = (ctx->noise_mode != SC_NOISE_NONE && ctx->hp.collider_noise_level == 0.0) ? SC_NOISE_NONE
                                                                                              : ctx->noise_mode;
+    if (ctx->ens) dp.noise_mode = ctx->noise_mode;  // each member's own effective mode is in its table row
     dp.tick_key = tick_key(ctx->seed, tick);
     return dp;
 }
@@ -989,18 +1070,20 @@ static DevParams step_params(const sc_ctx *ctx, uint64_t tick) {
 // The pair kernels of the last search, chosen by the precision alone: k_density / k_force (sc_pair.cuh) in fp64, the
 // tiled kernels (sc_tile.cuh) in mixed precision, in every noise mode.  `k4`, `k5`: which of the two to enqueue.
 // `noise_off`: the CSR offsets of SC_NOISE_HOST.  The sorted set's uids must be in uid_cur.
-static int launch_pair_kernels(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, bool k4, bool k5, bool keys) {
+static int launch_pair_kernels(sc_ctx *ctx, const DevParams &dp, const uint32_t *noise_off, bool k4, bool k5, bool keys,
+                               uint64_t tick) {
     const int64_t n = ctx->n_host;
     const bool f64 = ctx->precision == SC_PRECISION_F64;
+    const Members E = members_arg(ctx, ctx->uid_cur, tick);
     if (k4) {
         ProfScope ps(ctx, SLOT_DENSITY);
-        CKR(f64 ? launch_density(ctx, dp, noise_off, n) : launch_density_tile(ctx, dp, noise_off, n));
+        CKR(f64 ? launch_density(ctx, dp, noise_off, n, E) : launch_density_tile(ctx, dp, noise_off, n, E));
     }
     if (k5) {
         if (ctx->monitor_on) CK(cudaMemsetAsync(ctx->monitor, 0, sizeof(double) * 8, ctx->stream));
         ProfScope ps(ctx, SLOT_FORCE);
         const uint32_t *n_ptr = ctx->cell_start + ctx->grid.ncells;
-        CKR(f64 ? launch_force(ctx, dp, n_ptr, n, keys) : launch_force_tile(ctx, dp, n_ptr, n, keys));
+        CKR(f64 ? launch_force(ctx, dp, n_ptr, n, keys, E) : launch_force_tile(ctx, dp, n_ptr, n, keys, E));
     }
     return 0;
 }
@@ -1012,7 +1095,8 @@ static int enqueue_forces(sc_ctx *ctx, const uint32_t *noise_off) {
     // the force kernel runs the next tick's key pass (NextKeys) unless a call since the last step changed what the keys
     // depend on (drop_keys) or this is a strip, whose exchange changes the particle set between the ticks
     const bool keys = n > 0 && !ctx->keys_dropped && !ctx->dist_on;
-    if (n > 0) CKR(launch_pair_kernels(ctx, step_params(ctx, ctx->tick), noise_off, true, true, keys));
+    if (n > 0) CKR(launch_pair_kernels(ctx, step_params(ctx, ctx->tick), noise_off, true, true, keys, ctx->tick));
+    ctx->ens_stale = ctx->ens;  // the members' counts are now in this tick's cell scan
     // the force kernel carried the count; the density kernel cleared the next tick's wall set, k_place the counts
     if (n > 0) { ctx->next_clean = !keys; ctx->next_keyed = keys; ctx->carry_count = false; }
     else ctx->carry_count = true;  // nothing ran: cnt->n is refreshed by the next cold start or by sync_count
@@ -1041,6 +1125,7 @@ extern "C" int sc_step_n(sc_ctx *ctx, int nsteps) {
 
 extern "C" int sc_step_begin(sc_ctx *ctx, int64_t *n_particles, int64_t *n_pairs) {
     CKR(require_ready(ctx, "sc_step_begin", true));
+    CKR(no_ensemble(ctx, "sc_step_begin"));
     if (ctx->in_step) return fail(ctx, "sc_step_begin: a split step is already open");
     CKR(enqueue_search<true>(ctx));
     ctx->in_step = true;
@@ -1058,6 +1143,7 @@ extern "C" int sc_step_begin(sc_ctx *ctx, int64_t *n_particles, int64_t *n_pairs
 
 extern "C" int sc_step_finish(sc_ctx *ctx, const double *noise) {
     CKR(require_ready(ctx, "sc_step_finish"));
+    CKR(no_ensemble(ctx, "sc_step_finish"));
     if (!ctx->in_step) return fail(ctx, "sc_step_finish: no split step is open");
     const uint32_t *noise_off = nullptr;
     const bool host_noise = ctx->noise_mode == SC_NOISE_HOST && ctx->hp.collider_noise_level != 0.0;
@@ -1176,6 +1262,7 @@ extern "C" int sc_get_uids(sc_ctx *ctx, uint32_t *uid, int64_t cap, int64_t *n_o
 // ---- taps --------------------------------------------------------------------------------------------------
 static int tap_prologue(sc_ctx *ctx, const char *who, int64_t cap, int64_t *n_out) {
     CKR(enter(ctx, who));
+    CKR(no_ensemble(ctx, who));
     if (!ctx->srt_valid) return fail(ctx, std::string(who) + ": no search state (call sc_step or sc_step_begin first)");
     CKR(no_neighbors(ctx, who));
     uint32_t total = 0;
@@ -1406,7 +1493,7 @@ extern "C" int sc_debug_walls(sc_ctx *ctx, double *rects, double *seg_box, doubl
 // -1 before a step, inside a split step, and under SC_NOISE_HOST: the step's noise offsets live in count_by_rank, which
 // the next count kernel (sc_get_neighbors, say) overwrites.
 extern "C" double sc_debug_rerun(sc_ctx *ctx, int which, int reps) {
-    if (!ctx || !ctx->srt_valid || ctx->in_step) return -1.0;
+    if (!ctx || !ctx->srt_valid || ctx->in_step || ctx->ens) return -1.0;
     const DevParams dp = step_params(ctx, ctx->tick - 1);
     if (dp.noise_mode == SC_NOISE_HOST) return -1.0;
     cudaSetDevice(ctx->device);
@@ -1417,7 +1504,7 @@ extern "C" double sc_debug_rerun(sc_ctx *ctx, int which, int reps) {
     for (int r = 0; r < reps; ++r) {
         if (which == 4) cudaMemsetAsync(&ctx->cnt->pair_cursor, 0, 4, ctx->stream);  // the fp64 K4 allocates from zero
         cudaEventRecord(e0, ctx->stream);
-        launch_pair_kernels(ctx, dp, nullptr, which == 4, which != 4, false);
+        launch_pair_kernels(ctx, dp, nullptr, which == 4, which != 4, false, ctx->tick - 1);
         cudaEventRecord(e1, ctx->stream);
         cudaEventSynchronize(e1);
         float ms = 0;
@@ -1441,6 +1528,7 @@ extern "C" int64_t sc_debug_untiled_blocks(sc_ctx *ctx) {
 // ---- ForceMonitor (utils/force_monitor.py) ------------------------------------------------------------------------
 extern "C" int sc_set_monitor(sc_ctx *ctx, int on) {
     CKR(enter(ctx, "sc_set_monitor"));
+    if (on) CKR(no_ensemble(ctx, "sc_set_monitor"));
     if (on && !ctx->monitor) {
         CKR(dev_alloc(ctx, &ctx->monitor, 8));
         CK(cudaMemsetAsync(ctx->monitor, 0, sizeof(double) * 8, ctx->stream));
@@ -1500,6 +1588,7 @@ extern "C" int64_t sc_dist_wire_bytes(int64_t wire_capacity) {
 extern "C" int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_lo, int64_t row_hi, int halo_rows,
                                  int64_t wire_capacity) {
     CKR(enter(ctx, "sc_dist_configure"));
+    CKR(no_ensemble(ctx, "sc_dist_configure"));
     if (ctx->walls_set) {  // refused before anything is launched
         const int v = contact_bound(ctx->walls.seg_box, ctx->walls.S);
         if (halo_rows < halo_needed(v)) return fail(ctx, halo_message("sc_dist_configure", v, halo_rows));
@@ -1803,5 +1892,251 @@ extern "C" int sc_dist_emit_particles(sc_ctx *ctx, const sc_source *sources, int
     ctx->n_exact = false;
     ctx->srt_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
     ctx->dist_tail = true;  // behind the sorted rows: the next pack must reach them (enqueue_pack)
+    return 0;
+}
+
+// ---- ensembles (include/sandcrate.h "ensembles", DESIGN.md section 12) ----------------------------------------------
+// Host -> device copies of the tables below read pageable std::vector memory: cudaMemcpyAsync from pageable memory
+// returns only once the driver has staged the bytes, so a vector rewritten (or freed) after the call cannot change
+// what the device reads.  Nothing is uploaded per tick: the tick keys come from the seed table and the launch's tick.
+
+// per-member counts of the last step's cell scan folded into ens_count (before a re-grid frees that scan)
+static int ens_fold_counts(sc_ctx *ctx) {
+    if (!ctx->ens || !ctx->ens_stale) return 0;
+    ProfScope ps(ctx, SLOT_IO);
+    k_member_counts<<<blocks_for(ctx->members), SC_BLOCK, 0, ctx->stream>>>(
+        ctx->members, ctx->grid.ncells / ctx->members, 1, ctx->cell_start, ctx->ens_count, nullptr);
+    ctx->ens_stale = false;
+    CK(cudaGetLastError());
+    return 0;
+}
+
+// the members' DevParams (with their effective noise mode: a zero noise level is none, as in step_params) and seeds
+static int ens_upload(sc_ctx *ctx) {
+    std::vector<DevParams> t(ctx->members);
+    for (uint32_t m = 0; m < ctx->members; ++m) {
+        t[m] = dev_params_of(ctx->ens_hp[m]);
+        t[m].noise_mode = (ctx->noise_mode != SC_NOISE_NONE && ctx->ens_hp[m].collider_noise_level == 0.0)
+                              ? SC_NOISE_NONE : ctx->noise_mode;
+    }
+    CK(cudaMemcpyAsync(ctx->ens_params, t.data(), sizeof(DevParams) * t.size(), cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->ens_seed, ctx->ens_seeds.data(), sizeof(unsigned long long) * ctx->members,
+                       cudaMemcpyHostToDevice, ctx->stream));
+    return 0;
+}
+
+extern "C" int sc_ens_configure(sc_ctx *ctx, int members, int uid_bits) {
+    CKR(enter(ctx, "sc_ens_configure"));
+    if (ctx->ens) return fail(ctx, "sc_ens_configure: already an ensemble");
+    if (ctx->params_set || ctx->n_host || ctx->next_uid)
+        return fail(ctx, "sc_ens_configure: the context must be fresh (no parameters, no particles yet)");
+    if (ctx->dist_on) return fail(ctx, "sc_ens_configure: a strip context cannot be an ensemble");
+    if (ctx->monitor_on) return fail(ctx, "sc_ens_configure: the ForceMonitor is not available on an ensemble");
+    if (ctx->noise_mode == SC_NOISE_HOST)
+        return fail(ctx, "sc_ens_configure: an ensemble cannot take the reference's noise stream (SC_NOISE_HOST): "
+                         "that stream is one per process");
+    if (members < 1 || uid_bits < 1 || uid_bits > 30 || ((uint64_t)members << uid_bits) > (1ull << 31))
+        return fail(ctx, "sc_ens_configure: need members >= 1 and members * 2^uid_bits <= 2^31 (members " +
+                             std::to_string(members) + ", uid_bits " + std::to_string(uid_bits) + ")");
+    const size_t M = (size_t)members;
+    CKR(dev_alloc(ctx, &ctx->ens_params, M));
+    CKR(dev_alloc(ctx, &ctx->ens_seed, M));
+    CKR(dev_alloc(ctx, &ctx->ens_count, M));
+    CKR(dev_alloc(ctx, &ctx->ens_next_dev, M));
+    CK(cudaMemsetAsync(ctx->ens_count, 0, sizeof(uint32_t) * M, ctx->stream));
+    CK(cudaMemsetAsync(ctx->ens_next_dev, 0, sizeof(uint32_t) * M, ctx->stream));
+    ctx->ens = true;
+    ctx->members = (uint32_t)members; ctx->uid_bits = (uint32_t)uid_bits;
+    ctx->ens_hp.assign(M, sc_params{}); ctx->ens_seeds.assign(M, 0ull); ctx->ens_next.assign(M, 0u);
+    ctx->ens_bound.assign(M, 0u);
+    ctx->next_uid = (uint32_t)(M << uid_bits);  // every uid is below it: the readback map covers them all
+    return 0;
+}
+
+extern "C" int sc_ens_set_params(sc_ctx *ctx, const sc_params *p, const uint64_t *seeds) {
+    CKR(enter(ctx, "sc_ens_set_params"));
+    if (!ctx->ens) return fail(ctx, "sc_ens_set_params: sc_ens_configure has not been called");
+    if (!p || !seeds) return fail(ctx, "sc_ens_set_params: NULL argument");
+    for (uint32_t m = 1; m < ctx->members; ++m) {  // refused before anything changes
+        if (std::memcmp(&p[m].dt, &p[0].dt, sizeof(double)))
+            return fail(ctx, "sc_ens_set_params: dt differs between member 0 and member " + std::to_string(m) +
+                                 " (the members share dt)");
+        if (std::memcmp(&p[m].particle_radius, &p[0].particle_radius, sizeof(double)))
+            return fail(ctx, "sc_ens_set_params: particle_radius differs between member 0 and member " +
+                                 std::to_string(m) + " (the members share particle_radius)");
+    }
+    const bool same = ctx->params_set &&
+                      std::memcmp(ctx->ens_hp.data(), p, sizeof(sc_params) * ctx->members) == 0 &&
+                      std::memcmp(ctx->ens_seeds.data(), seeds, sizeof(uint64_t) * ctx->members) == 0;
+    CKR(set_params(ctx, &p[0]));  // the shared part: radius, grid, walls' padding
+    if (same) return 0;           // the same bytes again leave the next tick's keys valid
+    CKR(drop_keys(ctx));
+    std::memcpy(ctx->ens_hp.data(), p, sizeof(sc_params) * ctx->members);
+    std::memcpy(ctx->ens_seeds.data(), seeds, sizeof(uint64_t) * ctx->members);
+    return ens_upload(ctx);
+}
+
+extern "C" int sc_ens_set_state(sc_ctx *ctx, const double *pos, const double *vel, const int64_t *counts,
+                                const uint32_t *uid, const uint32_t *next_local) {
+    CKR(enter(ctx, "sc_ens_set_state"));
+    if (!ctx->ens) return fail(ctx, "sc_ens_set_state: sc_ens_configure has not been called");
+    if (!counts) return fail(ctx, "sc_ens_set_state: NULL argument");
+    if (ctx->in_step) return fail(ctx, "sc_ens_set_state: inside a split step");
+    const uint32_t M = ctx->members, B = ctx->uid_bits, mask = (1u << B) - 1u;
+    int64_t n = 0;
+    for (uint32_t m = 0; m < M; ++m) {
+        if (counts[m] < 0 || counts[m] > ((int64_t)1 << B))
+            return fail(ctx, "sc_ens_set_state: member " + std::to_string(m) + " has more particles than its " +
+                                 std::to_string(B) + " identity bits can number");
+        n += counts[m];
+    }
+    if (n > ctx->cap) return fail(ctx, "sc_ens_set_state: n exceeds capacity");
+    std::vector<uint32_t> u((size_t)n), cnt(M), next(M);
+    for (uint32_t m = 0, k = 0; m < M; ++m) {
+        uint64_t top = 0;  // one past the member's largest local uid
+        for (int64_t i = 0; i < counts[m]; ++i, ++k) {
+            u[k] = uid ? uid[k] : ((m << B) | (uint32_t)i);
+            if ((u[k] >> B) != m || (u[k] & SC_GHOST_BIT))
+                return fail(ctx, "sc_ens_set_state: uid of row " + std::to_string(k) + " is not one of member " +
+                                     std::to_string(m) + "'s (the rows are member-major)");
+            top = std::max<uint64_t>(top, (uint64_t)(u[k] & mask) + 1);
+        }
+        if (next_local && (uint64_t)next_local[m] < top)
+            return fail(ctx, "sc_ens_set_state: next_local of member " + std::to_string(m) + " is below its uids");
+        if (next_local && (uint64_t)next_local[m] > ((uint64_t)1 << B))
+            return fail(ctx, "sc_ens_set_state: next_local of member " + std::to_string(m) + " passes 2^uid_bits");
+        cnt[m] = (uint32_t)counts[m];
+        next[m] = next_local ? next_local[m] : (uint32_t)top;
+    }
+    CKR(set_state(ctx, pos, vel, n));
+    if (n) CK(cudaMemcpyAsync(ctx->uid_cur, u.data(), sizeof(uint32_t) * (size_t)n, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->ens_count, cnt.data(), sizeof(uint32_t) * M, cudaMemcpyHostToDevice, ctx->stream));
+    CK(cudaMemcpyAsync(ctx->ens_next_dev, next.data(), sizeof(uint32_t) * M, cudaMemcpyHostToDevice, ctx->stream));
+    for (uint32_t m = 0; m < M; ++m) { ctx->ens_next[m] = next[m]; ctx->ens_bound[m] = cnt[m]; }
+    ctx->ens_stale = false;
+    ctx->next_uid = (uint32_t)((uint64_t)M << B);
+    return 0;
+}
+
+// k_emit_members for members m0 .. m0 + mc - 1; `w` = their [max_particles | counts] (EnsEmitParams)
+template <int kWords>
+static int launch_emit_members(sc_ctx *ctx, const EnsEmitHead &H, const uint32_t *w, uint32_t words) {
+    EnsEmitParams<kWords> E{};
+    E.h = H;
+    std::memcpy(E.w, w, sizeof(uint32_t) * words);
+    if (ctx->precision == SC_PRECISION_F64)
+        CK(launch_pdl(k_emit_members<double, kWords>, dim3(1), dim3(SC_EMIT_THREADS), ctx->stream, ctx->cnt, E,
+                      ctx->ens_next_dev, (const unsigned long long *)ctx->ens_seed, ctx->ens_count,
+                      (const uint32_t *)ctx->cell_start, ctx->pos_cur, (double2 *)ctx->vel_cur, ctx->uid_cur,
+                      (uint32_t)ctx->cap));
+    else
+        CK(launch_pdl(k_emit_members<float, kWords>, dim3(1), dim3(SC_EMIT_THREADS), ctx->stream, ctx->cnt, E,
+                      ctx->ens_next_dev, (const unsigned long long *)ctx->ens_seed, ctx->ens_count,
+                      (const uint32_t *)ctx->cell_start, ctx->pos_cur, (float2 *)ctx->vel_cur, ctx->uid_cur,
+                      (uint32_t)ctx->cap));
+    return 0;
+}
+
+extern "C" int sc_ens_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsources, const int32_t *counts,
+                                     const int64_t *max_particles) {
+    CKR(enter(ctx, "sc_ens_emit_particles"));
+    if (!ctx->ens) return fail(ctx, "sc_ens_emit_particles: sc_ens_configure has not been called");
+    if (nsources > 0 && (!sources || !counts || !max_particles)) return fail(ctx, "sc_ens_emit_particles: NULL argument");
+    if (ctx->in_step) return fail(ctx, "sc_ens_emit_particles: inside a split step");
+    if (nsources < 0 || nsources > SC_MAX_SOURCES)
+        return fail(ctx, "sc_ens_emit_particles: more than SC_MAX_SOURCES sources");
+    const uint32_t M = ctx->members;
+    const uint64_t room = 1ull << ctx->uid_bits;
+    uint64_t total = 0, need = 0;
+    std::vector<uint64_t> drawn(M), bound(M);
+    std::vector<uint32_t> maxp(M);
+    for (uint32_t m = 0; m < M; ++m) {
+        for (int q = 0; q < nsources; ++q) {
+            const int32_t c = counts[(size_t)m * nsources + q];
+            if (c < 0) return fail(ctx, "sc_ens_emit_particles: negative count");
+            drawn[m] += (uint64_t)c;
+        }
+        if (ctx->ens_next[m] + drawn[m] > room)
+            return fail(ctx, "member " + std::to_string(m) + ": particle identities exhausted (2^" +
+                                 std::to_string(ctx->uid_bits) + " particles created in this member)");
+        maxp[m] = (uint32_t)std::min<int64_t>(std::max<int64_t>(max_particles[m], 0), 0xFFFFFFFFLL);
+        // the clamp takes a count P to at most max(P, min(P + drawn, max_particles)), which grows with P
+        bound[m] = std::max<uint64_t>(ctx->ens_bound[m], std::min<uint64_t>(ctx->ens_bound[m] + drawn[m], maxp[m]));
+        need += bound[m];
+        total += drawn[m];
+    }
+    if (!total) return 0;
+    // every particle the members' clamps let in must fit: refused here, before anything is launched, instead of the
+    // device dropping draws a separate context with these max_particles would keep
+    if (need > (uint64_t)ctx->cap)
+        return fail(ctx, "sc_ens_emit_particles: the members' max_particles let their counts reach " +
+                             std::to_string(need) + " particles, more than the capacity " + std::to_string(ctx->cap) +
+                             " (create the context with room for the sum of the members' max_particles)");
+    EnsEmitHead H{};
+    H.nsrc = nsources; H.from_scan = ctx->ens_stale;
+    H.uid_bits = ctx->uid_bits; H.ncells = ctx->grid.ncells / M; H.tick = ctx->tick;
+    for (int q = 0; q < nsources; ++q) {
+        EnsEmitSource &S = H.src[q];
+        S.px = sources[q].position_x; S.py = sources[q].position_y; S.radius = sources[q].radius;
+        S.vx = sources[q].velocity_x; S.vy = sources[q].velocity_y; S.vnoise = sources[q].velocity_noise;
+        S.index = sources[q].index;
+    }
+    CKR(drop_keys(ctx));  // the new particles have no keys
+    refresh_count(ctx);
+    // members go in launches of as many as fit one launch's parameters (one launch for every M * (nsources + 1) <= 7936)
+    const uint32_t per = SC_EMIT_WORDS / (uint32_t)(nsources + 1);
+    std::vector<uint32_t> w;
+    for (uint32_t m0 = 0; m0 < M; m0 += per) {
+        const uint32_t mc = std::min(per, M - m0), words = mc * (uint32_t)(nsources + 1);
+        w.assign(words, 0u);
+        for (uint32_t j = 0; j < mc; ++j) {
+            w[j] = maxp[m0 + j];
+            for (int q = 0; q < nsources; ++q) w[mc + (size_t)j * nsources + q] = (uint32_t)counts[(size_t)(m0 + j) * nsources + q];
+        }
+        H.m0 = m0; H.members = mc;
+        ProfScope ps(ctx, SLOT_IO);
+        if (words <= SC_EMIT_WORDS_SMALL) CKR(launch_emit_members<SC_EMIT_WORDS_SMALL>(ctx, H, w.data(), words));
+        else CKR(launch_emit_members<SC_EMIT_WORDS>(ctx, H, w.data(), words));
+    }
+    for (uint32_t m = 0; m < M; ++m) { ctx->ens_next[m] += (uint32_t)drawn[m]; ctx->ens_bound[m] = bound[m]; }
+    ctx->ens_stale = false;
+    ctx->n_host = std::min<int64_t>(ctx->n_host + (int64_t)total, ctx->cap);  // an upper bound: the clamp is on the device
+    ctx->n_exact = false;
+    ctx->srt_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
+    return 0;
+}
+
+extern "C" int sc_ens_member_counts(sc_ctx *ctx, int64_t *counts, uint32_t *counts_dev) {
+    CKR(enter(ctx, "sc_ens_member_counts"));
+    if (!ctx->ens) return fail(ctx, "sc_ens_member_counts: sc_ens_configure has not been called");
+    const uint32_t M = ctx->members;
+    if (ctx->ens_stale || counts_dev) {
+        ProfScope ps(ctx, SLOT_IO);
+        k_member_counts<<<blocks_for(M), SC_BLOCK, 0, ctx->stream>>>(M, ctx->grid.ncells / M, ctx->ens_stale ? 1 : 0,
+                                                                      ctx->cell_start, ctx->ens_count, counts_dev);
+        ctx->ens_stale = false;
+        CK(cudaGetLastError());
+    }
+    if (!counts) return 0;
+    std::vector<uint32_t> h(M);
+    CK(cudaMemcpyAsync(h.data(), ctx->ens_count, sizeof(uint32_t) * M, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(stream_sync(ctx));
+    for (uint32_t m = 0; m < M; ++m) counts[m] = h[m];
+    return 0;
+}
+
+extern "C" int sc_ens_get_state(sc_ctx *ctx, double *pos, double *vel, double *pressure, int64_t cap, int64_t *offsets) {
+    CKR(enter(ctx, "sc_ens_get_state"));
+    if (!ctx->ens) return fail(ctx, "sc_ens_get_state: sc_ens_configure has not been called");
+    if (!offsets) return fail(ctx, "sc_ens_get_state: NULL argument");
+    std::vector<int64_t> c(ctx->members);
+    CKR(sc_ens_member_counts(ctx, c.data(), nullptr));
+    offsets[0] = 0;
+    for (uint32_t m = 0; m < ctx->members; ++m) offsets[m + 1] = offsets[m] + c[m];
+    int64_t n = 0;
+    CKR(sc_get_state(ctx, pos, vel, pressure, cap, &n));
+    if (n != offsets[ctx->members])
+        return fail(ctx, "sc_ens_get_state: member counts (" + std::to_string(offsets[ctx->members]) +
+                             ") disagree with the live count (" + std::to_string(n) + ")");
     return 0;
 }

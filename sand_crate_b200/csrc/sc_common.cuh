@@ -60,6 +60,21 @@ struct DevParams {
     float f_dt, f_dt_gx, f_dt_gy, f_dt_amp, f_dt_visc, f_smooth, f_two_target, f_ignored;
 };
 
+// ---- ensembles (DESIGN.md section 12): M members of one scene stepped as one particle set ----------------------------
+// Member m's cells are m * ncells + its own cell of the scene's grid (whose margin rows and columns stay empty, so no 3x3
+// neighborhood reaches another member), and its uids are (m << uid_bits) | local uid.  The ensemble instantiations of
+// the step's kernels (kEns = true) take this as their LAST parameter, so the single-scene instantiations keep every
+// parameter offset.  `params` holds each member's DevParams (noise_mode = its effective mode; tick_key unused: the key
+// is tick_key(seed[m], tick), computed per thread from the launch's tick, so nothing is uploaded per tick).
+struct Members {
+    const DevParams *params;
+    const unsigned long long *seed;
+    const uint32_t *uid;  // the uids of the arrays the kernel indexes by particle
+    unsigned long long tick;
+    uint32_t uid_bits, ncells;  // identity bits of one member, cells of one member's grid
+    int nrows;                  // rows of one member's grid
+};
+
 struct WallParams {
     int S;
     int nbodies;
@@ -178,6 +193,26 @@ __host__ __device__ inline uint32_t pair_noise_bits(uint64_t tkey, uint32_t uid_
     const uint32_t a = uid_i & 0x7FFFFFFFu, b = uid_j & 0x7FFFFFFFu;
     return lowbias32((a * 0x9E3779B1u) ^ (b * 0x85EBCA77u) ^ ((uint32_t)tkey ^ (uint32_t)(tkey >> 32)));
 }
+__device__ __forceinline__ uint32_t member_of(const Members &E, uint32_t uid) { return uid >> E.uid_bits; }
+__device__ __forceinline__ DevParams member_params(const Members &E, uint32_t uid) {
+    const uint32_t m = member_of(E, uid);
+    DevParams p = E.params[m];
+    p.tick_key = tick_key(E.seed[m], E.tick);
+    return p;
+}
+// the kernel's own parameters, or the member's
+template <bool kEns>
+__device__ __forceinline__ const DevParams &pick_params(const DevParams &P, const DevParams &Pm) {
+    if constexpr (kEns) return Pm;
+    else return P;
+}
+// the uid the pair noise hashes: a member draws the noise of a separate context, so only its local identity counts
+template <bool kEns>
+__device__ __forceinline__ uint32_t noise_uid(const Members &E, uint32_t uid) {
+    if constexpr (kEns) return uid & ((1u << E.uid_bits) - 1u);
+    else return uid;
+}
+
 // ---- counter-based particle sources (production mode; oracle/step_oracle.c restates it) ---------------------
 // Stream of source q at a tick: element j is u(j) = (mix64(source_key(tick_key, q) + (j + 1) * GOLDEN) >> 11) * 2^-53.
 // j = 0 feeds the host's binomial draw of the emission count; particle k uses j = 1 + 4 k + {0: x, 1: y, 2: vx, 3: vy}.
@@ -261,9 +296,10 @@ struct KeyOut {
     uint32_t *wall_bits, *wall_slot, *n_wall;
     double2 *pos, *wall_pre;
 };
-template <bool kStep>
+// kEns: the particle belongs to the ensemble member whose grid starts at cell `cell_base` (Members)
+template <bool kStep, bool kEns = false>
 __device__ __forceinline__ void key_particle(const Grid &g, const DevParams &P, const WallParams &W, const KeyOut &O,
-                                             uint32_t i, double2 p) {
+                                             uint32_t i, double2 p, uint32_t cell_base = 0u) {
     if (kStep) {
         const bool out = (p.x < P.box_lo) | (p.x > P.box_hi) | (p.y < P.box_lo) | (p.y > P.box_hi);
         if (out) {
@@ -302,7 +338,8 @@ __device__ __forceinline__ void key_particle(const Grid &g, const DevParams &P, 
         }
     }
     int row;
-    const uint32_t c = cell_of(g, p.x, p.y, row);
+    uint32_t c = cell_of(g, p.x, p.y, row);
+    if constexpr (kEns) c += cell_base;
     atomicAdd(&O.cell_count[c], 1u);  // result unused: a fire-and-forget reduction (RED), no round trip
     O.cell_key[i] = c;
 }

@@ -104,11 +104,12 @@ __device__ __forceinline__ int collect_neighbors(uint32_t s, uint32_t c, const G
 // w = 1 - clip(dist / d, 0, 1) (crate.py:270).
 struct PairGeom { double nx, ny, w; };
 
-template <int kNoise>
+// kEns: P is a member's, whose own effective noise mode decides (a member with a zero noise level draws none)
+template <int kNoise, bool kEns = false>
 __device__ __forceinline__ PairGeom pair_geom_f64(const DevParams &P, double2 pi, double2 pj, uint32_t uid_i,
                                                   uint32_t uid_j, const double *host_noise, uint32_t noise_index) {
     double qx = pj.x, qy = pj.y;
-    if constexpr (kNoise != SC_NOISE_NONE) {
+    if constexpr (kNoise != SC_NOISE_NONE) if (!kEns || P.noise_mode == kNoise) {
         double ux, uy;
         if constexpr (kNoise == SC_NOISE_HOST) {
             ux = host_noise[2 * (size_t)noise_index];
@@ -161,14 +162,14 @@ __device__ inline double np_sum_1d(const double *a, int n) {
 // is consumed by K5, so the pair geometry - noise hash, reciprocal square root - is evaluated once per tick instead
 // of twice.  HBM is the idle resource on this path (the kernels are issue / L1 bound), so 12 bytes per pair are a
 // good trade.
-template <int kNoise>  // kNoise: SC_NOISE_* resolved at compile time (no branch in the pair loop)
+template <int kNoise, bool kEns = false>  // kNoise: SC_NOISE_* resolved at compile time (no branch in the pair loop)
 __global__ void __launch_bounds__(SC_BLOCK)
-k_density(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
+k_density(Counters *cnt, Grid g, DevParams P0, const uint32_t *cell_start,
           const double2 *pos, const float2 *rel, const uint32_t *cell_key,
           const uint32_t *uid, const double *host_noise,
           const uint32_t *noise_off, const uint32_t *rank_of_uid,
           uint32_t *pair_j, double2 *pair_n,
-          uint32_t *pair_off, uint8_t *pair_cnt, PS<double> *ps_out, NextWallClear next) {
+          uint32_t *pair_off, uint8_t *pair_cnt, PS<double> *ps_out, NextWallClear next, Members E) {
     pdl_enter();
     clear_next_walls(next);
     __shared__ uint32_t s_list[SC_MAX_NEIGHBORS * SC_BLOCK];
@@ -198,6 +199,9 @@ k_density(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
     pair_off[s] = off;
     pair_cnt[s] = (uint8_t)K;
     const uint32_t uid_s = uid[s];
+    DevParams Pm;
+    if constexpr (kEns) Pm = member_params(E, uid_s);
+    const DevParams &P = pick_params<kEns>(P0, Pm);
     uint32_t nbase = 0u;
     if constexpr (kNoise == SC_NOISE_HOST) nbase = noise_off[rank_of_uid[uid_s]];
     double ax = 0, ay = 0;
@@ -205,7 +209,8 @@ k_density(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
     const double2 ps64 = pos[s];
     for (int k = 0; k < K; ++k) {
         const uint32_t j = lst.get(k) & SC_IDX_MASK;
-        const PairGeom pg = pair_geom_f64<kNoise>(P, ps64, pos[j], uid_s, uid[j], host_noise, nbase + (uint32_t)k);
+        const PairGeom pg = pair_geom_f64<kNoise, kEns>(P, ps64, pos[j], noise_uid<kEns>(E, uid_s),
+                                                        noise_uid<kEns>(E, uid[j]), host_noise, nbase + (uint32_t)k);
         pair_j[(size_t)off + k] = j;
         pair_n[(size_t)off + k] = make_double2(pg.nx, pg.ny);
         wl[k] = pg.w;
@@ -234,7 +239,8 @@ struct NextKeys { Grid g; KeyOut out; };
 // Everything of K5 that follows the pair loop, for particle s: wall contact rows of F5, F3-F6 velocity updates, wall
 // bounce, continuous collision, integration, and the next tick's key pass.  `visc(vx, vy, ax, ay)` supplies
 // sum_j (v_j - v) (crate.py:319-323).
-template <typename Real, bool kMonitor, typename ViscFn>
+// kEns: P is the particle's member's, `cell_base` the first cell of its grid (Members); nk.g is one member's grid
+template <typename Real, bool kMonitor, bool kEns = false, typename ViscFn>
 __device__ __forceinline__ void force_tail(uint32_t s, int K, Real p_i, Real tx, Real ty, Real qx, Real qy,
                                            const DevParams &P, const WallParams &W, const double2 ps,
                                            const typename Vec2<Real>::type v0, const bool touching,
@@ -242,11 +248,11 @@ __device__ __forceinline__ void force_tail(uint32_t s, int K, Real p_i, Real tx,
                                            const double2 *wall_pre, double2 *pos_out,
                                            typename Vec2<Real>::type *vel_out,
                                            double *monitor, const uint32_t *n_ptr,
-                                           const NextKeys &nk, ViscFn visc) {
+                                           const NextKeys &nk, ViscFn visc, uint32_t cell_base = 0u) {
     typedef typename Vec2<Real>::type R2;
     auto store_pos = [&](double2 po) {
         pos_out[s] = po;
-        if (nk.out.cell_count) key_particle<true>(nk.g, P, W, nk.out, s, po);
+        if (nk.out.cell_count) key_particle<true, kEns>(nk.g, P, W, nk.out, s, po, cell_base);
     };
     double mon[6] = {0, 0, 0, 0, 0, 0};
     double mpx = 0, mpy = 0;  // velocity before the current stage
@@ -398,20 +404,28 @@ __device__ __forceinline__ void force_tail(uint32_t s, int K, Real p_i, Real tx,
 #ifndef SC_K5_MINBLOCKS
 #define SC_K5_MINBLOCKS 1
 #endif
-template <bool kMonitor>
+template <bool kMonitor, bool kEns = false>
 __global__ void __launch_bounds__(SC_BLOCK, SC_K5_MINBLOCKS)
-k_force(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallParams W,
+k_force(const uint32_t *n_ptr, DevParams P0, const __grid_constant__ WallParams W,
         const double2 *pos, const double2 *vel,
         const uint32_t *pair_j, const double2 *pair_n,
         const uint32_t *pair_off, const uint8_t *pair_cnt,
         const PS<double> *ps_in, const uint32_t *wall_bits,
         const uint32_t *wall_slot, const double2 *wall_pre,
         double2 *pos_out, double2 *vel_out,
-        double *monitor, TickDuty duty, NextKeys nk) {
+        double *monitor, TickDuty duty, NextKeys nk, Members E) {
     pdl_enter();
     end_of_tick(duty, n_ptr);
     const uint32_t s = blockIdx.x * blockDim.x + threadIdx.x;
     if (s >= *n_ptr) return;
+    DevParams Pm;
+    uint32_t cell_base = 0u;
+    if constexpr (kEns) {
+        const uint32_t u = E.uid[s];
+        Pm = member_params(E, u);
+        cell_base = member_of(E, u) * E.ncells;
+    }
+    const DevParams &P = pick_params<kEns>(P0, Pm);
     const PS<double> me = ps_in[s];
     const double p_i = me.p;
     const uint32_t off = pair_off[s];
@@ -458,14 +472,15 @@ k_force(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallParams W
     const double2 ps_own = pos[s];
     const double2 v_own = vel[s];
     const bool touching = (wall_bits[s >> 5] >> (s & 31)) & 1u;
-    force_tail<double, kMonitor>(s, K, p_i, tx, ty, qx, qy, P, W, ps_own, v_own, touching, wall_slot, wall_pre, pos_out,
-                                 vel_out, monitor, n_ptr, nk, [&](double vx, double vy, double &ax, double &ay) {
+    force_tail<double, kMonitor, kEns>(s, K, p_i, tx, ty, qx, qy, P, W, ps_own, v_own, touching, wall_slot, wall_pre,
+                                       pos_out, vel_out, monitor, n_ptr, nk,
+                                       [&](double vx, double vy, double &ax, double &ay) {
         for (int q = 0; q < K; ++q) {
             const double2 vj = vel[pair_j[(size_t)off + q]];
             const double ex = vj.x - vx, ey = vj.y - vy;
             if (q == 0) { ax = ex; ay = ey; } else { ax += ex; ay += ey; }
         }
-    });
+    }, cell_base);
 }
 
 }  // namespace sc

@@ -18,10 +18,11 @@ namespace sc {
 #ifndef SC_PREPASS_ILP
 #define SC_PREPASS_ILP 2
 #endif
-template <bool kStep, bool kUnpack = false>  // kUnpack: the strip variant that appends the neighbors' records itself
+// kEns: an ensemble (Members, sc_common.cuh); `g` is then the grid of ONE member
+template <bool kStep, bool kUnpack = false, bool kEns = false>  // kUnpack: the strip variant that appends the neighbors' records itself
 __global__ void __launch_bounds__(SC_BLOCK, 6)  // the wall path may spill; it is rare
 k_prepass(Counters *cnt, Grid g, DevParams P, const __grid_constant__ WallParams W, KeyOut O, uint32_t cap,
-          PrepassUnpack U) {
+          PrepassUnpack U, Members E) {
     pdl_enter();
     const uint32_t b0 = blockIdx.x * (SC_BLOCK * SC_PREPASS_ILP);
     const uint32_t i0 = b0 + threadIdx.x;
@@ -79,7 +80,11 @@ k_prepass(Counters *cnt, Grid g, DevParams P, const __grid_constant__ WallParams
 #pragma unroll
     for (int u = 0; u < SC_PREPASS_ILP; ++u) {
         const uint32_t i = i0 + u * SC_BLOCK;
-        if (i < n) key_particle<kStep>(g, P, W, O, i, p[u]);
+        if constexpr (kEns) {
+            if (i < n) key_particle<kStep, true>(g, P, W, O, i, p[u], member_of(E, E.uid[i]) * E.ncells);
+        } else {
+            if (i < n) key_particle<kStep>(g, P, W, O, i, p[u]);
+        }
     }
 }
 
@@ -207,7 +212,8 @@ k_place(const Counters *cnt, const uint32_t *cell_key, uint32_t *cell_count,
 
 // K3: rank inside the cell by (x, uid) and gather the particle record to its final sorted position.
 // Produces exactly np.lexsort((x, floor(y / d))) (collision_detector.py:127) as the concatenation of cells.
-template <typename Real>
+// kEns: the grid is the members' grids stacked (Members); a cell row is then a row of its member's grid
+template <typename Real, bool kEns = false>
 __global__ void __launch_bounds__(SC_BLOCK)
 k_rank_gather(Counters *cnt, Grid g, const uint32_t *cell_start, const uint32_t *tmpidx,
               const uint32_t *cell_key, const double2 *pos,
@@ -216,7 +222,7 @@ k_rank_gather(Counters *cnt, Grid g, const uint32_t *cell_start, const uint32_t 
               double2 *pos_s, float2 *rel_s,
               typename Vec2<Real>::type *vel_s, uint32_t *uid_s,
               uint32_t *cell_key_s, uint32_t *wall_bits_s,
-              uint32_t *wall_slot_s, SearchRec *rec_s, BlockDesc *desc) {
+              uint32_t *wall_slot_s, SearchRec *rec_s, BlockDesc *desc, Members E) {
     pdl_enter();
     const uint32_t n = cell_start[g.ncells];
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
@@ -247,7 +253,9 @@ k_rank_gather(Counters *cnt, Grid g, const uint32_t *cell_start, const uint32_t 
     const uint32_t f = beg + rank;
     pos_s[f] = p;
     {   // cell-relative fp32 copy for the pair kernels' screening (see collect_neighbors)
-        const uint32_t cr = c / (uint32_t)g.ncols, cc = c - cr * (uint32_t)g.ncols;
+        uint32_t cr = c / (uint32_t)g.ncols;
+        const uint32_t cc = c - cr * (uint32_t)g.ncols;
+        if constexpr (kEns) cr %= (uint32_t)E.nrows;
         float2 r;
         r.x = (float)(p.x - (double)((int)cc + g.col_min) * g.d);
         r.y = (float)(p.y - (double)((int)cr + g.row_min) * g.d);
@@ -459,6 +467,88 @@ k_emit(Counters *cnt, const __grid_constant__ EmitParams E, double2 *pos, typena
             uid[at] = S.uid_base + k;
         }
     }
+}
+
+// The same for the members of an ensemble (sc_ens_emit_particles).  Member m draws its own counts from its own stream
+// (key: the member's seed) and is clamped against ITS live count: mcount[m], or - when a step ran since mcount was
+// written (`from_scan`) - the member's share of that step's cell scan, which is its count after that tick's removal.  Its
+// identities continue from next_local[m] and advance by the drawn count.  Everything the host draws travels in the
+// launch's parameters (w = [max_particles | drawn counts members x nsrc] of members m0 .. m0 + members - 1), so no host
+// buffer is copied per tick; members beyond one launch's parameter space go in further launches, each appending behind
+// the last (the host caps the total, so the capacity test below never drops a particle).  One block, a thread per
+// member, members in chunks of the block.
+struct EnsEmitSource { double px, py, radius, vx, vy, vnoise; uint32_t index; };
+struct EnsEmitHead {
+    EnsEmitSource src[SC_MAX_SOURCES];
+    int nsrc, from_scan;
+    uint32_t m0, members, uid_bits, ncells;  // ncells: cells of one member's grid
+    unsigned long long tick;
+};
+template <int kWords> struct EnsEmitParams { EnsEmitHead h; uint32_t w[kWords]; };
+#define SC_EMIT_WORDS_SMALL 256   // launches whose draws fit 1 KB pay for no more parameter space
+#define SC_EMIT_WORDS 7936        // the largest that keeps the parameters within the 32 764 bytes a launch may take
+static_assert(sizeof(EnsEmitParams<SC_EMIT_WORDS>) <= 32764, "kernel parameter space");
+#define SC_EMIT_THREADS 1024
+template <typename Real, int kWords>
+__global__ void __launch_bounds__(SC_EMIT_THREADS)
+k_emit_members(Counters *cnt, const __grid_constant__ EnsEmitParams<kWords> E, uint32_t *next_local,
+               const unsigned long long *seed, uint32_t *mcount, const uint32_t *cell_start, double2 *pos,
+               typename Vec2<Real>::type *vel, uint32_t *uid, uint32_t cap) {
+    pdl_enter();
+    const uint32_t M = E.h.members;
+    const uint32_t *maxp = E.w, *draw = E.w + M;
+    const uint32_t n0 = cnt->n;
+    uint32_t run = 0;  // particles placed by the chunks before
+    for (uint32_t c0 = 0; c0 < M; c0 += SC_EMIT_THREADS) {
+        const uint32_t j = c0 + threadIdx.x, m = E.h.m0 + j;
+        uint32_t a[SC_MAX_SOURCES], mine = 0;
+        if (j < M) {
+            uint32_t P = E.h.from_scan ? cell_start[(size_t)(m + 1) * E.h.ncells] - cell_start[(size_t)m * E.h.ncells] : mcount[m];
+            for (int q = 0; q < E.h.nsrc; ++q) {
+                const uint32_t room = maxp[j] > P ? maxp[j] - P : 0u, n = draw[(size_t)j * E.h.nsrc + q];
+                a[q] = n < room ? n : room;
+                P += a[q];
+                mine += a[q];
+            }
+            mcount[m] = P;
+        }
+        uint32_t total;
+        const uint32_t before = block_exclusive_scan_n<SC_EMIT_THREADS>(mine, total);
+        if (j < M) {
+            const uint64_t tkey = tick_key(seed[m], E.h.tick);
+            uint32_t at = n0 + run + before, local = next_local[m];
+            for (int q = 0; q < E.h.nsrc; ++q) {
+                const EnsEmitSource &S = E.h.src[q];
+                const uint64_t key = source_key(tkey, S.index);
+                for (uint32_t k = 0; k < a[q]; ++k, ++at) {
+                    if (at >= cap) { cnt->overflow = 1u; break; }
+                    const double ux = source_uniform(key, 1ull + 4ull * k), uy = source_uniform(key, 2ull + 4ull * k);
+                    const double wx = source_uniform(key, 3ull + 4ull * k), wy = source_uniform(key, 4ull + 4ull * k);
+                    pos[at] = make_double2((ux - 0.5) * S.radius + S.px, (uy - 0.5) * S.radius + S.py);   // as k_emit
+                    typename Vec2<Real>::type v;
+                    v.x = (Real)(S.vx + (wx - 0.5) * S.vnoise);
+                    v.y = (Real)(S.vy + (wy - 0.5) * S.vnoise);
+                    vel[at] = v;
+                    uid[at] = (m << E.h.uid_bits) | (local + k);
+                }
+                local += draw[(size_t)j * E.h.nsrc + q];
+            }
+            next_local[m] = local;
+        }
+        run += total;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) cnt->n = n0 + run < cap ? n0 + run : cap;
+}
+
+// per-member live counts: mcount[m], refreshed from the last step's cell scan when `from_scan`; copied to `out` (or NULL)
+__global__ void __launch_bounds__(SC_BLOCK)
+k_member_counts(uint32_t M, uint32_t ncells, int from_scan, const uint32_t *cell_start, uint32_t *mcount, uint32_t *out) {
+    const uint32_t m = blockIdx.x * blockDim.x + threadIdx.x;
+    if (m >= M) return;
+    const uint32_t v = from_scan ? cell_start[(size_t)(m + 1) * ncells] - cell_start[(size_t)m * ncells] : mcount[m];
+    mcount[m] = v;
+    if (out) out[m] = v;
 }
 
 // min / max cell coordinates of an arbitrary point set (standalone detect_particle_collisions)

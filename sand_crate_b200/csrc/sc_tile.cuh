@@ -211,11 +211,14 @@ struct HostNoise { const double *u; const uint32_t *off, *rank_of_uid; };
 // K4 body for one particle.  s = sorted index; b[] = the six boundaries of its four candidate ranges as LOCAL
 // indices (m0, m3 | n0, n3 | p0, p3 of collect_neighbors, shifted into the staged windows).  List order = reference
 // list order.
-template <int kNoise, class Acc, class List>
+// kEns: the pair geometry and pressure take the particle's member's parameters and noise (Members); the search only
+// depends on the diameter, which all members share
+template <int kNoise, bool kEns, class Acc, class List>
 __device__ __forceinline__ void density_particle(const Acc &A, List lst, const TileWindows &w, bool live, uint32_t s,
                                                  const uint32_t (&b)[6], const Grid &g, const DevParams &P,
                                                  const double2 *pos, uint2 *pair_rec,
-                                                 uint8_t *pair_cnt, PS<float> *ps_out, const HostNoise &hn) {
+                                                 uint8_t *pair_cnt, PS<float> *ps_out, const HostNoise &hn,
+                                                 const Members &E) {
     const float df = P.f_d;
     const uint32_t d0 = w.off[0] - w.base[0], d1 = w.off[1] - w.base[1], d2 = w.off[2] - w.base[2];
     int K = 0;
@@ -267,8 +270,11 @@ __device__ __forceinline__ void density_particle(const Acc &A, List lst, const T
     if (!live) return;
     pair_cnt[s] = (uint8_t)K;
     const uint32_t uid_s = __float_as_uint(me.w);
+    DevParams Pm;
+    if constexpr (kEns) Pm = member_params(E, uid_s);
+    const DevParams &PP = pick_params<kEns>(P, Pm);
     const float inv_d = P.f_inv_d;
-    const float amp = P.f_amp;
+    const float amp = PP.f_amp;
     uint32_t nbase = 0u;
     if constexpr (kNoise == SC_NOISE_HOST) nbase = hn.off[hn.rank_of_uid[uid_s]];
     float ax = 0, ay = 0, psum = 0;
@@ -281,10 +287,13 @@ __device__ __forceinline__ void density_particle(const Acc &A, List lst, const T
         float ry = (me.y - r.y) - fmaf((float)code, df, -df);  // the neighbor's row is dr * d further down
         // crate.py:167-174: the neighbor's position is noised, then the unit vector from it to i and the distance
         if constexpr (kNoise == SC_NOISE_COUNTER) {
-            float fx, fy;  // uniforms + 1
-            pair_noise_f32_1to2(pair_noise_bits(P.tick_key, uid_s, __float_as_uint(r.w)), fx, fy);
-            rx = fmaf(1.5f - fx, amp, rx);  // 0.5 - u, exact
-            ry = fmaf(1.5f - fy, amp, ry);
+            if (!kEns || PP.noise_mode == SC_NOISE_COUNTER) {
+                float fx, fy;  // uniforms + 1
+                pair_noise_f32_1to2(pair_noise_bits(PP.tick_key, noise_uid<kEns>(E, uid_s),
+                                                    noise_uid<kEns>(E, __float_as_uint(r.w))), fx, fy);
+                rx = fmaf(1.5f - fx, amp, rx);  // 0.5 - u, exact
+                ry = fmaf(1.5f - fy, amp, ry);
+            }
         } else if constexpr (kNoise == SC_NOISE_HOST) {
             const size_t q = 2 * (size_t)(nbase + (uint32_t)k);
             const float ux = (float)hn.u[q], uy = (float)hn.u[q + 1];
@@ -304,7 +313,7 @@ __device__ __forceinline__ void density_particle(const Acc &A, List lst, const T
     }
     float p = 0;
     if (K > 0) {
-        const float pr = psum - P.f_ignored;
+        const float pr = psum - PP.f_ignored;
         p = (pr > 0 || pr != pr) ? pr : 0.0f;  // np.maximum(0, pr), crate.py:273
     }
     PS<float> o;
@@ -318,13 +327,13 @@ __device__ __forceinline__ void density_particle(const Acc &A, List lst, const T
 #ifndef SC_TILE_RESIDENT
 #define SC_TILE_RESIDENT 1536  // threads per SM the register allocation is held to (1536 = 40 registers)
 #endif
-template <int kNoise>
+template <int kNoise, bool kEns = false>
 __global__ void __launch_bounds__(SC_TILE, SC_TILE_RESIDENT / SC_TILE)
 k_density_tile(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
                const BlockDesc *desc, const double2 *pos,
                const SearchRec *rec, const uint32_t *cell_key,
                uint2 *pair_rec, uint8_t *pair_cnt, PS<float> *ps_out, NextWallClear next,
-               HostNoise hn) {  // last: the other parameters keep their offsets in every instantiation
+               HostNoise hn, Members E) {  // last: the other parameters keep their offsets in every instantiation
     pdl_enter();
     clear_next_walls(next);
     // staged: [records 20 KB | cell boundaries 4.7 KB | 16-bit lists 10 KB]; pass-through: [32-bit lists 20 KB]
@@ -381,8 +390,8 @@ k_density_tile(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
             b[2] = r1[0] + d1; b[3] = r1[3] + d1;
             b[4] = r2[0] + d2; b[5] = r2[3] + d2;
         }
-        density_particle<kNoise>(SmemAcc<SearchRec>{smem_addr_pinned(s_rec)}, TileList<uint16_t, 13>{s_list + threadIdx.x}, w, live,
-                                 s, b, g, P, pos, pair_rec, pair_cnt, ps_out, hn);
+        density_particle<kNoise, kEns>(SmemAcc<SearchRec>{smem_addr_pinned(s_rec)}, TileList<uint16_t, 13>{s_list + threadIdx.x},
+                                       w, live, s, b, g, P, pos, pair_rec, pair_cnt, ps_out, hn, E);
     } else {
         if (threadIdx.x == 0) atomicAdd(&cnt->n_untiled, 1u);  // rare; lets a test prove this path ran
         if (live) {
@@ -391,9 +400,9 @@ k_density_tile(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
             b[2] = cs0[nc]; b[3] = cs0[nc + 3u];
             b[4] = (cs0 - nc)[0]; b[5] = (cs0 - nc)[3];
         }
-        density_particle<kNoise>(GmemAcc<SearchRec>{rec},
-                                 TileList<uint32_t, 28>{reinterpret_cast<uint32_t *>(s_raw) + threadIdx.x}, w,
-                                 live, s, b, g, P, pos, pair_rec, pair_cnt, ps_out, hn);
+        density_particle<kNoise, kEns>(GmemAcc<SearchRec>{rec},
+                                       TileList<uint32_t, 28>{reinterpret_cast<uint32_t *>(s_raw) + threadIdx.x}, w,
+                                       live, s, b, g, P, pos, pair_rec, pair_cnt, ps_out, hn, E);
     }
 }
 
@@ -405,15 +414,16 @@ k_density_tile(Counters *cnt, Grid g, DevParams P, const uint32_t *cell_start,
 // Round 1 built this with a load/store staging loop and measured it SLOWER than gathering (60 vs 46 us): the loop's
 // instructions, its registers in flight and its barrier cost more than the gathers saved.  The bulk copy has none of
 // the three.
-template <bool kMonitor>
+template <bool kMonitor, bool kEns = false>
 #ifndef SC_K5_TILE_MINBLOCKS
 #define SC_K5_TILE_MINBLOCKS 4   // blocks per SM the register allocation is held to (4 = 64 registers)
 #endif
 __global__ void __launch_bounds__(SC_TILE, SC_K5_TILE_MINBLOCKS)
-k_force_tile(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallParams W, const BlockDesc *desc,
+k_force_tile(const uint32_t *n_ptr, DevParams P0, const __grid_constant__ WallParams W, const BlockDesc *desc,
              const double2 *pos, const float2 *vel, const uint2 *pair_rec,
              const uint8_t *pair_cnt, const PS<float> *ps_in, const uint32_t *wall_bits, const uint32_t *wall_slot,
-             const double2 *wall_pre, double2 *pos_out, float2 *vel_out, double *monitor, TickDuty duty, NextKeys nk) {
+             const double2 *wall_pre, double2 *pos_out, float2 *vel_out, double *monitor, TickDuty duty, NextKeys nk,
+             Members E) {
     pdl_enter();
     end_of_tick(duty, n_ptr);
     __shared__ __align__(128) float4 s_ps[SC_TILE_CAP];
@@ -446,7 +456,9 @@ k_force_tile(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallPar
     double2 ps_own = make_double2(0, 0);
     float2 v_own = make_float2(0, 0);
     bool touching = false;
+    uint32_t u = 0u;
     if (live) {
+        if constexpr (kEns) u = E.uid[s];
         me = ps_in[s];
         K = pair_cnt[s];
         ps_own = pos[s];
@@ -455,6 +467,9 @@ k_force_tile(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallPar
     }
     mbar_wait(bar, 0u);
     if (!live) return;
+    DevParams Pm;
+    if constexpr (kEns) Pm = member_params(E, u);
+    const DevParams &P = pick_params<kEns>(P0, Pm);
     const float p_i = me.p;
     const float smooth = P.f_smooth, two_target = P.f_two_target;
     float tx = 0, ty = 0;         // F3 sum
@@ -496,11 +511,11 @@ k_force_tile(const uint32_t *n_ptr, DevParams P, const __grid_constant__ WallPar
         for (int k = 0; k < Ks; ++k) pair(Arec.get((uint32_t)k * SC_TILE), gp, gv);
         for (int k = SC_K5_ROWS; k < K; ++k) pair(my_rec[k * SC_TILE], gp, gv);
     }
-    force_tail<float, kMonitor>(s, K, p_i, tx, ty, qx, qy, P, W, ps_own, v_own, touching, wall_slot, wall_pre, pos_out, vel_out,
-                                monitor, n_ptr, nk, [&](float vx, float vy, float &ax, float &ay) {
+    force_tail<float, kMonitor, kEns>(s, K, p_i, tx, ty, qx, qy, P, W, ps_own, v_own, touching, wall_slot, wall_pre,
+                                      pos_out, vel_out, monitor, n_ptr, nk, [&](float vx, float vy, float &ax, float &ay) {
         ax = sum_vx - (float)K * vx;
         ay = sum_vy - (float)K * vy;
-    });
+    }, kEns ? member_of(E, u) * E.ncells : 0u);
 }
 
 // ------------------------------------------------------------------------------------------------------------
