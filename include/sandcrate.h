@@ -82,6 +82,21 @@ int sc_particle_count(sc_ctx *ctx, int64_t *n);                     /* crate.py:
 /* any of pos / vel / pressure may be NULL.  pos, vel: n x 2; pressure: n (crate.py:26, 275). */
 int sc_get_state(sc_ctx *ctx, double *pos, double *vel, double *pressure, int64_t cap, int64_t *n);
 int sc_get_uids(sc_ctx *ctx, uint32_t *uid, int64_t cap, int64_t *n);
+/* The uid the next appended or emitted particle gets (identities advance by the drawn count, so a clamped emission
+ * leaves a gap that sc_set_state_uids alone cannot restore).  Refused below the context's current next uid and at or
+ * above 2^31.  With sc_set_state_uids it moves a scene into a new context with its identities intact. */
+int sc_set_next_uid(sc_ctx *ctx, uint32_t next_uid);
+
+/* Between ticks.  A call that returns an error leaves the context as it was.  Readbacks (sc_get_state, sc_get_uids,
+ * sc_particle_count), the parity taps, the diagnostics, measurement, the ForceMonitor switch, sc_synchronize and a
+ * configuration call with the bytes already set (sc_set_params, sc_set_walls, sc_set_tick) never change a later result.
+ * Pressure reads as the last tick computed it for each particle, and 0 for every particle once sc_set_state,
+ * sc_set_state_uids, sc_append_particles or sc_emit_particles changed the particle set since (crate.py:26); a re-grid (a
+ * new particle_radius, or walls that need more wall-contact room) keeps it, though the parity taps then refuse until the
+ * next step.  Inside a split step (between sc_step_begin and sc_step_finish) the parity taps but sc_get_tension,
+ * sc_set_params without a radius change, sc_set_noise, sc_set_tick, sc_set_walls with the walls already set,
+ * sc_last_pair_count, sc_synchronize and measurement are allowed; sc_get_state, sc_get_uids, sc_set_state,
+ * sc_append_particles, sc_emit_particles, sc_step, a radius change and a change of walls are refused. */
 
 /* create_new_particles + ParticleSource.generate_particles (crate.py:138-147, particle_source.py:17-24) on the DEVICE,
  * for the counter-based production mode (the reference-stream mode keeps drawing on the host and appends with
@@ -171,7 +186,9 @@ int sc_last_pair_count(sc_ctx *ctx, int64_t *n_pairs);
 
 /* ---- diagnostics (developer aids; no reference counterpart, results are never affected) ---------------------- */
 /* re-run the density (which = 4) or force (which = 5) kernel of the last tick `reps` times; mean milliseconds.
- * -1 before a step, inside a split step and under SC_NOISE_HOST (the step's noise offsets do not outlive it). */
+ * -1 before a step, inside a split step, under SC_NOISE_HOST (the step's noise offsets do not outlive it) and once a
+ * call has changed the parameters, walls or noise the step ran with.  The re-run takes back the next tick's keys (that
+ * tick then runs its own pre-pass), like every call that touches what they depend on. */
 double sc_debug_rerun(sc_ctx *ctx, int which, int reps);
 /* blocks of the tiled density kernel that ran in pass-through mode in the last tick (windows too large to stage) */
 int64_t sc_debug_untiled_blocks(sc_ctx *ctx);
@@ -290,6 +307,7 @@ int sc_dist_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsources, 
  *   refused: sc_set_params, sc_set_state, sc_set_state_uids, sc_append_particles, sc_emit_particles (use the sc_ens_
  *     forms), sc_step_begin / sc_step_finish, the parity taps, sc_debug_pair_records, sc_debug_rerun (returns -1),
  *     sc_set_monitor and sc_get_monitor (the monitor cannot be switched on, so there is nothing to read), sc_set_state_uids,
+ *     sc_set_next_uid,
  *     sc_dist_* (sc_dist_configure refuses; the other sc_dist_ calls need it). */
 int sc_ens_configure(sc_ctx *ctx, int members, int uid_bits);
 /* p[M], seeds[M]: each member's coefficients and noise seed.  dt and particle_radius must be the same in every member

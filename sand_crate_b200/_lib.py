@@ -90,6 +90,7 @@ SIGNATURES = {
     "sc_dist_set_rows": (C.c_int, [_ctx, C.c_int64, C.c_int64]),
     "sc_dist_set_reach": (C.c_int, [_ctx, C.c_int64, C.c_int64]),
     "sc_set_state_uids": (C.c_int, [_ctx, _dp, _dp, _up, C.c_int64]),
+    "sc_set_next_uid": (C.c_int, [_ctx, C.c_uint32]),
     "sc_dist_halo_rows": (C.c_int, [_dp, C.c_int, C.c_double]),
     "sc_dist_owned_count": (C.c_int, [_ctx, C.c_void_p]),
     "sc_dist_emit_particles": (C.c_int, [_ctx, C.POINTER(ScSource), C.c_int, C.c_int64, C.c_uint32, C.c_void_p]),
@@ -360,6 +361,10 @@ class Context:
         uid = np.ascontiguousarray(uid, dtype=np.uint32)
         assert pos.shape == vel.shape and uid.shape[0] == pos.shape[0]
         self._ck(self._L.sc_set_state_uids(self._h, _ptr(pos, _dp), _ptr(vel, _dp), _ptr(uid, _up), pos.shape[0]))
+
+    def set_next_uid(self, next_uid: int):
+        """The uid the next appended or emitted particle gets (sc_set_next_uid)."""
+        self._ck(self._L.sc_set_next_uid(self._h, C.c_uint32(next_uid)))
 
     def dist_configure(self, rank, nranks, row_lo, row_hi, halo_rows, wire_capacity):
         self._ck(self._L.sc_dist_configure(self._h, int(rank), int(nranks), int(row_lo), int(row_hi), int(halo_rows),

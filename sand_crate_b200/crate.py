@@ -111,6 +111,7 @@ class Crate:
         self._ctx = None
         self._open_context(cap)
         self._count = 0
+        self._next_uid = 0   # the uid the context gives the next new particle, tracked here so that growing keeps it
         self._cache: dict = {}
         self._kernel_ms: dict = {}
 
@@ -124,16 +125,22 @@ class Crate:
             self._ctx.set_monitor(True)
 
     def _ensure_capacity(self, needed: int) -> None:
+        """Moves the scene into a larger context with its identities: counter noise is keyed on uids, so renumbering
+        the particles would change the trajectory."""
         if needed <= self._ctx.capacity:
             return
         pos, vel, _ = self._ctx.get_state(want_pressure=False)   # own arrays: they must outlive the old context
+        uid = self._ctx.get_uids()
         self._cache = {}
         self._ctx.close()
         self._open_context(max(needed, 2 * self._ctx.capacity))
         self._push_params()
         self._ctx.set_tick(self.tick)
         if len(pos):
-            self._ctx.set_state(pos, vel)
+            self._ctx.set_state_uids(pos, vel, uid)
+        # set_state_uids continues after the largest uid; a clamped emission or a removal can leave a gap above it
+        if self._next_uid != (int(uid.max()) + 1 if len(uid) else 0):
+            self._ctx.set_next_uid(self._next_uid)
 
     def close(self) -> None:
         if self._ctx is not None:
@@ -192,6 +199,7 @@ class Crate:
         self._push_params()
         self._ctx.set_state(particles, velocities)
         self._count = len(particles)
+        self._next_uid = len(particles)
         self._cache = {}
 
     # ---- the tick ------------------------------------------------------------------------------------------
@@ -232,6 +240,7 @@ class Crate:
                 self._push_params()
                 self._ctx.append_particles(new_pos, new_vel)
                 self._count = self.particle_count + len(new_pos)
+                self._next_uid += len(new_pos)
                 self._cache = {}
 
     def _emit_on_device(self) -> None:
@@ -244,6 +253,7 @@ class Crate:
             self._push_params()
             self._ctx.set_tick(self.tick)
             self._ctx.emit_particles(records, int(self.max_particles))
+            self._next_uid += sum(max(int(r[6]), 0) for r in records)   # identities advance by the drawn counts
             self._count = None
             self._cache = {}
 

@@ -88,6 +88,10 @@ struct sc_ctx {
     bool n_exact = true;
     bool in_step = false;     // between sc_step_begin and sc_step_finish
     bool srt_valid = false;   // *_srt arrays hold the last tick's search state
+    bool prs_valid = false;   // ps holds the last tick's pressures of the current particle set (a re-grid keeps them)
+    // a call since the last step changed the parameters, walls or noise that step ran with: sc_debug_rerun refuses
+    bool step_inputs_changed = false;
+    uint64_t step_tick = 0;   // the tick the last step ran as (sc_debug_rerun re-runs it, whatever sc_set_tick did since)
     bool rows_valid = false;  // pos_cur / uid_cur are still in the order of the last search (cell rows ascending)
     bool lists_valid = false, rank_valid = false;
     bool carry_count = false; // the device count must be refreshed from the previous tick's scan total
@@ -280,7 +284,7 @@ static int setup_grid(sc_ctx *ctx, double d, int row_min, int row_max, int col_m
     return 0;
 }
 
-static void refresh_wall_boxes(sc_ctx *ctx);
+static void refresh_wall_boxes(WallParams &w, const DevParams &dp);
 static int contact_bound(const double (*seg_box)[4], int S);
 static int sync_count(sc_ctx *ctx);
 static void refresh_count(sc_ctx *ctx);
@@ -463,14 +467,17 @@ static int set_params(sc_ctx *ctx, const sc_params *p) {
     const bool regrid = !ctx->params_set || p->particle_radius != ctx->hp.particle_radius;
     if (regrid && ctx->in_step) return fail(ctx, "sc_set_params: radius change inside a split step");
     // the same bytes again (a Crate pushes its coefficients every tick) leave the next tick's keys valid
-    if (!ctx->params_set || std::memcmp(p, &ctx->hp, sizeof(sc_params)) != 0) CKR(drop_keys(ctx));
+    if (!ctx->params_set || std::memcmp(p, &ctx->hp, sizeof(sc_params)) != 0) {
+        CKR(drop_keys(ctx));
+        ctx->step_inputs_changed = true;
+    }
     if (regrid && ctx->params_set) CKR(sync_count(ctx));  // the live count sits in the old cell array's tail
     ctx->hp = *p;
     refresh_dev_params(ctx);
     if (regrid) {
         if (ctx->walls_set) {
             sc_pad_segments(&ctx->walls.seg[0][0], ctx->walls.S, ctx->dp.r, &ctx->walls.pad[0][0]);
-            refresh_wall_boxes(ctx);
+            refresh_wall_boxes(ctx->walls, ctx->dp);
             ctx->grid_contacts = std::max(ctx->grid_contacts, contact_bound(ctx->walls.seg_box, ctx->walls.S));
         }
         CKR(world_grid(ctx));  // room for the wall fix's shift (world_rows)
@@ -509,15 +516,14 @@ static void grow_box(double *box, double ax, double ay, double bx, double by, do
 }
 
 // bounding boxes for the conservative culls of WallParams
-static void refresh_wall_boxes(sc_ctx *ctx) {
-    WallParams &w = ctx->walls;
+static void refresh_wall_boxes(WallParams &w, const DevParams &dp) {
     auto grow = grow_box;
-    for (int k = 0; k < w.S; ++k) grow(w.seg_box[k], w.seg[k][0], w.seg[k][1], w.seg[k][2], w.seg[k][3], ctx->dp.touch);
+    for (int k = 0; k < w.S; ++k) grow(w.seg_box[k], w.seg[k][0], w.seg[k][1], w.seg[k][2], w.seg[k][3], dp.touch);
     for (int k = 0; k < 2 * w.S; ++k) grow(w.pad_box[k], w.pad[k][0], w.pad[k][1], w.pad[k][2], w.pad[k][3], 0.0);
     // Largest-area-greedy rectangle inside the world box that meets none of the boxes.  Only ever used as
     // "strictly inside -> nothing to test", so any rectangle that meets no box is correct; greedy just makes it big.
     auto safe_rect = [&](double (*boxes)[4], int nb, double *out) {
-        double r[4] = {ctx->dp.box_lo, ctx->dp.box_hi, ctx->dp.box_lo, ctx->dp.box_hi};
+        double r[4] = {dp.box_lo, dp.box_hi, dp.box_lo, dp.box_hi};
         auto meets = [&](const double *b) { return b[0] < r[1] && b[1] > r[0] && b[2] < r[3] && b[3] > r[2]; };
         for (int pass = 0; pass < nb + 1; ++pass) {
             bool changed = false;
@@ -590,38 +596,41 @@ extern "C" int sc_set_walls(sc_ctx *ctx, const double *segments, int S, const in
         const int v = segment_contact_bound(segments, S, ctx->dp.touch);
         if (halo_needed(v) > ctx->dist.halo) return fail(ctx, halo_message("sc_set_walls", v, ctx->dist.halo));
     }
-    WallParams &w = ctx->walls;
-    {   // the same walls again (a Crate pushes them every tick) leave the next tick's keys valid; moving ones do not
-        bool same = ctx->walls_set && S == w.S && nbodies == w.nbodies &&
-                    (S == 0 || std::memcmp(&w.seg[0][0], segments, sizeof(double) * 4 * (size_t)S) == 0);
-        int k = 0;
-        for (int b = 0; same && b < nbodies; ++b) {
-            same = std::memcmp(w.kin[b], body_kin + 5 * b, sizeof(double) * 5) == 0;
-            for (int q = 0; same && q < body_len[b]; ++q, ++k) same = k < S && w.seg_body[k] == b;
-        }
-        if (!same || k != S) CKR(drop_keys(ctx));
-    }
-    w.S = S; w.nbodies = nbodies;
-    int k = 0;
+    // everything is checked, and the new walls are built in a copy, before anything changes: a refused call leaves
+    // the context as it was
+    int64_t total = 0;
     for (int b = 0; b < nbodies; ++b) {
-        for (int q = 0; q < body_len[b]; ++q) {
-            if (k >= S) return fail(ctx, "sc_set_walls: body_len does not sum to S");
-            w.seg_body[k++] = b;
-        }
+        if (body_len[b] < 0) return fail(ctx, "sc_set_walls: negative body_len");
+        total += body_len[b];
+    }
+    if (total != S) return fail(ctx, "sc_set_walls: body_len does not sum to S");
+    WallParams w = ctx->walls;
+    w.S = S; w.nbodies = nbodies;
+    for (int b = 0, k = 0; b < nbodies; ++b) {
+        for (int q = 0; q < body_len[b]; ++q) w.seg_body[k++] = b;
         for (int q = 0; q < 5; ++q) w.kin[b][q] = body_kin[5 * b + q];
     }
-    if (k != S) return fail(ctx, "sc_set_walls: body_len does not sum to S");
     if (S) std::memcpy(&w.seg[0][0], segments, sizeof(double) * 4 * (size_t)S);
+    // the same walls again (a Crate pushes them every tick) change nothing and leave the next tick's keys valid
+    const WallParams &o = ctx->walls;
+    if (ctx->walls_set && S == o.S && nbodies == o.nbodies &&
+        std::memcmp(w.seg, o.seg, sizeof(double) * 4 * (size_t)S) == 0 &&
+        std::memcmp(w.seg_body, o.seg_body, sizeof(int) * (size_t)S) == 0 &&
+        std::memcmp(w.kin, o.kin, sizeof(double) * 5 * (size_t)nbodies) == 0)
+        return 0;
+    // sc_step_begin ran the wall fix and the contacts on the walls it found; the finish must bounce on the same ones
+    if (ctx->in_step) return fail(ctx, "sc_set_walls: the walls cannot change inside a split step");
     sc_pad_segments(&w.seg[0][0], S, ctx->dp.r, &w.pad[0][0]);
-    refresh_wall_boxes(ctx);
+    refresh_wall_boxes(w, ctx->dp);
+    CKR(drop_keys(ctx));
+    ctx->walls = w;
     ctx->walls_set = true;
+    ctx->step_inputs_changed = true;
     // walls that can give a particle more contacts than the grid has room for: a larger grid (never a smaller one, so
     // a moving body does not re-grid back and forth).  refresh_count carries the live count out of the old cell
     // array on the stream: no host wait.
     const int v = contact_bound(w.seg_box, w.S);
     if (v > ctx->grid_contacts) {
-        if (ctx->in_step) return fail(ctx, "sc_set_walls: walls that need a larger cell grid inside a split step");
-        CKR(drop_keys(ctx));
         refresh_count(ctx);
         ctx->grid_contacts = v;
         CKR(world_grid(ctx));
@@ -636,6 +645,7 @@ extern "C" int sc_set_noise(sc_ctx *ctx, int mode, uint64_t seed) {
     if (ctx->ens && mode == SC_NOISE_HOST)
         return fail(ctx, "sc_set_noise: an ensemble cannot take the reference's noise stream (SC_NOISE_HOST): that "
                          "stream is one per process");
+    if (mode != ctx->noise_mode || seed != ctx->seed) ctx->step_inputs_changed = true;
     ctx->noise_mode = mode; ctx->seed = seed;
     if (ctx->ens && ctx->params_set) CKR(ens_upload(ctx));  // the members' effective modes follow the mode
     return 0;
@@ -695,11 +705,11 @@ static int upload_particles(sc_ctx *ctx, const double *pos, const double *vel, i
 }
 
 static int set_state(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
-    CKR(drop_keys(ctx));
     if (n < 0 || n > ctx->cap) return fail(ctx, "sc_set_state: n exceeds capacity");
     if (ctx->in_step) return fail(ctx, "sc_set_state: inside a split step");
+    CKR(drop_keys(ctx));
     ctx->next_uid = 0;
-    ctx->srt_valid = false; ctx->lists_valid = false; ctx->rows_valid = false;
+    ctx->srt_valid = false; ctx->prs_valid = false; ctx->lists_valid = false; ctx->rows_valid = false;
     ctx->carry_count = false;  // the count is (re)defined by the host below
     const uint32_t zero = 0;
     CK(cudaMemcpyAsync(&ctx->cnt->n, &zero, sizeof(uint32_t), cudaMemcpyHostToDevice, ctx->stream));
@@ -728,15 +738,25 @@ extern "C" int sc_set_state_uids(sc_ctx *ctx, const double *pos, const double *v
     return 0;
 }
 
+extern "C" int sc_set_next_uid(sc_ctx *ctx, uint32_t next_uid) {
+    CKR(enter(ctx, "sc_set_next_uid"));
+    CKR(no_ensemble(ctx, "sc_set_next_uid"));
+    if (next_uid < ctx->next_uid)
+        return fail(ctx, "sc_set_next_uid: below the next uid (" + std::to_string(ctx->next_uid) + "): a uid would repeat");
+    if (next_uid & SC_GHOST_BIT) return fail(ctx, "sc_set_next_uid: uids must be < 2^31");
+    ctx->next_uid = next_uid;
+    return 0;
+}
+
 extern "C" int sc_append_particles(sc_ctx *ctx, const double *pos, const double *vel, int64_t n) {
     CKR(enter(ctx, "sc_append_particles"));
     CKR(no_ensemble(ctx, "sc_append_particles"));
-    CKR(drop_keys(ctx));
     if (ctx->in_step) return fail(ctx, "sc_append_particles: inside a split step");
     if (n < 0) return fail(ctx, "sc_append_particles: n < 0");
     CKR(sync_count(ctx));
     if (ctx->n_host + n > ctx->cap) return fail(ctx, "sc_append_particles: capacity exceeded");
-    ctx->srt_valid = false; ctx->lists_valid = false;  // (appended rows sit behind the sorted ones: rows_valid stays)
+    CKR(drop_keys(ctx));
+    ctx->srt_valid = false; ctx->prs_valid = false; ctx->lists_valid = false;  // (appended rows sit behind the sorted ones: rows_valid stays)
     return upload_particles(ctx, pos, vel, ctx->n_host, n);
 }
 
@@ -769,9 +789,9 @@ extern "C" int sc_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsou
         total += S.n;
     }
     if (!E.nsrc) return 0;
-    CKR(drop_keys(ctx));  // the new particles have no keys
     if ((uint64_t)ctx->next_uid + total >= (uint64_t)SC_GHOST_BIT)
         return fail(ctx, "particle identities exhausted (2^31 particles created in this context)");
+    CKR(drop_keys(ctx));  // the new particles have no keys
     refresh_count(ctx);
     {
         ProfScope ps(ctx, SLOT_IO);
@@ -785,7 +805,7 @@ extern "C" int sc_emit_particles(sc_ctx *ctx, const sc_source *sources, int nsou
     ctx->next_uid += (uint32_t)total;
     ctx->n_host = std::min<int64_t>(ctx->n_host + (int64_t)total, ctx->cap);  // an upper bound: the clamp happened on the device
     ctx->n_exact = false;
-    ctx->srt_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
+    ctx->srt_valid = false; ctx->prs_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
     return 0;
 }
 
@@ -1101,6 +1121,9 @@ static int enqueue_forces(sc_ctx *ctx, const uint32_t *noise_off) {
     if (n > 0) { ctx->next_clean = !keys; ctx->next_keyed = keys; ctx->carry_count = false; }
     else ctx->carry_count = true;  // nothing ran: cnt->n is refreshed by the next cold start or by sync_count
     ctx->keys_dropped = false;
+    ctx->prs_valid = true;
+    ctx->step_inputs_changed = false;
+    ctx->step_tick = ctx->tick;
     CK(cudaGetLastError());
     ctx->rows_valid = n > 0;
     ctx->dist_tail = false;
@@ -1226,8 +1249,8 @@ extern "C" int sc_get_state(sc_ctx *ctx, double *pos, double *vel, double *press
         CK(cudaMemcpyAsync(vel, ctx->stage2, sizeof(double2) * (size_t)n, cudaMemcpyDeviceToHost, ctx->stream));
     }
     if (pressure) {
-        if (!ctx->srt_valid) {
-            CK(cudaMemsetAsync(ctx->stage1, 0, sizeof(double) * (size_t)n, ctx->stream));  // crate.py:26 before any tick
+        if (!ctx->prs_valid) {  // no tick since the particle set changed: crate.py:26 before any tick
+            CK(cudaMemsetAsync(ctx->stage1, 0, sizeof(double) * (size_t)n, ctx->stream));
         } else {
             ProfScope ps(ctx, SLOT_IO);
             if (ctx->precision == SC_PRECISION_F64)
@@ -1491,10 +1514,13 @@ extern "C" int sc_debug_walls(sc_ctx *ctx, double *rects, double *seg_box, doubl
 // ---- developer aids (declared in include/sandcrate.h under "diagnostics"): re-run one pair kernel of the last tick
 // `reps` times and return the mean milliseconds.  K4 and K5 only read the sorted set, so re-running them is harmless.
 // -1 before a step, inside a split step, and under SC_NOISE_HOST: the step's noise offsets live in count_by_rank, which
-// the next count kernel (sc_get_neighbors, say) overwrites.
+// the next count kernel (sc_get_neighbors, say) overwrites.  -1 as well once a call has changed the parameters, walls
+// or noise the step ran with (the re-run would compute a different tick), and after a step with no particles.  It re-runs the step's own tick whatever
+// sc_set_tick did since.
 extern "C" double sc_debug_rerun(sc_ctx *ctx, int which, int reps) {
-    if (!ctx || !ctx->srt_valid || ctx->in_step || ctx->ens) return -1.0;
-    const DevParams dp = step_params(ctx, ctx->tick - 1);
+    if (!ctx || !ctx->srt_valid || ctx->in_step || ctx->ens || ctx->step_inputs_changed) return -1.0;
+    if (ctx->n_host == 0) return -1.0;  // nothing to re-run (an empty launch would be a launch error)
+    const DevParams dp = step_params(ctx, ctx->step_tick);
     if (dp.noise_mode == SC_NOISE_HOST) return -1.0;
     cudaSetDevice(ctx->device);
     if (drop_keys(ctx)) return -1.0;  // the force kernel re-run below computes no keys, and its own must not be counted twice
@@ -1504,7 +1530,7 @@ extern "C" double sc_debug_rerun(sc_ctx *ctx, int which, int reps) {
     for (int r = 0; r < reps; ++r) {
         if (which == 4) cudaMemsetAsync(&ctx->cnt->pair_cursor, 0, 4, ctx->stream);  // the fp64 K4 allocates from zero
         cudaEventRecord(e0, ctx->stream);
-        launch_pair_kernels(ctx, dp, nullptr, which == 4, which != 4, false, ctx->tick - 1);
+        launch_pair_kernels(ctx, dp, nullptr, which == 4, which != 4, false, ctx->step_tick);
         cudaEventRecord(e1, ctx->stream);
         cudaEventSynchronize(e1);
         float ms = 0;
@@ -1593,13 +1619,13 @@ extern "C" int sc_dist_configure(sc_ctx *ctx, int rank, int nranks, int64_t row_
         const int v = contact_bound(ctx->walls.seg_box, ctx->walls.S);
         if (halo_rows < halo_needed(v)) return fail(ctx, halo_message("sc_dist_configure", v, halo_rows));
     }
-    CKR(drop_keys(ctx));
     if (nranks < 1 || rank < 0 || rank >= nranks) return fail(ctx, "sc_dist_configure: bad rank");
     if (halo_rows < 1) return fail(ctx, "sc_dist_configure: halo_rows must be >= 1");
     if (wire_capacity < 1 || wire_capacity > ctx->cap) return fail(ctx, "sc_dist_configure: bad wire capacity");
     if (rank > 0 && rank < nranks - 1 && row_hi - row_lo < 2 * (int64_t)halo_rows)
         return fail(ctx, "sc_dist_configure: a strip must be at least 2 * halo_rows high");
     if (ctx->noise_mode == SC_NOISE_HOST) return fail(ctx, "sc_dist_configure: SC_NOISE_HOST is single-GPU only");
+    CKR(drop_keys(ctx));
     ctx->dist.row_lo = row_lo; ctx->dist.row_hi = row_hi; ctx->dist.halo = halo_rows;
     ctx->dist.far_lo = row_lo - halo_rows; ctx->dist.far_hi = row_hi + halo_rows;  // until sc_dist_set_reach says more
     ctx->dist.reach_set = 0;
@@ -1739,7 +1765,8 @@ static int enqueue_pack(sc_ctx *ctx, const char *who, void *send_lo_dev, void *s
 #undef SC_PACK
     }
     CK(cudaGetLastError());
-    ctx->srt_valid = false; ctx->rank_valid = false; ctx->lists_valid = false; ctx->rows_valid = false;
+    ctx->srt_valid = false; ctx->prs_valid = false; ctx->rank_valid = false; ctx->lists_valid = false;
+    ctx->rows_valid = false;
     ctx->n_exact = false;
     return 0;
 }
@@ -1890,7 +1917,7 @@ extern "C" int sc_dist_emit_particles(sc_ctx *ctx, const sc_source *sources, int
     ctx->next_uid = std::max<uint32_t>(ctx->next_uid, first_uid + (uint32_t)total);
     ctx->n_host = std::min<int64_t>(ctx->n_host + (int64_t)total, ctx->cap);  // an upper bound
     ctx->n_exact = false;
-    ctx->srt_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
+    ctx->srt_valid = false; ctx->prs_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
     ctx->dist_tail = true;  // behind the sorted rows: the next pack must reach them (enqueue_pack)
     return 0;
 }
@@ -2102,7 +2129,7 @@ extern "C" int sc_ens_emit_particles(sc_ctx *ctx, const sc_source *sources, int 
     ctx->ens_stale = false;
     ctx->n_host = std::min<int64_t>(ctx->n_host + (int64_t)total, ctx->cap);  // an upper bound: the clamp is on the device
     ctx->n_exact = false;
-    ctx->srt_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
+    ctx->srt_valid = false; ctx->prs_valid = false; ctx->lists_valid = false; ctx->rank_valid = false;
     return 0;
 }
 

@@ -6,6 +6,7 @@ touch oracle/; the product never sees it."""
 import numpy as np
 
 from oracle import oracle as O
+from sand_crate_b200._lib import SandCrateError
 
 
 class OracleContext:
@@ -145,6 +146,12 @@ class OracleContext:
         self.set_state(pos, vel)
         self.uid = np.array(uid, dtype=np.uint32)
         self.next_uid = int(self.uid.max()) + 1 if len(self.uid) else 0
+
+    def set_next_uid(self, next_uid):
+        """sc_set_next_uid: refused below the current next uid and at or above 2^31."""
+        if not self.next_uid <= next_uid < 2 ** 31:
+            raise SandCrateError(f"sc_set_next_uid: {next_uid} out of range")
+        self.next_uid = int(next_uid)
 
     def dist_configure(self, rank, nranks, row_lo, row_hi, halo_rows, wire_capacity):
         self.dist = dict(lo=row_lo, hi=row_hi, halo=halo_rows, has_lo=rank > 0, has_hi=rank < nranks - 1,

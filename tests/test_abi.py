@@ -21,7 +21,7 @@ def declared_functions():
 def test_header_declares_the_expected_surface():
     names = declared_functions()
     for must in ("sc_create", "sc_destroy", "sc_step", "sc_step_begin", "sc_step_finish", "sc_set_walls",
-                 "sc_get_state", "sc_detect_particle_collisions", "sc_points_to_segments_distance"):
+                 "sc_get_state", "sc_set_next_uid", "sc_detect_particle_collisions", "sc_points_to_segments_distance"):
         assert must in names
 
 

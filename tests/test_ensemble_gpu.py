@@ -161,28 +161,32 @@ def test_members_of_different_sizes_straddle_blocks():
 
 def test_max_particles_raised_mid_run():
     """Raising one member's max_particles past what the context was sized for grows the context, identities kept, and
-    the member stays bit-identical to a Crate edited the same way (one with room for it, so it keeps its own uids)."""
+    the member stays bit-identical to a Crate edited the same way: one with room for it and one with the default
+    capacity, which grows its own context, so both growth paths must keep the identities."""
     world, _ = world_from_freerun("wave_machine")
     overrides = [{"max_particles": 300}, {"max_particles": 300}, {"max_particles": 500}]
     ens = Ensemble(world, overrides, seeds=[1, 2, 3])
     crates = [Crate(with_coeffs(world, o), precision="mixed", noise="counter", noise_seed=s, capacity=4000)
               for o, s in zip(overrides, [1, 2, 3])]
+    grown = Crate(with_coeffs(world, overrides[1]), precision="mixed", noise="counter", noise_seed=2)
     try:
         cap0 = ens._ctx.capacity
         for t in range(1, 201):
             if t == 61:
                 ens.member(1).max_particles = 3000
-                crates[1].max_particles = 3000
+                crates[1].max_particles = grown.max_particles = 3000
             ens.physics_tick()
-            for c in crates:
+            for c in crates + [grown]:
                 c.physics_tick()
             if t % 40 == 0:
                 for m, c in enumerate(crates):
                     assert_member_equal(ens, m, c, f"tick {t}")
+                assert_member_equal(ens, 1, grown, f"tick {t}, grown Crate")
         assert ens._ctx.capacity > cap0 and ens.member(1).particle_count > 300
+        assert grown._ctx.capacity > 300
     finally:
         ens.close()
-        for c in crates:
+        for c in crates + [grown]:
             c.close()
 
 

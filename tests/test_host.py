@@ -175,3 +175,67 @@ def test_counter_sources_host_protocol(oracle_backend):
         crate.physics_tick()
     assert crate.particle_count == len(pos) == 100
     assert np.array_equal(crate.particles, pos)
+
+
+def _same_crates(a, b, tick):
+    assert a.particle_count == b.particle_count, tick
+    assert np.array_equal(a._ctx.get_uids(), b._ctx.get_uids()), tick
+    assert np.array_equal(a.particles, b.particles), tick
+    assert np.array_equal(a.particle_velocities, b.particle_velocities), tick
+
+
+def _wave_machine(max_particles):
+    import copy
+    world, _ = world_from_freerun("wave_machine")
+    c = copy.deepcopy(dict(world.coefficients))
+    c["max_particles"] = max_particles
+    return sand_crate_b200.WorldConfig(rigid_bodies=world.rigid_bodies, particle_sources=world.particle_sources,
+                                       coefficients=c)
+
+
+def test_crate_growth_keeps_identities_counter_noise(oracle_backend):
+    """A Crate that grows its context keeps every uid and the next one: counter noise is keyed on uids, so a grown
+    Crate and one with room from the start stay identical.  The clamp binds before the raise, so the emission leaves
+    gaps in the identities that the next uid must jump over."""
+    grown = Crate(_wave_machine(300), noise="counter", noise_seed=2)
+    roomy = Crate(_wave_machine(300), noise="counter", noise_seed=2, capacity=4000)
+    clamped = False
+    for tick in range(1, 91):
+        if tick == 61:
+            clamped = grown.particle_count == 300
+            grown.max_particles = roomy.max_particles = 3000
+        grown.physics_tick()
+        roomy.physics_tick()
+        _same_crates(grown, roomy, tick)
+    assert clamped and grown._ctx.capacity > 300 and grown.particle_count > 300
+
+
+def test_crate_growth_through_set_particles_keeps_identities(oracle_backend):
+    rs = np.random.RandomState(4)
+    pos = 0.2 + 0.6 * rs.rand(400, 2)
+    grown = Crate(_wave_machine(500), noise="counter", noise_seed=5, capacity=64)
+    roomy = Crate(_wave_machine(500), noise="counter", noise_seed=5, capacity=4000)
+    for c in (grown, roomy):
+        c.set_particles(pos)                     # beyond the capacity of `grown`: it grows here ...
+    for tick in range(1, 61):
+        if tick == 31:
+            grown.max_particles = roomy.max_particles = 2000   # ... and again here, after clamped emissions
+        grown.physics_tick()
+        roomy.physics_tick()
+        _same_crates(grown, roomy, tick)
+    assert grown._ctx.capacity > 500 and grown.particle_count > 500
+
+
+def test_crate_growth_keeps_identities_reference_noise(oracle_backend):
+    world, _ = world_from_freerun("stirring_cup")
+    grown = Crate(world, capacity=8)
+    states = []
+    for _ in range(40):
+        grown.physics_tick()
+        states.append((grown._ctx.get_uids(), grown.particles.copy(), grown.particle_velocities.copy()))
+    roomy = Crate(world, capacity=4000)           # (each Crate reseeds the global stream the sources draw from)
+    for tick, (uid, pos, vel) in enumerate(states, 1):
+        roomy.physics_tick()
+        assert np.array_equal(roomy._ctx.get_uids(), uid), tick
+        assert np.array_equal(roomy.particles, pos) and np.array_equal(roomy.particle_velocities, vel), tick
+    assert grown._ctx.capacity > 8
